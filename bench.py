@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — Msamples/s (and Mrays/s) of the radiance loop on BASELINE.json's configurations.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C2] [--also C3,C4,C5] [--impl ptb|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C2] [--also C3,C4,C5] [--impl ptb|reference] [--dump-outputs DIR]
 
 A step is one full render of the named configuration (default C2 = BASELINE.json configs[1]: 1,000,000-triangle
 Phong mesh + HDR-style envmap, 1024x1024, 256 spp, depth 5) on synthetic, closed-form inputs.  Scene generation,
@@ -19,6 +19,9 @@ For N > 1 (torchrun, one rank per GPU) the frame is tile-sharded and gathered on
 (ptb_render_sharded); value = samples of all ranks / max-over-ranks time: strong scaling on the fixed frame.
 `--impl reference` times the reference's CPU implementation on a FIXED number of samples per pixel per step (REF_SPP below),
 whatever --steps / --warmup are, so that this arm and `cpu_baseline` measure the same thing.
+`--dump-outputs DIR` writes the frame the last timed step of the named workload computed (see dump_outputs) as DIR/<name>.npy,
+so that two builds can be compared output for output: the scenes are closed-form and the seed is fixed, so the inputs are identical
+from run to run.
 """
 import argparse
 import ctypes as C
@@ -52,6 +55,24 @@ REF_SPP = {"C1": 64, "C2": 32, "C3": 8, "C4": 16, "C5": 2}
 SHADE_BYTES = 340      # queue 4 + hit/ray o/ray d/weight/radiance 80 + rng 8 + pixel 4 + TriUV 32 + TriShade 80 + rpp 8 read; ray, weight, hit 64 + rng 8 + queue 4 + shadow entry 48 written
 KERNEL_LABEL = {"extend": "k_trace<closest-hit> (BVH8 traversal)", "shadow": "k_trace<any-hit> (BVH8 traversal, shadow rays)",
                 "shade": "k_shade (material fetch, BRDF eval / sampling, next-event estimation)", "raygen": "k_raygen", "splat": "k_splat"}
+DUMP_BYTES = 60 * 10 ** 6      # --dump-outputs stays below 64 MB with the .npy headers
+
+
+def dump_outputs(rt, out_dir):
+    """The frame the last timed step of `value` left on the device, resolved (ptb_resolve_last) into the arrays
+    Raytracer::render_image_nopreviz() hands its caller, as float32 .npy files: the linear image (imagedouble), the per-pixel filter
+    weight sums (sample_count) and the 8-bit display image (image).  A frame larger than
+    DUMP_BYTES (C5) is cut down to the same seeded sample of pixels in every run; pixel_index.npy lists them (row-major)."""
+    arrays = {k: np.asarray(getattr(rt, k), np.float32) for k in ("imagedouble", "sample_count", "image")}
+    if sum(a.nbytes for a in arrays.values()) > DUMP_BYTES:
+        n_px = rt.H * rt.W
+        per_px = sum(a.nbytes for a in arrays.values()) // n_px
+        idx = np.sort(np.random.default_rng(0).choice(n_px, DUMP_BYTES // (per_px + 8), replace=False))
+        arrays = {k: a.reshape(n_px, *a.shape[2:])[idx] for k, a in arrays.items()}
+        arrays["pixel_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), a)
 
 
 class ClockSampler:
@@ -202,7 +223,13 @@ def main():
     ap.add_argument("--also", default=None, help="comma-separated workloads measured briefly in the same run (default: C3,C4,C5 next to C2; '' for none)")
     ap.add_argument("--impl", default="ptb", choices=["ptb", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step of --workload as DIR/<name>.npy (float32, under 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; --impl reference renders fewer spp than the workload")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -242,9 +269,10 @@ def main():
         if world > 1:
             dist.barrier()
 
-    def measure(workload, steps, warmup, brief):
+    def measure(workload, steps, warmup, brief, dump_dir=None):
         """One workload on this rank's GPU.  brief: the warm-up steps and the instrumented steps run at reduced spp (they warm clocks and
-        allocations and time single launches, which do not depend on the number of passes); the timed steps are always full renders."""
+        allocations and time single launches, which do not depend on the number of passes); the timed steps are always full renders.
+        dump_dir: where rank 0 writes the outputs of the last timed step (dump_outputs)."""
         t0 = time.time(); rt = make_rt(lib, workload, device=local); gen_s = time.time() - t0
         rt.build_threads = max(1, (os.cpu_count() or 1) // max(1, world))   # torchrun exports OMP_NUM_THREADS=1
         t0 = time.time(); rt.commit(); commit_s = time.time() - t0
@@ -313,6 +341,9 @@ def main():
         if rank == 0:
             sampler.start()
         wall_ms, dev_ms, launches, rays = timed(rt.render_resident, steps)
+        if dump_dir and rank == 0:
+            rt.resolve_last()          # the frame the last timed step left on the device
+            dump_outputs(rt, dump_dir)
         # per-kernel CUDA-event timing (two event records per launch on the launching stream).  The timed region above runs the passes
         # on two pipelines (streams) whose kernels overlap, so a kernel's own duration is taken from one more step of the same
         # workload, right here, with the pipelines serialised: `roofline.launch_ms` is the kernel running alone on the GPU.
@@ -350,7 +381,7 @@ def main():
         return res
 
     line = dict(base_line)
-    line.update(measure(args.workload, args.steps, max(args.warmup, 3), brief=False))
+    line.update(measure(args.workload, args.steps, max(args.warmup, 3), brief=False, dump_dir=args.dump_outputs))
     if also:
         line["also"] = {}
         for w in also:

@@ -4,8 +4,8 @@
 TEST INFRASTRUCTURE ONLY.  Nothing in the product (pathtracer_b200/) may import, link or execute
 anything produced here; only tests/, __graft_entry__.smoke() and bench.py's CPU-baseline legs do.
 
-The reference (/root/reference, read-only) does not compile with GCC as shipped, so its sources are
-copied to a throw-away temp dir, patched there, compiled together with oracle/ref_driver.cpp (ours)
+The reference (the checkout of nbonneel/pathtracer given as the argument, read-only; tests/oracles.py passes the one
+PTB_REFERENCE_DIR names) does not compile with GCC as shipped, so its sources are copied to a throw-away temp dir, patched there, compiled together with oracle/ref_driver.cpp (ours)
 and the temp dir is deleted.  No reference source enters the repo; the only output is the .so under
 oracle/_ref/ (git-ignored, travels to the GPU box).
 
@@ -38,7 +38,6 @@ import sys
 import tempfile
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = os.environ.get("PTB_REFERENCE_DIR", "/root/reference")
 OUT = os.path.join(HERE, "_ref")
 
 UNITY = ["Vector.cpp", "Geometry.cpp", "TriangleMesh.cpp", "PointSet.cpp", "fluid.cpp", "Raytracer.cpp"]
@@ -140,10 +139,11 @@ def patch(tmp):
     wr("Geometry.cpp", g)
 
 
-def main():
-    if not os.path.isdir(REF):
-        print(f"build_ref: {REF} not present; keeping any prebuilt oracle/_ref", file=sys.stderr)
-        return 0
+def main(argv):
+    if len(argv) != 2 or not os.path.isdir(argv[1]):
+        print("usage: build_ref.py <checkout of nbonneel/pathtracer>", file=sys.stderr)
+        return 2
+    REF = argv[1]
     os.makedirs(OUT, exist_ok=True)
     tmp = tempfile.mkdtemp(prefix="ptb_ref_build_")
     try:
@@ -179,4 +179,4 @@ def main():
 
 
 if __name__ == "__main__":
-    sys.exit(main())
+    sys.exit(main(sys.argv))

@@ -24,7 +24,7 @@ def ref():
     from oracles import ref_lib
     lib = ref_lib()
     if lib is None:
-        pytest.skip("oracle/_ref not built (needs /root/reference); the golden fixtures carry its outputs")
+        pytest.skip("oracle/_ref not built (PTB_REFERENCE_DIR names no checkout of the reference); the golden fixtures carry its outputs")
     return lib
 
 

@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
 """Generate the golden vectors under tests/golden/ from oracle/_ref — the REFERENCE's own sources
-compiled headless by oracle/build_ref.py (only possible where /root/reference is mounted).
+compiled headless by oracle/build_ref.py (only possible where PTB_REFERENCE_DIR names a checkout of the reference).
 
 The fixtures pin oracle/port (and through it the CUDA path) to outputs of the reference itself:
   kat.npz        function-level known answers: inputs + reference outputs for every PTB_KAT_* block
@@ -100,7 +100,7 @@ def modes_golden(R):
 
 def main():
     R = ref_lib()
-    assert R is not None, "oracle/_ref is not built (needs /root/reference)"
+    assert R is not None, "oracle/_ref is not built (set PTB_REFERENCE_DIR to a checkout of the reference)"
     only = [a.split("=", 1)[1].split(",") for a in sys.argv if a.startswith("--only=")]      # --only=NGAN,C1: just these scene fixtures
     if "--sceneio-only" in sys.argv:
         sceneio_golden(R)

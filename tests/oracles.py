@@ -13,11 +13,23 @@ PORT_SO = os.path.join(ROOT, "oracle", "port", "libptb_port.so")
 _cache = {}
 
 
+def reference_dir():
+    """The checkout of the reference (nbonneel/pathtracer) that PTB_REFERENCE_DIR names, or None.  The repository holds only the
+    reference's outputs (tests/golden/); its sources, and oracle/_ref built from them, come from there or not at all."""
+    d = os.environ.get("PTB_REFERENCE_DIR")
+    return d if d and os.path.isdir(d) else None
+
+
+def build_ref():
+    """Compile oracle/_ref from reference_dir() (oracle/build_ref.py)."""
+    subprocess.check_call([sys.executable, os.path.join(ROOT, "oracle", "build_ref.py"), reference_dir()])
+
+
 def ref_lib():
     """oracle/_ref: the reference's own sources compiled headless (None if it was never built)."""
     if "ref" not in _cache:
-        if not os.path.exists(REF_SO) and os.path.isdir("/root/reference"):
-            subprocess.check_call([sys.executable, os.path.join(ROOT, "oracle", "build_ref.py")])
+        if not os.path.exists(REF_SO) and reference_dir():
+            build_ref()
         _cache["ref"] = Lib(ctypes.CDLL(REF_SO, mode=ctypes.RTLD_LOCAL), "ref_") if os.path.exists(REF_SO) else None
     return _cache["ref"]
 

@@ -169,16 +169,18 @@ def test_generators_are_deterministic_and_sized():
 def test_material_presets_equal_the_reference_menu():
     """Phong / Ngan material presets (north_star: "Phong/Ngan/MERL materials"): the table of the Python mirror, the table inside the
     library (ptb_preset_get) and the constants of the reference's object menu (mainApp.cpp:1499-1597, committed as
-    tests/golden/presets.json by tests/golden/make_presets.py; re-parsed live when /root/reference is present) are the same numbers."""
+    tests/golden/presets.json by tests/golden/make_presets.py; re-parsed live when PTB_REFERENCE_DIR names the reference) are the same numbers."""
     import ctypes as C
     import json
     import pathtracer_b200
     from pathtracer_b200 import api
     gold = json.load(open(os.path.join(ROOT, "tests", "golden", "presets.json")))
-    if os.path.exists("/root/reference/mainApp.cpp"):
+    from oracles import reference_dir
+    menu = os.path.join(reference_dir(), "mainApp.cpp") if reference_dir() else None
+    if menu and os.path.exists(menu):
         sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
         import make_presets
-        assert make_presets.parse() == gold
+        assert make_presets.parse(menu) == gold
     assert sorted(gold) == sorted(api.PRESETS) and len(gold) == 14 and sum(k.endswith("_ngan") for k in gold) == 7
     lib = pathtracer_b200.load()
     assert lib.preset_count() == 14 and lib.preset_find(b"nope") == -1

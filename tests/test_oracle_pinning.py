@@ -1,7 +1,7 @@
 """Pins the oracle: oracle/port (plain-C restatement) must reproduce the REFERENCE's own outputs —
 (1) the known answers recorded in SURVEY.md App. E, (2) the golden vectors under tests/golden/ that
 tests/golden/make_golden.py generated from oracle/_ref, bit for bit, and (3) oracle/_ref itself when it is
-present in this checkout (it is whenever /root/reference is mounted or a prebuilt .so travelled)."""
+present in this checkout (it is whenever PTB_REFERENCE_DIR names a checkout of the reference at build time)."""
 import os
 
 import numpy as np
