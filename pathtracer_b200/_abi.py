@@ -15,17 +15,19 @@ SLOT_KD, SLOT_KS, SLOT_NE, SLOT_TRANSP, SLOT_REFR, SLOT_NORMAL, SLOT_ALPHA, SLOT
 OBJ_MIRROR, OBJ_FLIP_NORMALS, OBJ_FLAT_NORMALS, OBJ_GHOST, OBJ_DISPLAY_EDGES = 1, 2, 4, 8, 16
 BRDF_PHONG, BRDF_MERL = 0, 1
 KEY_SCALE, KEY_TRANSLATION, KEY_ROTATION = 0, 1, 2
-OPT_COUNT_TRAVERSAL, OPT_POOL_PATHS, OPT_TIME_KERNELS, OPT_REFILL_BELOW, OPT_TRACE_BLOCKS, OPT_TRI_FRACTION, OPT_TRI_MIN_PCT, OPT_SORT_HITS, OPT_PIPES = 1, 2, 3, 4, 5, 6, 7, 8, 9
+OPT_COUNT_TRAVERSAL, OPT_POOL_PATHS, OPT_TIME_KERNELS, OPT_REFILL_BELOW, OPT_TRACE_BLOCKS, OPT_TRI_FRACTION, OPT_TRI_MIN_PCT = 1, 2, 3, 4, 5, 6, 7
+OPT_PIPES = 9   # 8 is retired (terminal-hit compaction, removed): do not reuse
 OPT_BUILD_THREADS, OPT_STACK_LIMIT = 10, 11
 COMM_ID_BYTES = 128
 KERNEL_NAMES = ["raygen", "extend", "shade", "shadow", "splat"]
 ORC_OPT_THREADS = 100
 (KAT_PCG32, KAT_LATTICE, KAT_CAMERA, KAT_RANDOM_COS, KAT_RANDOM_PHONG, KAT_PHONG_EVAL, KAT_MERL_EVAL,
- KAT_FAST_EXP, KAT_FAST_NORMALIZE, KAT_RANDOM_PER_PIXEL, KAT_FILTER_RATIO, KAT_MERL_INDEX, KAT_NODE_HALF) = range(1, 14)
+ KAT_FAST_EXP, KAT_FAST_NORMALIZE, KAT_RANDOM_PER_PIXEL, KAT_FILTER_RATIO, KAT_MERL_INDEX) = range(1, 13)
+# KAT 13 is retired (the half-factor node test, removed): do not reuse
 KAT_SHAPES = {  # which -> (n_in, n_out)
     KAT_PCG32: (2, 4), KAT_LATTICE: (1, 2), KAT_CAMERA: (6, 6), KAT_RANDOM_COS: (5, 3),
     KAT_RANDOM_PHONG: (6, 3), KAT_PHONG_EVAL: (18, 3), KAT_MERL_EVAL: (9, 3), KAT_FAST_EXP: (1, 1),
-    KAT_FAST_NORMALIZE: (3, 3), KAT_RANDOM_PER_PIXEL: (1, 2), KAT_FILTER_RATIO: (3, 1), KAT_MERL_INDEX: (6, 2), KAT_NODE_HALF: (8, 2),
+    KAT_FAST_NORMALIZE: (3, 3), KAT_RANDOM_PER_PIXEL: (1, 2), KAT_FILTER_RATIO: (3, 1), KAT_MERL_INDEX: (6, 2),
 }
 
 _fp = C.POINTER(C.c_float)

@@ -3,8 +3,8 @@
 // Replaces TriMesh::build_bvh / build_bvh_recur (reference TriangleMesh.cpp:878-885, 1029-1130: one
 // binary BVH per mesh, 16 candidate planes on the longest centroid axis, <=4 triangles per leaf).
 // Here: one BVH over ALL meshes' triangles baked to world space (scenes are static during a render,
-// SURVEY §3.4), binned SAH on all three axes (16 bins), leaves of <=3 triangles, then a greedy
-// surface-area collapse to 8-wide nodes, octant-ordered child slots and 8-bit quantised child boxes.
+// SURVEY §3.4), binned SAH on all three axes (16 bins) down to single triangles, then the cost-optimal
+// collapse to 8-wide nodes with leaves of <=3 triangles, octant-ordered child slots and 8-bit quantised child boxes.
 // The result is only an acceleration structure: which triangle a ray hits is decided by the triangle
 // test, so parity with the reference does not depend on reproducing its tree.
 #include "ptb_host.h"
@@ -12,7 +12,6 @@
 #include <algorithm>
 #include <atomic>
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
 
 namespace ptb {
@@ -42,7 +41,7 @@ struct BNode {   // binary node: leaf iff count > 0
 //   C(n,1) = min( leaf: A(n) * P(n) * c_prim  [P(n) <= 3],  wide node: A(n) * c_node + D(n,8) )
 //   C(n,i) = min( D(n,i), C(n,i-1) )                      the subtree of n as a forest of at most i children of a wide node
 //   D(n,j) = min over 0 < k < j of C(left,k) + C(right,j-k)
-// The greedy collapse (open the child of largest area until 8) leaves the lowest wide nodes with 2-3 small leaves: 275k nodes of
+// A greedy collapse (open the child of largest area until 8) leaves the lowest wide nodes with 2-3 small leaves: 275k nodes of
 // 2.8 children on average for the 1M-triangle mesh, hence one node visit per level of a deep tree; the optimal collapse decides
 // leaf sizes and node shapes together.
 struct Collapse {
@@ -58,8 +57,7 @@ struct Builder {
     std::vector<float> pcen;       // 3 per prim
     std::vector<uint32_t> idx;
     std::vector<BNode> nodes;
-    std::vector<Collapse> dp;      // empty: greedy collapse
-    int max_leaf = 3;
+    std::vector<Collapse> dp;
     std::atomic<int64_t> n_nodes{0};
     void solve(int64_t node);
 
@@ -68,15 +66,9 @@ struct Builder {
     void build(int64_t node, int64_t b, int64_t e, int depth);
 };
 
-constexpr int NBINS_MAX = 64;
 constexpr int64_t PAR_NODE = 1 << 18;      // nodes with at least this many primitives run their passes in chunks (tasks)
-// builder knobs (environment overrides are for experiments only; the defaults are what ships)
-static float env_f(const char* n, float d) { const char* v = getenv(n); return v ? (float)atof(v) : d; }
-static const float C_TRAV = env_f("PTB_BVH_CTRAV", 0.25f);   // binary nodes mostly vanish in the collapse
-static const int MAX_LEAF = (int)env_f("PTB_BVH_MAXLEAF", 3.f);
-static const int NBINS = std::min(NBINS_MAX, std::max(4, (int)env_f("PTB_BVH_NBINS", 16.f)));   // SAH bins per axis
-static const int COLLAPSE_DP = (int)env_f("PTB_BVH_COLLAPSE_DP", 1.f);   // 0: greedy surface-area collapse of a binary tree with <= 3-triangle leaves
-static const float C_NODE = env_f("PTB_BVH_CNODE", 1.f), C_PRIM = env_f("PTB_BVH_CPRIM", 0.5f);   // measured (profiles/r01m): 0.5 beats 0.3 and 0.15 on C2 and C3
+constexpr int NBINS = 16;                  // SAH bins per axis
+constexpr float C_NODE = 1.f, C_PRIM = 0.5f;   // measured (profiles/r01m): 0.5 beats 0.3 and 0.15 on C2 and C3
 
 void Builder::solve(int64_t node) {
     const BNode& nd = nodes[node];
@@ -133,15 +125,17 @@ void Builder::build(int64_t node, int64_t b, int64_t e, int depth) {
     for (int64_t i = b; i < e; i++) { box.grow(pbox[idx[i]]); cb.grow(&pcen[3 * (size_t)idx[i]]); }
     nd.box = box;
     nd.sfirst = (int32_t)b; nd.scount = (int32_t)cnt;
-    const int MAX_LEAF = max_leaf;
-    auto make_leaf = [&]() { nd.left = nd.right = -1; nd.first = (int32_t)b; nd.count = (int32_t)cnt; if (!dp.empty()) solve(node); };
-    if (cnt == 1) { make_leaf(); return; }
+    if (cnt == 1) {   // the collapse forms the leaves itself, from single triangles
+        nd.left = nd.right = -1; nd.first = (int32_t)b; nd.count = 1;
+        solve(node);
+        return;
+    }
 
     // binned SAH over the three axes: ONE pass over the node's primitives fills the bins of all three (the boxes are reached through
     // the index array, a cache miss each: three passes were three misses per primitive)
     float best_cost = INFINITY;
     int best_axis = -1, best_bin = -1;
-    struct Bins { Box bb[3][NBINS_MAX]; int64_t bc[3][NBINS_MAX]; };
+    struct Bins { Box bb[3][NBINS]; int64_t bc[3][NBINS]; };
     float lo3[3], scale3[3];
     bool use[3];
     for (int ax = 0; ax < 3; ax++) {
@@ -163,7 +157,7 @@ void Builder::build(int64_t node, int64_t b, int64_t e, int depth) {
             }
         }
     };
-    Bins bins;      // 6 KB of stack per level of the recursion
+    Bins bins;      // 1.5 KB of stack per level of the recursion
     if (n_chunks > 1) {
         std::vector<Bins> part((size_t)n_chunks);
         for (int c = 0; c < n_chunks; c++) {
@@ -178,7 +172,7 @@ void Builder::build(int64_t node, int64_t b, int64_t e, int depth) {
     for (int ax = 0; ax < 3; ax++) {
         if (!use[ax]) continue;
         const Box* bb = bins.bb[ax]; const int64_t* bc = bins.bc[ax];
-        float ra[NBINS_MAX]; int64_t rc[NBINS_MAX];
+        float ra[NBINS]; int64_t rc[NBINS];
         Box acc; acc.reset(); int64_t c = 0;
         for (int k = NBINS - 1; k > 0; k--) { acc.grow(bb[k]); c += bc[k]; ra[k] = acc.area(); rc[k] = c; }
         acc.reset(); c = 0;
@@ -191,13 +185,8 @@ void Builder::build(int64_t node, int64_t b, int64_t e, int depth) {
     }
     int64_t mid;
     if (best_axis < 0) {
-        if (cnt <= MAX_LEAF) { make_leaf(); return; }
         mid = b + cnt / 2;  // coincident centroids: split by index
     } else {
-        if (cnt <= MAX_LEAF) {
-            const float A = box.area();
-            if (!(C_TRAV * A + best_cost < (float)cnt * A)) { make_leaf(); return; }
-        }
         const float lo = cb.lo[best_axis], scale = NBINS / (cb.hi[best_axis] - cb.lo[best_axis]);
         auto it = std::partition(idx.begin() + b, idx.begin() + e, [&](uint32_t p) {
             int k = (int)((pcen[3 * (size_t)p + best_axis] - lo) * scale);
@@ -219,13 +208,13 @@ void Builder::build(int64_t node, int64_t b, int64_t e, int depth) {
         build(c0, b, mid, depth + 1);
         build(c0 + 1, mid, e, depth + 1);
     }
-    if (!dp.empty()) solve(node);
+    solve(node);
 }
 
 inline uint8_t exponent_byte(float extent, float coord_slack, int e_lo) {
     // smallest e with extent + 2 * slack <= 255 * 2^e, where slack = 4e-3 cells + coord_slack is what the quantisation adds on either
-    // side (the 1.0001 pays for the cell-relative part: 255 / 1.0001 + 0.008 < 255).  Never below e_lo: the cell must have a half
-    // exponent byte (ptb_bvh8.h half_exp_byte); a flat or tiny box simply gets cells coarser than it needs.
+    // side (the 1.0001 pays for the cell-relative part: 255 / 1.0001 + 0.008 < 255).  Never below e_lo (Bvh8Stats::e_floor): a flat or
+    // tiny box simply gets cells coarser than it needs.
     const double x = ((double)extent + 2.0 * (double)coord_slack) * 1.0001 / 255.0;
     int e = x > 0 ? (int)std::ceil(std::log2(x)) : e_lo;
     if (e < e_lo) e = e_lo;
@@ -255,8 +244,7 @@ void build_bvh8(const float* verts9, int64_t n_tri, std::vector<Node8>& out_node
         B.idx[i] = (uint32_t)i;
     }
     B.nodes.resize(2 * (size_t)n_tri + 2);
-    B.max_leaf = COLLAPSE_DP ? 1 : MAX_LEAF;          // the optimal collapse forms the leaves itself, from single triangles
-    if (COLLAPSE_DP) B.dp.resize(B.nodes.size());
+    B.dp.resize(B.nodes.size());
     B.n_nodes = 1;
 #pragma omp parallel
     {
@@ -282,14 +270,14 @@ void build_bvh8(const float* verts9, int64_t n_tri, std::vector<Node8>& out_node
         root.bnode = 0; root.wide = 0;
         level.push_back(root);
     }
-    {   // the half grid of the scene (ptb_bvh8.h half_grid_c): fixed by the root box, whose cells are the largest of the tree
+    {   // the finest cell: 2^-25 of the root's, whose cells are the largest of the tree
         const Box& rb = B.nodes[0].box;
         int e_root = -100;
         for (int k = 0; k < 3; k++)
             e_root = std::max(e_root, (int)exponent_byte(rb.hi[k] - rb.lo[k], node_coord_slack(rb.lo[k], rb.hi[k]), -100) - 127);
-        stats.half_c = half_grid_c(e_root);
+        stats.e_floor = e_root - 25;
     }
-    const int e_lo = PTB_HALF_E_LO - stats.half_c;
+    const int e_lo = stats.e_floor;
     uint64_t tri_running = 0;
     int64_t leaves = 0;
     for (int depth = 1; !level.empty(); depth++) {
@@ -302,40 +290,22 @@ void build_bvh8(const float* verts9, int64_t n_tri, std::vector<Node8>& out_node
             Item& w = level[(size_t)it_];
             int32_t* ch = w.ch; bool* ch_leaf = w.ch_leaf; int nc = 0;
             const BNode& root = B.nodes[w.bnode];
-            if (!B.dp.empty()) {
-                // children of the wide node rooted at w.bnode: follow the recorded decisions
-                struct It { int32_t n; int i; };
-                It st[16]; int sp = 0;
-                if (root.count > 0 || root.scount <= 3) { ch[nc] = w.bnode; ch_leaf[nc++] = true; }   // a tiny mesh: the root holds one leaf
-                else {
-                    const int k = B.dp[w.bnode].k8;
-                    st[sp++] = {root.right, 8 - k}; st[sp++] = {root.left, k};
-                }
-                while (sp > 0) {
-                    const It it = st[--sp];
-                    const BNode& m = B.nodes[it.n];
-                    if (m.count > 0) { ch[nc] = it.n; ch_leaf[nc++] = true; continue; }
-                    if (it.i == 1) { ch[nc] = it.n; ch_leaf[nc++] = B.dp[it.n].d[0] == 0; continue; }
-                    const int k = B.dp[it.n].d[it.i - 1];
-                    if (k == 0) st[sp++] = {it.n, it.i - 1};
-                    else { st[sp++] = {m.right, it.i - k}; st[sp++] = {m.left, k}; }
-                }
-            } else {
-                if (root.count > 0) ch[nc++] = w.bnode;           // a leaf root: one leaf child
-                else { ch[nc++] = root.left; ch[nc++] = root.right; }
-                while (nc < 8) {
-                    int best = -1; float best_area = -1.f;
-                    for (int i = 0; i < nc; i++) {
-                        const BNode& c = B.nodes[ch[i]];
-                        if (c.count > 0) continue;
-                        const float a = c.box.area();
-                        if (a > best_area) { best_area = a; best = i; }
-                    }
-                    if (best < 0) break;
-                    const BNode& c = B.nodes[ch[best]];
-                    ch[best] = c.left; ch[nc++] = c.right;
-                }
-                for (int i = 0; i < nc; i++) ch_leaf[i] = B.nodes[ch[i]].count > 0;
+            // children of the wide node rooted at w.bnode: follow the recorded decisions
+            struct It { int32_t n; int i; };
+            It st[16]; int sp = 0;
+            if (root.count > 0 || root.scount <= 3) { ch[nc] = w.bnode; ch_leaf[nc++] = true; }   // a tiny mesh: the root holds one leaf
+            else {
+                const int k = B.dp[w.bnode].k8;
+                st[sp++] = {root.right, 8 - k}; st[sp++] = {root.left, k};
+            }
+            while (sp > 0) {
+                const It it = st[--sp];
+                const BNode& m = B.nodes[it.n];
+                if (m.count > 0) { ch[nc] = it.n; ch_leaf[nc++] = true; continue; }
+                if (it.i == 1) { ch[nc] = it.n; ch_leaf[nc++] = B.dp[it.n].d[0] == 0; continue; }
+                const int k = B.dp[it.n].d[it.i - 1];
+                if (k == 0) st[sp++] = {it.n, it.i - 1};
+                else { st[sp++] = {m.right, it.i - k}; st[sp++] = {m.left, k}; }
             }
             w.nc = nc;
             Box nb; nb.reset();
@@ -397,10 +367,9 @@ void build_bvh8(const float* verts9, int64_t n_tri, std::vector<Node8>& out_node
             nd.ex = exponent_byte(nb.hi[0] - nb.lo[0], node_coord_slack(nb.lo[0], nb.hi[0]), e_lo);
             nd.ey = exponent_byte(nb.hi[1] - nb.lo[1], node_coord_slack(nb.lo[1], nb.hi[1]), e_lo);
             nd.ez = exponent_byte(nb.hi[2] - nb.lo[2], node_coord_slack(nb.lo[2], nb.hi[2]), e_lo);
-            nd.hx = half_exp_byte((int)nd.ex - 127, stats.half_c); nd.hy = half_exp_byte((int)nd.ey - 127, stats.half_c); nd.hz = half_exp_byte((int)nd.ez - 127, stats.half_c);
             const float cell[3] = {std::ldexp(1.f, (int)nd.ex - 127), std::ldexp(1.f, (int)nd.ey - 127), std::ldexp(1.f, (int)nd.ez - 127)};
-            // conservative slack: 4e-3 of a cell (covers the rounding of the traversal's folded plane bias in either form of
-            // ptb_bvh8.h planes4) plus a few ulps of the coordinate
+            // conservative slack: 4e-3 of a cell (covers the rounding of the traversal's folded plane bias, ptb_bvh8.h planes4) plus a
+            // few ulps of the coordinate
             float eps[3], p[3];
             for (int k = 0; k < 3; k++) {
                 eps[k] = cell[k] * 4e-3f + node_coord_slack(nb.lo[k], nb.hi[k]);

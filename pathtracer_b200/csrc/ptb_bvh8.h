@@ -13,11 +13,7 @@
 //         20-23  tri_base     index of the node's first triangle (leaf children contiguous)
 //         24-26  valid24  bit 3*s + k set <=> slot s is a leaf with more than k triangles (at most 3 per leaf); the node's
 //                         triangles are stored compactly in this bit order: index = tri_base + popcount(valid24 below the bit)
-//            27  reserved (0)
-//         28-30  hx hy hz  the same cell sizes as the exponent byte of an IEEE half: (25 + e + half_c) << 2, so that one PRMT puts a
-//                          quantised plane q under it and gets the half (1024 + q) * 2^(e + half_c) (node_hitmask_h; half_c is chosen
-//                          per scene, half_grid_c)
-//            31  reserved (0)
+//         27-31  reserved (0)
 //         32-79  qlo_x[8] qlo_y[8] qlo_z[8] qhi_x[8] qhi_y[8] qhi_z[8]
 //
 // Triangles are stored in leaf order as 3 x float4 = 48 bytes {v0, e1 = v1-v0, e2 = v2-v0}; v0.w carries
@@ -38,38 +34,16 @@ struct alignas(16) Node8 {
     uint8_t ex, ey, ez, imask;
     uint32_t child_base, tri_base;
     uint8_t valid24[3];   // see the layout above
-    uint8_t reserved0;
-    uint8_t hx, hy, hz;   // half exponent bytes, see the layout above
-    uint8_t reserved1;
+    uint8_t reserved[5];  // bytes 27-31, 0
     uint8_t qlox[8], qloy[8], qloz[8], qhix[8], qhiy[8], qhiz[8];
 };
 static_assert(sizeof(Node8) == 80, "Node8 must be 80 bytes");
 
-#if !defined(PTB_EDGE_EPS_ON)
-#define PTB_EDGE_EPS_ON 1      /* 0: the fast triangle test decides everything (A/B: profiles/r02d_ab_exact_edges.txt) */
-#endif
 #define PTB_TRI_FLAG_ALPHA 1u  /* tri.w0 bit: this triangle's group has an alpha map that can reject */
 #define PTB_TRI_FLAG_DISC 4u   /* tri.w0 bit: the triangle covers a disc of a point set (disc_cover_triangle, ptb_scene.h); tri_exact runs the disc test */
 #define PTB_TRI_T_CUT (1.f - 1e-4f)   /* tri.w2 (e2.w) of an ordinary triangle: the fast test drops a hit when t * w2 >= t_best; 0 = never (volume covers, ptb_scene.h) */
 #define PTB_TRI_FLAG_GHOST 2u  /* tri.w0 bit: the triangle belongs to a ghost object; shadow rays pass through it (Geometry.cpp:722) */
 
-// ---- the half grid ---------------------------------------------------------------------------------------------------------------
-// k_trace evaluates the 48 plane distances of a node with the mixed-precision FMA of sm_100 (fma.rn.f32.f16 = FHFMA: two half
-// factors, float addend and result): t = half(1024 + q) * 2^(e + c)  x  half(1 / d * 2^-c)  +  float bias.  The first factor is the
-// plane byte under a per-node exponent byte (hx, hy, hz of Node8), exact; the second is the ray's inverse direction rounded DOWN for
-// entry planes and UP for exit planes, so that the box a ray sees is never smaller than the quantised box (q >= 0); c = half_c is one
-// constant per scene that puts the cell sizes 2^e of the whole tree into the exponent range a half has next to a 11-bit integer.
-// MEASURED AND NOT KEPT (profiles/r02n-r_*): 32 fewer instructions per node step (48 HADD2.F32 + 48 FFMA become 54 FHFMA), yet k_trace is
-// 3 % SLOWER at equal occupancy (C2 43.1 vs 41.8 ms, C3 115.6 vs 112.5 ms per 134 M samples) and 4 % slower at the 64 registers the
-// kernel then takes: FHFMA issues at the rate of one FFMA when alone (scripts/ubench/pipe_rates.cu: 0.60 vs 0.64 per cycle and
-// scheduler) but not next to the min / max / select stream of the node step.  -DPTB_NODE_HALF=1 builds it; the float test is the default.
-#if !defined(PTB_NODE_HALF)
-#define PTB_NODE_HALF 0
-#endif
-#define PTB_HALF_E_HI 5       /* (1024 + 255) * 2^5 = 40928 < 65504 */
-#define PTB_HALF_E_LO (-24)   /* exponent field 1: the smallest normal half under 1024 + q */
-PTB_HD int half_grid_c(int e_root) { return 1 - e_root; }   // root cells (the largest) at 2^1: a re-posed scene may grow 16x before a refit has to refuse
-PTB_HD uint8_t half_exp_byte(int e, int c) { return (uint8_t)((25 + e + c) << 2); }
 // what the quantisation adds to a node box next to the cell-relative part: a few ulps of the coordinates
 PTB_HD float node_coord_slack(float lo, float hi) { return 4e-7f * fmaxf(fabsf(lo), fabsf(hi)); }
 
@@ -125,12 +99,7 @@ PTB_HD bool alpha_rejects(const AlphaCtx* ctx, int prim, float b1, float b2);
 // Triangle::intersection (TriangleMesh.h:82-104) in the reference's own arithmetic: object-space ray, plane + Gram barycentrics, every
 // operation rounded separately (ptb_scene.h).  Decides the hits the fast test below cannot call: rays within PTB_EDGE_EPS of an edge.
 PTB_HD bool tri_exact_available(const AlphaCtx* ctx);
-#if defined(PTB_EXACT_INLINE)
-#define PTB_EXACT_LINKAGE PTB_HD
-#else
-#define PTB_EXACT_LINKAGE PTB_HD_NOINLINE     /* out of line: the hot loop keeps its registers */
-#endif
-PTB_EXACT_LINKAGE bool tri_exact(const AlphaCtx* ctx, int prim, V3 o, V3 d, float tbest, float& t, float& b1, float& b2);
+PTB_HD_NOINLINE bool tri_exact(const AlphaCtx* ctx, int prim, V3 o, V3 d, float tbest, float& t, float& b1, float& b2);   // out of line: the hot loop keeps its registers
 
 // Tests the 8 children of `n` against the ray; returns the hit mask in SLOT order: bit 24 + s = the internal child in slot s,
 // bits 3s..3s+2 = the triangles of the leaf in slot s (only bits that exist: valid24 / imask).
@@ -140,8 +109,7 @@ PTB_EXACT_LINKAGE bool tri_exact(const AlphaCtx* ctx, int prim, V3 o, V3 d, floa
 // into the FFMA constant.
 // Both the fma pipe (FFMA, HADD2, IMAD) and the alu pipe (PRMT, FMNMX, LOP3, SHF, SEL, ISETP) issue one warp instruction
 // every 2 cycles per SM sub-partition; the node test is bound by the alu pipe (about 116 alu vs 96 fma instructions per node).
-#if !defined(PTB_PLANES_PRMT32)
-// default: one PRMT (alu) builds a half2 {1024+q0, 1024+q1} (0x6400 | q) for TWO planes and HADD2.F32 (fma pipe) widens each;
+// One PRMT (alu) builds a half2 {1024+q0, 1024+q1} (0x6400 | q) for TWO planes and HADD2.F32 (fma pipe) widens each;
 // the bias folds into the FFMA constant: t = (1024+q)*ad + (bo - 1024*ad), at most 2^-24 * 1024 = 6e-5 of a cell of rounding.
 #define PTB_PLANE_BIAS 1024.f
 __device__ __forceinline__ void planes4(uint32_t w, float ad, float bo, float& t0, float& t1, float& t2, float& t3) {
@@ -150,18 +118,6 @@ __device__ __forceinline__ void planes4(uint32_t w, float ad, float bo, float& t
     t0 = fmaf(__low2float(a), ad, bo); t1 = fmaf(__high2float(a), ad, bo);
     t2 = fmaf(__low2float(b), ad, bo); t3 = fmaf(__high2float(b), ad, bo);
 }
-#else
-// measured alternative (r01e, 1.5 % SLOWER on C2/C3): one PRMT per plane drops the byte into bits 8..15 of 0x47000000 = the
-// float 32768 + q, no conversion instruction: 23 fewer instructions per node, but all 48 byte moves land on the alu pipe,
-// which is the busier one.  Fold rounding 2^-24 * 32768 = 2e-3 of a cell (builder slack: 4e-3).
-#define PTB_PLANE_BIAS 32768.f
-__device__ __forceinline__ void planes4(uint32_t w, float ad, float bo, float& t0, float& t1, float& t2, float& t3) {
-    t0 = fmaf(__uint_as_float(__byte_perm(w, 0x47000000u, 0x7404)), ad, bo);
-    t1 = fmaf(__uint_as_float(__byte_perm(w, 0x47000000u, 0x7414)), ad, bo);
-    t2 = fmaf(__uint_as_float(__byte_perm(w, 0x47000000u, 0x7424)), ad, bo);
-    t3 = fmaf(__uint_as_float(__byte_perm(w, 0x47000000u, 0x7434)), ad, bo);
-}
-#endif
 __device__ __forceinline__ uint32_t node_hitmask(const F4& n0, const F4& n1, const F4& n2, const F4& n3, const F4& n4, const RayPrep& r, float tmax) {
     const uint32_t e_imask = f2u(n0.w);
     const float sx = u2f(((e_imask >> 0) & 0xffu) << 23), sy = u2f(((e_imask >> 8) & 0xffu) << 23), sz = u2f(((e_imask >> 16) & 0xffu) << 23);
@@ -172,11 +128,7 @@ __device__ __forceinline__ uint32_t node_hitmask(const F4& n0, const F4& n1, con
     // The mask is built in SLOT order with immediates (slot s: its three triangle bits and its internal-child bit) and cut down to
     // what exists with one AND; the octant order is applied when a child is picked (pick_slot).  The per-child byte extracts and
     // variable shifts of a traversal-ordered mask were a quarter of the node step's instructions.
-#if defined(PTB_MASK_FMA)
-    uint32_t hitmask = 0xffffffffu;     // A/B: the mask accumulated on the fma pipe (FADD, IMAD.HI, IMAD per child instead of FSETP + predicated add)
-#else
     uint32_t hitmask = 0;
-#endif
 #pragma unroll
     for (int half = 0; half < 2; half++) {
         const uint32_t lox = f2u(half ? n2.y : n2.x), loy = f2u(half ? n2.w : n2.z), loz = f2u(half ? n3.y : n3.x);
@@ -193,13 +145,7 @@ __device__ __forceinline__ uint32_t node_hitmask(const F4& n0, const F4& n1, con
             const float tn = fmaxf(fmaxf(tnx[j], tny[j]), fmaxf(tnz[j], 0.f));
             const float tf = fminf(fminf(tfx[j], tfy[j]), fminf(tfz[j], tmax));
             const int s = 4 * half + j;
-#if defined(PTB_MASK_FMA)
-            // tn <= tf  <=>  the sign of tf - tn is clear (both finite or tf = +inf; never NaN: the min / max drop NaNs and 0, tmax are numbers)
-            const int32_t miss = __mulhi((int32_t)f2u(tf - tn), 2);                 // 0 or -1, IMAD.HI
-            hitmask += (uint32_t)miss * ((7u << (3 * s)) | (1u << (24 + s)));        // IMAD: a missed child takes its bits out of the full mask
-#else
             if (tn <= tf) hitmask |= (7u << (3 * s)) | (1u << (24 + s));
-#endif
         }
     }
     return hitmask & ((e_imask & 0xff000000u) | (f2u(n1.z) & 0x00ffffffu));
@@ -240,115 +186,6 @@ inline uint32_t node_hitmask(const F4& n0, const F4& n1, const F4& n2, const F4&
 }
 #endif
 
-#if defined(__CUDACC__)
-// ---- the same test with half factors (see "the half grid" above): 48 FHFMA instead of 48 HADD2.F32 + 48 FFMA -----------------------
-// d = a * b + c, a and b halves picked from half2 registers ("l_" / "h_" of the first, "m_" / "n_" of the second), c and d floats
-#define PTB_FHFMA(d, a2, asel, b2, bsel, c) \
-    asm("{.reg .f16 l_, h_, m_, n_; mov.b32 {l_, h_}, %1; mov.b32 {m_, n_}, %2; fma.rn.f32.f16 %0, " asel ", " bsel ", %3;}" : "=f"(d) : "r"(a2), "r"(b2), "f"(c))
-// The ray's slopes on the half grid: {round-down, round-up}(1 / d * 2^-half_c) as a half2 per axis.  A component too steep for a half
-// (|1 / d| * 2^-half_c > 65504: the ray runs along the planes of that axis) becomes the largest finite half on the side that has to stay
-// below and an infinity on the other; the infinite side turns its plane distances into NaN (inf - inf), which the min / max of the
-// interval test drop (IEEE minNum / maxNum): that side simply does not constrain the interval any more.
-struct RaySlopes { uint32_t x, y, z; };
-__device__ __forceinline__ uint32_t half_slope2(float idir, float scale) {
-    const float v = idir * scale;
-#if defined(PTB_SLOPES_CVT_DIRECTED)      // A/B: the directed conversions themselves (F2F.F16.F32.RM / .RP)
-    uint16_t dn, up;
-    asm("cvt.rm.f16.f32 %0, %1;" : "=h"(dn) : "f"(v));
-    asm("cvt.rp.f16.f32 %0, %1;" : "=h"(up) : "f"(v));
-    return (uint32_t)dn | ((uint32_t)up << 16);
-#else
-    // round to nearest, then step to the neighbour on the side the rounding left: halves of one sign are ordered like their bit patterns
-    const __half h = __float2half_rn(v);
-    const float back = __half2float(h);
-    const uint32_t b = (uint32_t)__half_as_ushort(h);
-    const uint32_t away = (b & 0x8000u) ? 0xffffffffu : 1u;                  // bit-pattern step that moves a half towards +inf ... (negative: b - 1)
-    const uint32_t dn = (back > v) ? b - away : b;                             // ... and towards -inf.  +-0 cannot occur (|v| >= 2^-half_c), an overflow gives
-    const uint32_t up = (back < v) ? b + away : b;                             // +-inf, whose inner neighbour is the largest finite half: what the directed conversion returns
-    return (dn & 0xffffu) | (up << 16);
-#endif
-}
-#define PTB_RAY_STEEP 8u     /* bit of RayPrep::oct_inv4: some component of 1 / d does not fit a half on this scene's grid (or is NaN) */
-__device__ __forceinline__ RaySlopes ray_slopes(RayPrep& r, int half_c) {
-    const float scale = u2f((uint32_t)(127 - half_c) << 23);
-    RaySlopes s;
-    s.x = half_slope2(r.idir.x, scale); s.y = half_slope2(r.idir.y, scale); s.z = half_slope2(r.idir.z, scale);
-    // A ray that runs along the planes of an axis (|1 / d| * 2^-half_c beyond the largest half) would lose that axis' constraint in
-    // the half form: correct, but such a ray then visits every box above and below it, and one ray that takes milliseconds holds a
-    // whole persistent launch (measured, profiles/r02n_ab_node_half.txt).  These rays (a few in a million) and NaN rays, which
-    // must fail every test, take the float node test.
-    const float lim = 65504.f / scale;
-    const float osum = r.o.x + r.o.y + r.o.z;
-    if (!(fabsf(r.idir.x) <= lim && fabsf(r.idir.y) <= lim && fabsf(r.idir.z) <= lim && osum == osum)) r.oct_inv4 |= PTB_RAY_STEEP;   // (a NaN fails every comparison)
-    return s;
-}
-// four planes of one axis: bytes of `w` under the node's half exponent byte (byte AXIS of `hw`), times the entry (FAR = false: rounded
-// down) or exit slope, plus the folded bias
-template <int AXIS, bool FAR>
-__device__ __forceinline__ void planes4h(uint32_t w, uint32_t hw, uint32_t slope2, float bo, float& t0, float& t1, float& t2, float& t3) {
-    const uint32_t h01 = __byte_perm(w, hw, 0x4040u + 0x1010u * AXIS + 0x0100u), h23 = __byte_perm(w, hw, 0x4040u + 0x1010u * AXIS + 0x0302u);
-    if (FAR) {
-        PTB_FHFMA(t0, h01, "l_", slope2, "n_", bo); PTB_FHFMA(t1, h01, "h_", slope2, "n_", bo);
-        PTB_FHFMA(t2, h23, "l_", slope2, "n_", bo); PTB_FHFMA(t3, h23, "h_", slope2, "n_", bo);
-    } else {
-        PTB_FHFMA(t0, h01, "l_", slope2, "m_", bo); PTB_FHFMA(t1, h01, "h_", slope2, "m_", bo);
-        PTB_FHFMA(t2, h23, "l_", slope2, "m_", bo); PTB_FHFMA(t3, h23, "h_", slope2, "m_", bo);
-    }
-}
-// bias of an axis: t(q) = (1024 + q) * A * s + (B - 1024 * A * s) with A = 2^(e + c) (the half under the exponent byte with q = 0 is
-// 1024 * A), s the half slope and B = (p - o) / d the distance of the grid origin, in float as in the float form
-template <int AXIS>
-__device__ __forceinline__ void bias2h(uint32_t hw, uint32_t slope2, float B, float& bo_near, float& bo_far) {
-    const uint32_t a0 = __byte_perm(hw, 0u, 0x4404u + 0x0010u * AXIS);     // {1024 * A, 0}
-    const uint32_t neg = slope2 ^ 0x80008000u;
-    PTB_FHFMA(bo_near, a0, "l_", neg, "m_", B);
-    PTB_FHFMA(bo_far, a0, "l_", neg, "n_", B);
-}
-__device__ __forceinline__ uint32_t node_hitmask_h(const F4& n0, const F4& n1, const F4& n2, const F4& n3, const F4& n4, const RayPrep& r, const RaySlopes& rs, float tmax) {
-    const uint32_t hw = f2u(n1.w);
-    float bnx, bfx, bny, bfy, bnz, bfz;
-    bias2h<0>(hw, rs.x, (n0.x - r.o.x) * r.idir.x, bnx, bfx);
-    bias2h<1>(hw, rs.y, (n0.y - r.o.y) * r.idir.y, bny, bfy);
-    bias2h<2>(hw, rs.z, (n0.z - r.o.z) * r.idir.z, bnz, bfz);
-    const bool negx = r.d.x < 0, negy = r.d.y < 0, negz = r.d.z < 0;
-    uint32_t hitmask = 0;
-#pragma unroll
-    for (int half = 0; half < 2; half++) {
-        const uint32_t lox = f2u(half ? n2.y : n2.x), loy = f2u(half ? n2.w : n2.z), loz = f2u(half ? n3.y : n3.x);
-        const uint32_t hix = f2u(half ? n3.w : n3.z), hiy = f2u(half ? n4.y : n4.x), hiz = f2u(half ? n4.w : n4.z);
-        float tnx[4], tny[4], tnz[4], tfx[4], tfy[4], tfz[4];
-        planes4h<0, false>(negx ? hix : lox, hw, rs.x, bnx, tnx[0], tnx[1], tnx[2], tnx[3]);
-        planes4h<0, true>(negx ? lox : hix, hw, rs.x, bfx, tfx[0], tfx[1], tfx[2], tfx[3]);
-        planes4h<1, false>(negy ? hiy : loy, hw, rs.y, bny, tny[0], tny[1], tny[2], tny[3]);
-        planes4h<1, true>(negy ? loy : hiy, hw, rs.y, bfy, tfy[0], tfy[1], tfy[2], tfy[3]);
-        planes4h<2, false>(negz ? hiz : loz, hw, rs.z, bnz, tnz[0], tnz[1], tnz[2], tnz[3]);
-        planes4h<2, true>(negz ? loz : hiz, hw, rs.z, bfz, tfz[0], tfz[1], tfz[2], tfz[3]);
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            const float tn = fmaxf(fmaxf(tnx[j], tny[j]), fmaxf(tnz[j], 0.f));
-            const float tf = fminf(fminf(tfx[j], tfy[j]), fminf(tfz[j], tmax));
-            const int s = 4 * half + j;
-            if (tn <= tf) hitmask |= (7u << (3 * s)) | (1u << (24 + s));
-        }
-    }
-    return hitmask & ((f2u(n0.w) & 0xff000000u) | (f2u(n1.z) & 0x00ffffffu));
-}
-// the node test of k_trace
-#if defined(PTB_STEEP_NOINLINE)
-__device__ __noinline__ uint32_t node_hitmask_steep(F4 n0, F4 n1, F4 n2, F4 n3, F4 n4, V3 o, V3 d, V3 idir, float tmax) {
-    RayPrep r; r.o = o; r.d = d; r.idir = idir; r.oct_inv4 = 0;
-    return node_hitmask(n0, n1, n2, n3, n4, r, tmax);
-}
-#endif
-__device__ __forceinline__ uint32_t node_hitmask_k(const F4& n0, const F4& n1, const F4& n2, const F4& n3, const F4& n4, const RayPrep& r, const RaySlopes& rs, float tmax) {
-#if defined(PTB_STEEP_NOINLINE)
-    if (r.oct_inv4 & PTB_RAY_STEEP) return node_hitmask_steep(n0, n1, n2, n3, n4, r.o, r.d, r.idir, tmax);
-#else
-    if (r.oct_inv4 & PTB_RAY_STEEP) return node_hitmask(n0, n1, n2, n3, n4, r, tmax);
-#endif
-    return node_hitmask_h(n0, n1, n2, n3, n4, r, rs, tmax);
-}
-#endif
 
 // Barycentric band around the triangle's edges inside which the fast test defers to tri_exact.  The fast test works on world-space
 // float vertices, the reference on object-space ones: their barycentrics differ by up to a few 1e-5 (coordinates of magnitude 50
@@ -363,7 +200,7 @@ PTB_HD bool tri_test(const F4& a, const F4& b, const F4& c, const RayPrep& r, fl
     const V3 v0 = v3(a.x, a.y, a.z), e1 = v3(b.x, b.y, b.z), e2 = v3(c.x, c.y, c.z);
     const V3 pvec = cross(r.d, e2);
     const float det = dot(e1, pvec);
-#if defined(__CUDA_ARCH__) && !defined(PTB_TRI_RCP_EXACT)
+#if defined(__CUDA_ARCH__)
     // one MUFU.RCP instead of the IEEE division sequence (9 instructions + a slow path): the signs of u, v, t and hence every
     // accept test but the last ulp of `1-u-v >= 0` and `t < tbest` are unaffected; |det| below 1.2e-38 flushes to a miss.
     float inv;
@@ -378,7 +215,6 @@ PTB_HD bool tri_test(const F4& a, const F4& b, const F4& c, const RayPrep& r, fl
     const float tt = dot(e2, qvec) * inv;
     // written so that NaN (degenerate triangle, det == 0) fails every test
     const float m = fminf(fminf(u, v), 1.f - u - v);
-#if PTB_EDGE_EPS_ON
     // inside the triangle grown by PTB_EDGE_EPS, in front of the origin and not clearly beyond the best hit ...
     // (c.w = PTB_TRI_T_CUT, or 0 on the covering triangles of a volume, whose own hit may be nearer than the face the ray crosses)
     if (!(m >= -PTB_EDGE_EPS) || !(tt >= 0.f) || !(tt * c.w < tbest)) return false;
@@ -386,9 +222,6 @@ PTB_HD bool tri_test(const F4& a, const F4& b, const F4& c, const RayPrep& r, fl
     // the reference's arithmetic decides
     if (m < b.w && tri_exact_available(ex)) return tri_exact(ex, prim, r.o, r.d, tbest, t, b1, b2);
     if (!(m >= 0.f) || !(tt < tbest)) return false;
-#else
-    if (!(m >= 0.f) || !(tt >= 0.f) || !(tt < tbest)) return false;
-#endif
     t = tt; b1 = u; b2 = v;
     return true;
 }
@@ -401,7 +234,7 @@ PTB_HD int tri_test_classify(const F4& a, const F4& b, const F4& c, const RayPre
     const V3 v0 = v3(a.x, a.y, a.z), e1 = v3(b.x, b.y, b.z), e2 = v3(c.x, c.y, c.z);
     const V3 pvec = cross(r.d, e2);
     const float det = dot(e1, pvec);
-#if defined(__CUDA_ARCH__) && !defined(PTB_TRI_RCP_EXACT)
+#if defined(__CUDA_ARCH__)
     float inv;
     asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(inv) : "f"(det));
 #else
@@ -413,14 +246,10 @@ PTB_HD int tri_test_classify(const F4& a, const F4& b, const F4& c, const RayPre
     const float v = dot(r.d, qvec) * inv;
     const float tt = dot(e2, qvec) * inv;
     const float m = fminf(fminf(u, v), 1.f - u - v);
-#if PTB_EDGE_EPS_ON
     // same instruction count as the plain accept test for the common outcome (a miss): one min3 and three compares
     if (!(m >= -PTB_EDGE_EPS) || !(tt >= 0.f) || !(tt * c.w < tbest)) return 0;   // c.w = PTB_TRI_T_CUT (t of the two formulations differs in the last bits) or 0 (yarn covers)
     if (m < b.w) return 2;            // b.w = PTB_EDGE_EPS, or +inf on alpha-tested triangles
     if (!(tt < tbest)) return 0;
-#else
-    if (!(m >= 0.f) || !(tt >= 0.f) || !(tt < tbest)) return 0;
-#endif
     t = tt; b1 = u; b2 = v;
     return 1;
 }

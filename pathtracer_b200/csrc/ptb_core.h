@@ -364,9 +364,7 @@ PTB_HD_NOINLINE int merl_index(double theta_in, double fi_in, double theta_out, 
 // the inputs, 1-3 ulp; float rounding here): 1.5e-6 on the unit vectors, propagated to each position.  Otherwise it returns false
 // and the caller runs the double path, so the bin index is the reference's in both cases (checked against the double path on 1e8
 // random direction pairs by tests/test_host_logic.py::test_merl_index_fast, and on the device by the MERL KAT).
-#if !defined(PTB_MERL_EPS0)
 #define PTB_MERL_EPS0 2.5e-6f   /* device atan2f: 2 ulp of an azimuth up to 2 pi = 1e-6; acosf; the float arithmetic here */
-#endif
 PTB_HD bool merl_index_fast(V3 wil, V3 wol, int& ind) {
     const float HALF_PI = 1.57079632679489662f, INV_PI_180 = 57.2957795130823209f;   // 180/pi = 90/(pi/2)
     // the reference goes through theta = acosf(z), phi = atan2f(y, x) and rebuilds (sin theta cos phi, sin theta sin phi, cos theta):
@@ -425,10 +423,7 @@ PTB_HD V3 merl_eval(const float* table, V3 wi, V3 wo, V3 N) {
     float thetao = acosf(wol.z);
     if ((double)thetao >= PTB_PI_D / 2) return v3(0, 0, 0);
     int ind;
-#if !defined(PTB_MERL_DOUBLE_ONLY)
-    if (!merl_index_fast(wil, wol, ind))
-#endif
-    {
+    if (!merl_index_fast(wil, wol, ind)) {
         float phio = atan2f(wol.y, wol.x);
         if (phio < 0) phio = (float)((double)phio + 2 * PTB_PI_D);
         float phii = atan2f(wil.y, wil.x);

@@ -7,7 +7,6 @@
 // Queues are index lists compacted with warp ballots + one atomic per warp (k_shade); every kernel reads
 // its element count from device memory, so the host never waits for a count.
 // There is no CPU implementation behind this ABI: a missing device or a failed launch is an error code.
-#include <cub/device/device_radix_sort.cuh>
 #include <cuda_runtime.h>
 #include <dlfcn.h>
 #include <nccl.h>
@@ -45,40 +44,13 @@ using namespace ptb;
 #define PTB_CNT_ALLOC (5 * (PTB_MAX_BOUNCES + 1))       // branching renders: side-branch slots handed out in this pass
 #define PTB_CNT_DROPS (5 * (PTB_MAX_BOUNCES + 1) + 1)   // side branches that found the pool full
 #define PTB_CNT_PROBE (5 * (PTB_MAX_BOUNCES + 1) + 2)   // subsurface probes emitted at the current level
-#define PTB_CNT_SURF (5 * (PTB_MAX_BOUNCES + 1) + 3)    // [+ b] surface hits of bounce b (the queue k_sort_hits leaves for k_shade)
-#define PTB_CNT_DEFER (6 * (PTB_MAX_BOUNCES + 1) + 3)   // [+ 2*b] / [+ 2*b + 1]: rays of bounce b (closest / any-hit) that left candidates for k_exact
-#define PTB_N_COUNTERS (8 * (PTB_MAX_BOUNCES + 1) + 3)
+#define PTB_CNT_DEFER (5 * (PTB_MAX_BOUNCES + 1) + 3)   // [+ 2*b] / [+ 2*b + 1]: rays of bounce b (closest / any-hit) that left candidates for k_exact
+#define PTB_N_COUNTERS (7 * (PTB_MAX_BOUNCES + 1) + 3)
 #define PTB_DEFER_K 4    /* candidates a ray can leave for k_exact; a ray with more is re-traced there with the immediate exact test */
 // 64-bit totals: 0 closest rays, 1 shadow rays, 2/3 node visits / triangle tests of the closest-hit trace, 4/5 of the any-hit trace
 #define PTB_N_TOTALS 10   /* 0-1 rays, 2-5 node visits / triangle tests (closest, any hit), 6-9 triangle-phase warp iterations and their packed minimum (COUNT kernels) */
 #define PTB_BRANCH_MAX_LEVELS 512
 #define PTB_MAX_PIPES 4
-#ifndef PTB_TRACE_MINB
-#define PTB_TRACE_MINB 0    /* > 0 forces the register allocation of k_trace to allow that many resident blocks per SM (A/B only: the kernel
-                               compiles to 56 registers = 9 blocks of 128 threads by itself, and a forced 9 measured 2 % slower) */
-#endif
-#ifndef PTB_SMEM_STACK
-#define PTB_SMEM_STACK 0   /* entries of k_trace's traversal stack held in shared memory (A/B: profiles/r02a_ab_smem_stack.txt) */
-#endif
-// L1 policy of k_trace's two gathers (A/B): nodes are re-read by every ray of a warp and by its neighbours (the top levels by everybody),
-// a triangle is read by the few rays that reach its leaf.  PTB_LD_TRI: 1 = triangles do not allocate in L1, 2 = evict first;
-// PTB_LD_NODE: 1 = nodes evict last.  0 = plain read-only loads (__ldg).
-#if !defined(PTB_LD_TRI)
-#define PTB_LD_TRI 0
-#endif
-#if !defined(PTB_LD_NODE)
-#define PTB_LD_NODE 0
-#endif
-__device__ __forceinline__ float4 ld_hint(const float4* q, int hint) {
-    float4 v;
-    if (hint == 1) asm("ld.global.nc.L1::no_allocate.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(q));
-    else if (hint == 2) asm("ld.global.nc.L1::evict_first.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(q));
-    else if (hint == 3) asm("ld.global.nc.L1::evict_last.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(q));
-    else v = __ldg(q);
-    return v;
-}
-#define PTB_LDN(q) ld_hint((q), PTB_LD_NODE ? 3 : 0)
-#define PTB_LDT(q) ld_hint((q), PTB_LD_TRI)
 
 // ------------------------------------------------------------------------------------------------ kernels
 __global__ void __launch_bounds__(256) k_rpp(float* rpp, int n) {
@@ -108,19 +80,11 @@ __global__ void __launch_bounds__(256) k_raygen(SceneDev sc, FrameDev f, PoolDev
 // ANY_HIT = shadow rays (queue = shadow entries, first accepted triangle ends the ray; an unoccluded ray adds its deferred
 // direct term to the path's radiance).  Closest-hit results overwrite the analytic hit record the ray's producer wrote.
 template <bool ANY_HIT, bool COUNT, bool BRANCH = false>
-#if defined(PTB_TRACE_MAXNREG)
-__global__ void __maxnreg__(PTB_TRACE_MAXNREG) k_trace(
-#elif PTB_TRACE_MINB > 0
-__global__ void __launch_bounds__(128, PTB_TRACE_MINB) k_trace(
-#else
-__global__ void __launch_bounds__(128) k_trace(
-#endif
-SceneDev sc, PoolDev p, const uint32_t* __restrict__ queue, const uint32_t* __restrict__ count,
+__global__ void __launch_bounds__(128) k_trace(SceneDev sc, PoolDev p, const uint32_t* __restrict__ queue, const uint32_t* __restrict__ count,
                                                int n_static, uint32_t* cursor, unsigned long long* totals, int refill_below, int tri_den, int tri_min_pct,
                                                uint32_t* defer_count) {
     const uint32_t FULL = 0xffffffffu;
     const uint32_t lane = threadIdx.x & 31;
-#if !defined(PTB_NO_PICK_LUT)
     // pick_slot as a table: slot = lut[7 - octant][hit internal children] (2 KB of shared memory, filled once per persistent block):
     // one LDS instead of thirteen ALU instructions per node visit (+1.2 % on C2 / C3, profiles/r01p_ab_pick_lut.txt)
     __shared__ uint8_t pick_lut[8 * 256];
@@ -130,9 +94,7 @@ SceneDev sc, PoolDev p, const uint32_t* __restrict__ queue, const uint32_t* __re
         pick_lut[i] = (i & 0xffu) ? (uint8_t)pick_slot(i & 0xffu, packed) : (uint8_t)0;
     }
     __syncthreads();
-#endif
     const uint32_t n = count ? *count : (uint32_t)n_static;
-    const AlphaCtx ac = alpha_ctx(sc);
     const F4* __restrict__ nodes = sc.nodes;
     const F4* __restrict__ tris = sc.tris;
     bool live = false, exhausted = false;
@@ -140,23 +102,8 @@ SceneDev sc, PoolDev p, const uint32_t* __restrict__ queue, const uint32_t* __re
     RayPrep r;
     float tbest = 0.f, hb1 = 0.f, hb2 = 0.f;
     int32_t hprim = -1;
-    // Traversal stack: the first PTB_SMEM_STACK entries of every lane live in shared memory ([entry][thread]: a warp's 8-byte accesses
-    // are conflict-free whatever the lanes' depths), deeper entries in local memory.
     U2 ngroup, tgroup;
-#if PTB_SMEM_STACK > 0 && defined(PTB_SMEM_STACK_ONLY)   // A/B only: no local-memory part at all (entries beyond PTB_SMEM_STACK would be lost)
-    __shared__ uint2 sstack[PTB_SMEM_STACK * 128];
-#define PTB_STK_PUSH(e) do { sstack[(sp < PTB_SMEM_STACK ? sp : PTB_SMEM_STACK - 1) * 128 + threadIdx.x] = make_uint2((e).x, (e).y); sp++; } while (0)
-#define PTB_STK_POP(e) do { --sp; const uint2 q_ = sstack[sp * 128 + threadIdx.x]; (e).x = q_.x; (e).y = q_.y; } while (0)
-#elif PTB_SMEM_STACK > 0
-    __shared__ uint2 sstack[PTB_SMEM_STACK * 128];
-    U2 lstack[PTB_STACK - PTB_SMEM_STACK];
-#define PTB_STK_PUSH(e) do { if (sp < PTB_SMEM_STACK) sstack[sp * 128 + threadIdx.x] = make_uint2((e).x, (e).y); else lstack[sp - PTB_SMEM_STACK] = (e); sp++; } while (0)
-#define PTB_STK_POP(e) do { --sp; if (sp < PTB_SMEM_STACK) { const uint2 q_ = sstack[sp * 128 + threadIdx.x]; (e).x = q_.x; (e).y = q_.y; } else (e) = lstack[sp - PTB_SMEM_STACK]; } while (0)
-#else
-    U2 lstack[PTB_STACK];
-#define PTB_STK_PUSH(e) do { lstack[sp++] = (e); } while (0)
-#define PTB_STK_POP(e) do { (e) = lstack[--sp]; } while (0)
-#endif
+    U2 lstack[PTB_STACK];   // traversal stack (local memory)
     // candidates the ray has left for k_exact (tri_test_classify case 2) are counted in a register the variant has no other use for:
     // `entry` for closest-hit rays, `hprim` for any-hit rays
     uint32_t tvalid = 0;   // valid24 of the node the live triangle group came from (all ones for a group popped from the stack: compact bits)
@@ -165,10 +112,6 @@ SceneDev sc, PoolDev p, const uint32_t* __restrict__ queue, const uint32_t* __re
     uint32_t cn = 0, ct = 0;
     uint32_t w_iters = 0, w_ideal = 0;   // COUNT: triangle-phase iterations of this warp, and how few would do if its tests were packed 32 to an iteration
     r.o = r.d = r.idir = v3(0, 0, 0); r.oct_inv4 = 0;
-#if PTB_NODE_HALF
-    RaySlopes rs; rs.x = rs.y = rs.z = 0;
-    const int half_c = sc.half_c;
-#endif
     for (;;) {
         // ---- refill idle lanes from the queue
         const uint32_t live_mask = __ballot_sync(FULL, live);
@@ -183,17 +126,14 @@ SceneDev sc, PoolDev p, const uint32_t* __restrict__ queue, const uint32_t* __re
                     F4 o, d;
                     float tmax;
                     bool ok = true;
-                    if (ANY_HIT) { entry = qi; o = pool_ld(&p.sh_o[qi]); d = pool_ld(&p.sh_d[qi]); tmax = o.w; }
+                    if (ANY_HIT) { entry = qi; o = p.sh_o[qi]; d = p.sh_d[qi]; tmax = o.w; }
                     else {
                         item = queue ? queue[qi] : qi;
                         ok = p.pixel[item] != 0xffffffffu;
-                        o = pool_ld(&p.ray_o[item]); d = pool_ld(&p.ray_d[item]); tmax = p.hit[item].x;
+                        o = p.ray_o[item]; d = p.ray_d[item]; tmax = p.hit[item].x;
                     }
                     if (ok) {
                         r = ray_prep(v3(o.x, o.y, o.z), v3(d.x, d.y, d.z));
-#if PTB_NODE_HALF
-                        rs = ray_slopes(r, half_c);
-#endif
                         tbest = tmax; hprim = ANY_HIT ? 0 : -1; sp = 0;
                         if (!ANY_HIT) entry = 0;
                         ngroup.x = 0; ngroup.y = 0x80000000u; tgroup.x = 0; tgroup.y = 0;
@@ -211,28 +151,27 @@ SceneDev sc, PoolDev p, const uint32_t* __restrict__ queue, const uint32_t* __re
         // ---- pop / finish: lanes with neither node nor triangle work
         if (live && ngroup.y <= 0x00ffffffu && tgroup.y == 0) {
             if (sp > 0) {
-                U2 e;
-                PTB_STK_POP(e);
+                const U2 e = lstack[--sp];
                 if (e.y > 0x00ffffffu) ngroup = e; else { tgroup = e; tvalid = 0x00ffffffu; }
             } else {
                 // candidates left for k_exact: it finishes the ray (the nearest of them may beat the hit found here; a shadow ray is only
                 // unoccluded if none of them blocks it)
                 const uint32_t nd = ANY_HIT ? (uint32_t)hprim : entry;
-                if (PTB_EDGE_EPS_ON && nd) {
+                if (nd) {
                     const uint32_t qi = atomicAdd(defer_count, 1u);
                     U2 dr; dr.x = ANY_HIT ? entry : item; dr.y = nd;
                     p.defer_rays[qi] = dr;
                 }
-                if (PTB_EDGE_EPS_ON && ANY_HIT && nd) { /* k_exact delivers or settles */ }
+                if (ANY_HIT && nd) { /* k_exact delivers or settles */ }
                 else if (ANY_HIT && BRANCH) shadow_settle_branch(p, (int)entry, item, false);
                 else if (ANY_HIT) {   // unoccluded: deliver the deferred direct term (Raytracer.cpp:545-566)
-                    const F4 c = pool_ld(&p.sh_c[entry]);
-                    F4 L = pool_ld(&p.radiance[item]);
+                    const F4 c = p.sh_c[entry];
+                    F4 L = p.radiance[item];
                     L.x += c.x; L.y += c.y; L.z += c.z;
-                    pool_st(&p.radiance[item], L);
+                    p.radiance[item] = L;
                 } else if (hprim >= 0) {
                     F4 q; q.x = tbest; q.y = hb1; q.z = hb2; q.w = u2f((uint32_t)hprim);
-                    pool_st(&p.hit[item], q);
+                    p.hit[item] = q;
                 }
                 live = false;
             }
@@ -247,31 +186,23 @@ SceneDev sc, PoolDev p, const uint32_t* __restrict__ queue, const uint32_t* __re
                     cm |= 1u << popcount32(tvalid & ~(0xffffffffu << b));
                 } while (m);
                 tgroup.y = cm;
-                PTB_STK_PUSH(tgroup);   // never full: ptb_commit refuses trees deeper than PTB_STACK / 2
+                lstack[sp++] = tgroup;   // never full: ptb_commit refuses trees deeper than PTB_STACK / 2
                 tgroup.y = 0;
             }
             const uint32_t hits_imask = ngroup.y;
-#if !defined(PTB_NO_PICK_LUT)
             const uint32_t slot = pick_lut[((r.oct_inv4 & 7u) << 8) | (hits_imask >> 24)];
-#else
-            const uint32_t slot = pick_slot(hits_imask >> 24, r.oct_inv4);
-#endif
             const uint32_t child_base = ngroup.x;
             ngroup.y &= ~(1u << (24u + slot));
-            if (ngroup.y > 0x00ffffffu) PTB_STK_PUSH(ngroup);
+            if (ngroup.y > 0x00ffffffu) lstack[sp++] = ngroup;
             const uint32_t rel = popcount32(hits_imask & ~(0xffffffffu << slot));
             const float4* np = reinterpret_cast<const float4*>(nodes) + (size_t)(child_base + rel) * 5;
-            const float4 l0 = PTB_LDN(np), l1 = PTB_LDN(np + 1), l2 = PTB_LDN(np + 2), l3 = PTB_LDN(np + 3), l4 = PTB_LDN(np + 4);
+            const float4 l0 = __ldg(np), l1 = __ldg(np + 1), l2 = __ldg(np + 2), l3 = __ldg(np + 3), l4 = __ldg(np + 4);
             F4 n0, n1, n2, n3, n4;
             n0.x = l0.x; n0.y = l0.y; n0.z = l0.z; n0.w = l0.w; n1.x = l1.x; n1.y = l1.y; n1.z = l1.z; n1.w = l1.w;
             n2.x = l2.x; n2.y = l2.y; n2.z = l2.z; n2.w = l2.w; n3.x = l3.x; n3.y = l3.y; n3.z = l3.z; n3.w = l3.w;
             n4.x = l4.x; n4.y = l4.y; n4.z = l4.z; n4.w = l4.w;
             if (COUNT) cn++;
-#if PTB_NODE_HALF
-            const uint32_t hm = node_hitmask_k(n0, n1, n2, n3, n4, r, rs, tbest);
-#else
             const uint32_t hm = node_hitmask(n0, n1, n2, n3, n4, r, tbest);
-#endif
             ngroup.x = f2u(n1.x);
             tgroup.x = f2u(n1.y);
             ngroup.y = (hm & 0xff000000u) | (f2u(n0.w) >> 24);
@@ -293,23 +224,19 @@ SceneDev sc, PoolDev p, const uint32_t* __restrict__ queue, const uint32_t* __re
                     tgroup.y &= ~(1u << ti);
                     const uint32_t prim = tgroup.x + popcount32(tvalid & ~(0xffffffffu << ti));
                     const float4* tp = reinterpret_cast<const float4*>(tris) + (size_t)prim * 3;
-                    const float4 l0 = PTB_LDT(tp), l1 = PTB_LDT(tp + 1), l2 = PTB_LDT(tp + 2);
+                    const float4 l0 = __ldg(tp), l1 = __ldg(tp + 1), l2 = __ldg(tp + 2);
                     F4 a, b, c;
                     a.x = l0.x; a.y = l0.y; a.z = l0.z; a.w = l0.w; b.x = l1.x; b.y = l1.y; b.z = l1.z; b.w = l1.w;
                     c.x = l2.x; c.y = l2.y; c.z = l2.z; c.w = l2.w;
                     if (COUNT) ct++;
                     float t, b1, b2;
                     const int res = tri_test_classify(a, b, c, r, tbest, t, b1, b2);
-                    if (PTB_EDGE_EPS_ON && res == 2) {            // near an edge / alpha-tested / a disc: left for k_exact (the reference's own arithmetic)
+                    if (res == 2) {            // near an edge / alpha-tested / a disc: left for k_exact (the reference's own arithmetic)
                         const uint32_t nd = ANY_HIT ? (uint32_t)hprim : entry;
                         if (nd < PTB_DEFER_K) p.defer_prims[(size_t)(ANY_HIT ? entry : item) * PTB_DEFER_K + nd] = prim | ((f2u(a.w) & 7u) << 28);
                         if (ANY_HIT) hprim++; else entry++;
                     } else if (res == 1) {
-#if PTB_EDGE_EPS_ON
                         if (!(ANY_HIT && (f2u(a.w) & PTB_TRI_FLAG_GHOST))) {     // (alpha-tested triangles always take the deferred route)
-#else
-                        if (!((f2u(a.w) & PTB_TRI_FLAG_ALPHA) && alpha_rejects(&ac, (int)prim, b1, b2)) && !(ANY_HIT && (f2u(a.w) & PTB_TRI_FLAG_GHOST))) {
-#endif
                             if (ANY_HIT) { live = false; tgroup.y = 0; if (BRANCH) shadow_settle_branch(p, (int)entry, item, true); }   // occluded: nothing to deliver
                             else { tbest = t; hb1 = b1; hb2 = b2; hprim = (int32_t)prim; }
                         }
@@ -387,54 +314,7 @@ __device__ __forceinline__ uint32_t warp_push(uint32_t* counter, bool want) {
     return base + __popc(mask & ((1u << lane) - 1u));
 }
 
-// EXPERIMENT (PTB_SORT_QUEUE=1|2, one pass pipeline): how much would `k_trace` gain from a coherent bounce queue?  The queue of a bounce
-// >= 1 is sorted by {direction octant, Morton code of the origin on a 512^3 grid} (1) or {Morton code, octant} (2) with a separate
-// radix sort before the traversal kernel; the sort's own time is not part of the kernel's.  An upper bound for what binning the queue
-// inside k_shade's append could buy (VERDICT round 1, item 3 ii); measured in profiles/r02aj_ab_sorted_queue.txt.
-__device__ __forceinline__ uint32_t spread3(uint32_t v) {   // 9 bits -> every third bit
-    v &= 0x1ffu;
-    v = (v | (v << 16)) & 0x030000ffu;
-    v = (v | (v << 8)) & 0x0300f00fu;
-    v = (v | (v << 4)) & 0x030c30c3u;
-    v = (v | (v << 2)) & 0x09249249u;
-    return v;
-}
-__global__ void __launch_bounds__(256) k_queue_keys(PoolDev p, const uint32_t* __restrict__ queue, const uint32_t* __restrict__ count, int n, uint32_t* keys, int mode) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    uint32_t key = 0xffffffffu;
-    if ((uint32_t)i < *count) {
-        const uint32_t item = queue[i];
-        const F4 o = p.ray_o[item], d = p.ray_d[item];
-        const uint32_t oct = (d.x < 0 ? 4u : 0u) | (d.y < 0 ? 2u : 0u) | (d.z < 0 ? 1u : 0u);
-        const float sc_ = 512.f / 160.f;
-        const uint32_t qx = (uint32_t)fminf(fmaxf((o.x + 80.f) * sc_, 0.f), 511.f), qy = (uint32_t)fminf(fmaxf((o.y + 80.f) * sc_, 0.f), 511.f),
-                       qz = (uint32_t)fminf(fmaxf((o.z + 80.f) * sc_, 0.f), 511.f);
-        const uint32_t m = spread3(qx) | (spread3(qy) << 1) | (spread3(qz) << 2);
-        key = mode == 2 ? ((m << 3) | oct) : ((oct << 27) | m);
-        key &= 0x7fffffffu;
-    }
-    keys[i] = key;
-}
-
-// Shades the terminal hits of a bounce (miss / light / dome) and compacts the surface hits into `out_queue` for k_shade.
-__global__ void __launch_bounds__(256) k_sort_hits(SceneDev sc, PoolDev p, const uint32_t* __restrict__ queue, const uint32_t* __restrict__ count, int n_static,
-                                                   uint32_t* __restrict__ out_queue, uint32_t* out_count) {
-    const int tid = blockIdx.x * blockDim.x + threadIdx.x;
-    const int n = count ? (int)*count : n_static;
-    bool surface = false;
-    int path = 0;
-    if (tid < n) {
-        path = queue ? (int)queue[tid] : tid;
-        surface = !shade_terminal_one(sc, p, path);
-    }
-    const uint32_t qi = warp_push(out_count, surface);
-    if (surface) out_queue[qi] = (uint32_t)path;
-}
-
-#ifndef PTB_SHADE_BLOCK
 #define PTB_SHADE_BLOCK 256    /* threads per k_shade block: half as many blocks for a later bounce to launch only to see them return (r02w: k_shade -4 % on C2, -3 % on C4 against 128; 512 is no better) */
-#endif
 template <bool MERL, int MINB, bool AOV, bool EXOTIC = false>
 __global__ void __launch_bounds__(PTB_SHADE_BLOCK, (MINB * 128) / PTB_SHADE_BLOCK) k_shade(SceneDev sc, FrameDev f, PoolDev p, const uint32_t* __restrict__ queue,
                                                const uint32_t* __restrict__ count, int n_static, uint32_t* __restrict__ next_queue,
@@ -464,7 +344,7 @@ __global__ void __launch_bounds__(PTB_SHADE_BLOCK, (MINB * 128) / PTB_SHADE_BLOC
     bc = __shfl_sync(0xffffffffu, bc, 0); bs = __shfl_sync(0xffffffffu, bs, 0);
     const uint32_t below = (1u << lane) - 1u;
     if (out.cont) next_queue[bc + __popc(mc & below)] = (uint32_t)path;
-    if (out.shadow) { const uint32_t si = bs + __popc(ms & below); pool_st(&p.sh_o[si], out.sh_o); pool_st(&p.sh_d[si], out.sh_d); pool_st(&p.sh_c[si], out.sh_c); }
+    if (out.shadow) { const uint32_t si = bs + __popc(ms & below); p.sh_o[si] = out.sh_o; p.sh_d[si] = out.sh_d; p.sh_c[si] = out.sh_c; }
 }
 
 // Branching renders (fog, ghost objects, background photograph): one getColor loop iteration per queue entry; side branches
@@ -576,7 +456,7 @@ __device__ __forceinline__ uint32_t refit_exponent_byte(float extent, float coor
     return (uint32_t)(e + 127);
 }
 __global__ void __launch_bounds__(128) k_refit_level(Node8* nodes, F4* node_box, const F4* __restrict__ tris_obj, const ObjectDev* __restrict__ objects,
-                                                     uint32_t first, uint32_t count, int half_c, uint32_t* outgrown) {
+                                                     uint32_t first, uint32_t count, int e_lo) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= count) return;
     Node8 nd = nodes[first + i];
@@ -619,13 +499,9 @@ __global__ void __launch_bounds__(128) k_refit_level(Node8* nodes, F4* node_box,
     F4 q;
     q.x = nlo[0]; q.y = nlo[1]; q.z = nlo[2]; q.w = 0; node_box[2 * (size_t)(first + i)] = q;
     q.x = nhi[0]; q.y = nhi[1]; q.z = nhi[2]; node_box[2 * (size_t)(first + i) + 1] = q;
-    const int e_lo = PTB_HALF_E_LO - half_c;
     const uint32_t eb[3] = {refit_exponent_byte(nhi[0] - nlo[0], node_coord_slack(nlo[0], nhi[0]), e_lo), refit_exponent_byte(nhi[1] - nlo[1], node_coord_slack(nlo[1], nhi[1]), e_lo),
                             refit_exponent_byte(nhi[2] - nlo[2], node_coord_slack(nlo[2], nhi[2]), e_lo)};
     nd.ex = (uint8_t)eb[0]; nd.ey = (uint8_t)eb[1]; nd.ez = (uint8_t)eb[2];
-    // cells too large for the scene's half grid (the re-posed scene is more than 16x the size it was committed at): the caller refuses the frame
-    if ((int)max(eb[0], max(eb[1], eb[2])) - 127 + half_c > PTB_HALF_E_HI) *outgrown = 1u;
-    nd.hx = half_exp_byte((int)eb[0] - 127, half_c); nd.hy = half_exp_byte((int)eb[1] - 127, half_c); nd.hz = half_exp_byte((int)eb[2] - 127, half_c);
     float cell[3], eps[3], p[3];
     for (int k = 0; k < 3; k++) {
         cell[k] = u2f(eb[k] << 23);                                                       // 2^(e - 127 + 127 - 127)... the byte IS the float's exponent field
@@ -763,15 +639,6 @@ __global__ void k_kat(int which, SceneDev sc, CameraDev cam, FilterDev filt, int
     case PTB_KAT_RANDOM_PER_PIXEL: { float x, y; random_per_pixel((uint32_t)a[0], x, y); o[0] = x; o[1] = y; } break;
     case PTB_KAT_FILTER_RATIO: { int b0, b1, b2, b3; o[0] = filter_ratio(filt, (int)a[0], (int)a[1], W, H, b0, b1, b2, b3); } break;
     case PTB_KAT_MERL_INDEX: { int f, e; merl_index_both(v3((float)a[0], (float)a[1], (float)a[2]), v3((float)a[3], (float)a[4], (float)a[5]), f, e); o[0] = f; o[1] = e; } break;
-#if PTB_NODE_HALF
-    case PTB_KAT_NODE_HALF: {      // the node test of k_trace (half factors) next to the float form: it may only ever see MORE children
-        RayPrep r = ray_prep(v3((float)a[0], (float)a[1], (float)a[2]), v3((float)a[3], (float)a[4], (float)a[5]));
-        const RaySlopes rs = ray_slopes(r, sc.half_c);
-        const F4* np = sc.nodes + (size_t)a[7] * 5;
-        o[0] = (double)node_hitmask(np[0], np[1], np[2], np[3], np[4], r, (float)a[6]);
-        o[1] = (double)node_hitmask_k(np[0], np[1], np[2], np[3], np[4], r, rs, (float)a[6]);
-    } break;
-#endif
     default: break;
     }
 }
@@ -791,11 +658,6 @@ struct ptb_ctx {
     int64_t pool_paths = (int64_t)1 << 25, pool_cap = 0;   // measured: larger pools amortise the tails of the persistent kernels (tune4.log)
     PoolDev pool;
     uint32_t* d_queue[2] = {nullptr, nullptr};
-    uint32_t* d_queue_surf = nullptr;          // the surface hits of the current bounce (k_sort_hits -> k_shade)
-    bool sort_hits = false;                    // PTB_OPT_SORT_HITS (measured r01k: slower, see DESIGN.md section 5)
-    int sort_queue = 0;                        // PTB_SORT_QUEUE experiment (k_queue_keys): 0 off, 1 octant-major, 2 origin-major
-    uint32_t *d_sort_keys = nullptr, *d_sort_keys2 = nullptr, *d_sort_vals = nullptr;
-    void* d_sort_tmp = nullptr; size_t sort_tmp_bytes = 0; int sort_cap = 0;
     uint32_t* d_counters = nullptr;
     unsigned long long* d_totals = nullptr;
     float* d_rpp = nullptr;
@@ -829,8 +691,6 @@ struct ptb_ctx {
     bool count_traversal = false;
     bool time_kernels = false;
     bool has_merl = false;
-    int shade_minb_merl = 8;                   // the same for scenes with a MERL object (PTB_SHADE_MINB_MERL: 5, 6 or 8; measured r01m: 89.0 / 81.2 / 76.8 ms on C4)
-    int shade_minb = 8;                        // k_shade variant (resident blocks/SM the compiler must allow); PTB_SHADE_MINB overrides for experiments
     int exact_blocks = 148 * 8;                // grid of k_exact: one thread per ray that left candidates for the usual counts (it strides beyond that); most threads exit at once
     int trace_blocks = 148 * 8;                // persistent grid of k_trace, set from the occupancy query in ptb_create
     int refill_below = 24;                     // a warp refills its idle lanes once fewer than this many are live
@@ -863,12 +723,10 @@ static void free_scene(ptb_ctx* c) {
 }
 static void free_pool(ptb_ctx* c) {
     void* ptrs[] = {c->pool.ray_o, c->pool.ray_d, c->pool.weight, c->pool.radiance, c->pool.hit, c->pool.rng, c->pool.pixel,
-                    c->pool.sh_o, c->pool.sh_d, c->pool.sh_c, c->d_queue[0], c->d_queue[1], c->d_queue_surf, c->pool.aov_n, c->pool.aov_kd, c->pool.root, c->pool.probe_o, c->pool.probe_d, c->pool.probe_x, c->pool.hit2, c->pool.defer_prims, c->pool.defer_rays};
+                    c->pool.sh_o, c->pool.sh_d, c->pool.sh_c, c->d_queue[0], c->d_queue[1], c->pool.aov_n, c->pool.aov_kd, c->pool.root, c->pool.probe_o, c->pool.probe_d, c->pool.probe_x, c->pool.hit2, c->pool.defer_prims, c->pool.defer_rays};
     for (void* p : ptrs) if (p) cudaFree(p);
     memset(&c->pool, 0, sizeof(c->pool));
-    c->d_queue[0] = c->d_queue[1] = nullptr; c->d_queue_surf = nullptr;
-    cudaFree(c->d_sort_keys); cudaFree(c->d_sort_keys2); cudaFree(c->d_sort_vals); cudaFree(c->d_sort_tmp);     // (the PTB_SORT_QUEUE experiment's buffers)
-    c->d_sort_keys = c->d_sort_keys2 = c->d_sort_vals = nullptr; c->d_sort_tmp = nullptr; c->sort_cap = 0;
+    c->d_queue[0] = c->d_queue[1] = nullptr;
     c->pool_cap = 0;
 }
 
@@ -901,7 +759,6 @@ static int ensure_pool(ptb_ctx* c, int64_t paths, bool aov = false, bool branch 
     CK(cudaMalloc((void**)&c->pool.sh_c, n * sizeof(F4)));
     CK(cudaMalloc((void**)&c->d_queue[0], n * sizeof(uint32_t)));
     CK(cudaMalloc((void**)&c->d_queue[1], n * sizeof(uint32_t)));
-    CK(cudaMalloc((void**)&c->d_queue_surf, n * sizeof(uint32_t)));
     CK(cudaMalloc((void**)&c->pool.defer_prims, n * PTB_DEFER_K * sizeof(uint32_t)));
     CK(cudaMalloc((void**)&c->pool.defer_rays, n * sizeof(U2)));
     if (aov) {
@@ -1014,30 +871,20 @@ static int refit_device(ptb_ctx* c, FlatScene& f, const HostScene& host) {
     const bool mesh = sc.has_mesh && n_tri > 0;
     if (mesh) {   // (the first re-pose of a context allocates the per-node boxes: not part of the measured device time)
         if (!sc.tris_obj) { c->err = "refit: the scene was committed without object-space triangles"; return PTB_ERR_STATE; }
-        if ((rc = grow(c, &c->d_node_box, &c->node_box_n, 2 * (int64_t)f.bvh.n_nodes + 1))) return rc;
+        if ((rc = grow(c, &c->d_node_box, &c->node_box_n, 2 * (int64_t)f.bvh.n_nodes))) return rc;
     }
     CK(cudaEventRecord(c->ev0, c->stream));
     CK(cudaMemcpyAsync(const_cast<ObjectDev*>(sc.objects), f.objects.data(), f.objects.size() * sizeof(ObjectDev), cudaMemcpyHostToDevice, c->stream));
     if (mesh) {
-        uint32_t* outgrown = reinterpret_cast<uint32_t*>(c->d_node_box + 2 * (size_t)f.bvh.n_nodes);      // one flag behind the boxes
-        CK(cudaMemsetAsync(outgrown, 0, sizeof(uint32_t), c->stream));
         k_refit_tris<<<(unsigned)((n_tri + 255) / 256), 256, 0, c->stream>>>(sc.tris_obj, sc.objects, const_cast<F4*>(sc.tris), n_tri);
         const std::vector<uint32_t>& ls = f.bvh.level_start;
         for (int l = (int)ls.size() - 2; l >= 0; l--) {
             const uint32_t first = ls[l], count = ls[l + 1] - ls[l];
-            if (count) k_refit_level<<<(count + 127) / 128, 128, 0, c->stream>>>(reinterpret_cast<Node8*>(const_cast<F4*>(sc.nodes)), c->d_node_box, sc.tris_obj, sc.objects, first, count, sc.half_c, outgrown);
+            if (count) k_refit_level<<<(count + 127) / 128, 128, 0, c->stream>>>(reinterpret_cast<Node8*>(const_cast<F4*>(sc.nodes)), c->d_node_box, sc.tris_obj, sc.objects, first, count, f.bvh.e_floor);
         }
         CK(cudaGetLastError());
-        CK(cudaEventRecord(c->ev1, c->stream));      // device time of the re-pose: upload of the object table, triangles, node boxes (no host round trip inside)
-        uint32_t flag = 0;
-        CK(cudaMemcpyAsync(&flag, outgrown, sizeof(flag), cudaMemcpyDeviceToHost, c->stream));
-        CK(cudaStreamSynchronize(c->stream));
-        if (flag) {
-            c->committed = false;      // the node planes of this frame are not usable
-            c->err = "refit: the re-posed scene is more than 16x larger than the committed one (the half grid of the BVH8 cannot hold its cells); commit it at this frame instead";
-            return PTB_ERR_UNSUPPORTED;
-        }
-    } else CK(cudaEventRecord(c->ev1, c->stream));
+    }
+    CK(cudaEventRecord(c->ev1, c->stream));      // device time of the re-pose: upload of the object table, triangles, node boxes (no host round trip inside)
     CK(cudaStreamSynchronize(c->stream));
     float ms = 0;
     CK(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
@@ -1070,11 +917,7 @@ int ptb_create(int device_id, ptb_ctx** out) {
     if (device_id < 0 || device_id >= n) { g_create_err = "device id out of range"; return PTB_ERR_INVALID; }
     ptb_ctx* c = new ptb_ctx();
     c->device = device_id;
-    if (const char* e = getenv("PTB_SHADE_MINB")) c->shade_minb = atoi(e);
-    if (const char* e = getenv("PTB_SHADE_MINB_MERL")) c->shade_minb_merl = atoi(e);
     if (const char* e = getenv("PTB_PIPES")) c->n_pipes = std::max(1, std::min(atoi(e), PTB_MAX_PIPES));
-    if (const char* e = getenv("PTB_SORT_HITS")) c->sort_hits = atoi(e) != 0;   // experiments: 0 = k_shade sees every hit
-    if (const char* e = getenv("PTB_SORT_QUEUE")) c->sort_queue = atoi(e);
     memset(&c->pool, 0, sizeof(c->pool));
     memset(&c->sc, 0, sizeof(c->sc));
     if (cudaSetDevice(device_id) != cudaSuccess || cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking) != cudaSuccess ||
@@ -1388,7 +1231,6 @@ static int render_passes(ptb_ctx* c, FrameDev f, int nrays, F4* d_rgbw, ptb_stat
                 cudaStream_t ps = pi ? c->pipe_stream[pi] : c->stream;
                 const PoolDev pp = pool_slice(c->pool, (size_t)pi * (size_t)stride);
                 uint32_t* const pq[2] = {c->d_queue[0] + (size_t)pi * stride, c->d_queue[1] + (size_t)pi * stride};
-                uint32_t* const pqs = c->d_queue_surf + (size_t)pi * stride;
                 uint32_t* const pc = c->d_counters + (size_t)pi * PTB_N_COUNTERS;
                 CK(cudaMemsetAsync(pc, 0, PTB_N_COUNTERS * sizeof(uint32_t), ps));
                 lt.begin(0, ps);
@@ -1486,21 +1328,6 @@ static int render_passes(ptb_ctx* c, FrameDev f, int nrays, F4* d_rgbw, ptb_stat
                     const bool mesh = c->sc.has_mesh != 0;
                     // persistent grid: as many blocks as are resident at once, but no more than the queue can feed
                     const unsigned gt = (unsigned)std::max(1, std::min<int>(n_pipes > 1 ? c->trace_blocks_piped : c->trace_blocks, (n_paths + 127) / 128));
-                    if (mesh && c->sort_queue && b >= 1 && n_pipes == 1) {     // experiment: a coherent queue for this bounce (untimed)
-                        if (c->sort_cap < n_paths) {
-                            cudaFree(c->d_sort_keys); cudaFree(c->d_sort_keys2); cudaFree(c->d_sort_vals); cudaFree(c->d_sort_tmp);
-                            CK(cudaMalloc((void**)&c->d_sort_keys, (size_t)n_paths * 4)); CK(cudaMalloc((void**)&c->d_sort_keys2, (size_t)n_paths * 4));
-                            CK(cudaMalloc((void**)&c->d_sort_vals, (size_t)n_paths * 4));
-                            c->sort_tmp_bytes = 0;
-                            cub::DeviceRadixSort::SortPairs(nullptr, c->sort_tmp_bytes, c->d_sort_keys, c->d_sort_keys2, c->d_sort_vals, c->d_sort_vals, n_paths, 0, 32, ps);
-                            CK(cudaMalloc(&c->d_sort_tmp, c->sort_tmp_bytes));
-                            c->sort_cap = n_paths;
-                        }
-                        k_queue_keys<<<g256, 256, 0, ps>>>(pp, q, cnt, n_paths, c->d_sort_keys, c->sort_queue);
-                        size_t tb = c->sort_tmp_bytes;
-                        cub::DeviceRadixSort::SortPairs(c->d_sort_tmp, tb, c->d_sort_keys, c->d_sort_keys2, q, c->d_sort_vals, n_paths, 0, 32, ps);
-                        CK(cudaMemcpyAsync(const_cast<uint32_t*>(q), c->d_sort_vals, (size_t)n_paths * 4, cudaMemcpyDeviceToDevice, ps));
-                    }
                     if (mesh) {
                         lt.begin(1 | (b << 8), ps);
                         if (c->count_traversal) k_trace<false, true><<<gt, 128, 0, ps>>>(c->sc, pp, q, cnt, n_paths, pc + PTB_CNT_CUR + 2 * b, c->d_totals, c->refill_below, c->tri_den, c->tri_min_pct, pc + PTB_CNT_DEFER + 2 * b);
@@ -1510,27 +1337,16 @@ static int render_passes(ptb_ctx* c, FrameDev f, int nrays, F4* d_rgbw, ptb_stat
                         launches += 2;
                     }
                     lt.begin(2 | (b << 8), ps);
-                    // optional: terminal hits (miss / light / dome) shaded by a compaction pass, k_shade sees surface hits only (off: measured slower)
-                    const bool sorted = c->sort_hits && !(aov && b == 0);
-                    const uint32_t* sq = q; const uint32_t* scnt = cnt;
-                    if (sorted) {
-                        k_sort_hits<<<g256, 256, 0, ps>>>(c->sc, pp, q, cnt, n_paths, pqs, pc + PTB_CNT_SURF + b);
-                        sq = pqs; scnt = pc + PTB_CNT_SURF + b;
-                        launches++;
-                    }
-#define PTB_SHADE(M, MB, A) k_shade<M, MB, A><<<(unsigned)((n_paths + PTB_SHADE_BLOCK - 1) / PTB_SHADE_BLOCK), PTB_SHADE_BLOCK, 0, ps>>>(c->sc, f, pp, sq, scnt, n_paths, pq[(b + 1) & 1], pc + 2 * (b + 1), pc + 2 * b + 1, pc + PTB_CNT_SQ + b)
-#define PTB_SHADE_X(M, MB, A) k_shade<M, MB, A, true><<<(unsigned)((n_paths + PTB_SHADE_BLOCK - 1) / PTB_SHADE_BLOCK), PTB_SHADE_BLOCK, 0, ps>>>(c->sc, f, pp, sq, scnt, n_paths, pq[(b + 1) & 1], pc + 2 * (b + 1), pc + 2 * b + 1, pc + PTB_CNT_SQ + b)
+#define PTB_SHADE(M, MB, A) k_shade<M, MB, A><<<(unsigned)((n_paths + PTB_SHADE_BLOCK - 1) / PTB_SHADE_BLOCK), PTB_SHADE_BLOCK, 0, ps>>>(c->sc, f, pp, q, cnt, n_paths, pq[(b + 1) & 1], pc + 2 * (b + 1), pc + 2 * b + 1, pc + PTB_CNT_SQ + b)
+#define PTB_SHADE_X(M, MB, A) k_shade<M, MB, A, true><<<(unsigned)((n_paths + PTB_SHADE_BLOCK - 1) / PTB_SHADE_BLOCK), PTB_SHADE_BLOCK, 0, ps>>>(c->sc, f, pp, q, cnt, n_paths, pq[(b + 1) & 1], pc + 2 * (b + 1), pc + 2 * b + 1, pc + PTB_CNT_SQ + b)
                     if (c->sc.has_exotic) {      // scenes with Cylinder / PointSet objects: the kernels that carry their code (not register-squeezed)
                         if (aov && b == 0) { if (c->has_merl) PTB_SHADE_X(true, 5, true); else PTB_SHADE_X(false, 6, true); }
                         else if (c->has_merl) PTB_SHADE_X(true, 5, false);
                         else PTB_SHADE_X(false, 6, false);
                     } else
                     if (aov && b == 0) { if (c->has_merl) PTB_SHADE(true, 5, true); else PTB_SHADE(false, 6, true); }   // camera rays of a denoiser-input render
-                    else if (c->has_merl) { if (c->shade_minb_merl == 8) PTB_SHADE(true, 8, false); else if (c->shade_minb_merl == 7) PTB_SHADE(true, 7, false); else if (c->shade_minb_merl == 6) PTB_SHADE(true, 6, false); else PTB_SHADE(true, 5, false); }
-                    else if (c->shade_minb == 8) PTB_SHADE(false, 8, false);
-                    else if (c->shade_minb == 7) PTB_SHADE(false, 7, false);
-                    else if (c->shade_minb == 10) PTB_SHADE(false, 10, false);
-                    else PTB_SHADE(false, 6, false);
+                    else if (c->has_merl) PTB_SHADE(true, 8, false);
+                    else PTB_SHADE(false, 8, false);
 #undef PTB_SHADE
 #undef PTB_SHADE_X
                     lt.end();
@@ -1832,7 +1648,6 @@ int ptb_set_option(ptb_ctx* c, int option, int64_t value) {
     case PTB_OPT_TRI_FRACTION: if (value < 1 || value > 64) return PTB_ERR_INVALID; c->tri_den = (int)value; return PTB_OK;
     case PTB_OPT_TRI_MIN_PCT: if (value < 0 || value > 100) return PTB_ERR_INVALID; c->tri_min_pct = (int)value; return PTB_OK;
     case PTB_OPT_TRACE_BLOCKS: if (value < 1) return PTB_ERR_INVALID; c->trace_blocks = c->trace_blocks_piped = (int)value; return PTB_OK;
-    case PTB_OPT_SORT_HITS: c->sort_hits = value != 0; return PTB_OK;
     case PTB_OPT_PIPES: if (value < 1 || value > PTB_MAX_PIPES) return PTB_ERR_INVALID; c->n_pipes = (int)value; return PTB_OK;
     case PTB_OPT_STACK_LIMIT: if (value < 2 || value > PTB_STACK) return PTB_ERR_INVALID; c->stack_limit = (int)value; return PTB_OK;
     case PTB_OPT_BUILD_THREADS: if (value < 0 || value > 4096) return PTB_ERR_INVALID; c->build_threads = (int)value; return PTB_OK;
@@ -1868,12 +1683,6 @@ int ptb_kat(ptb_ctx* c, int which, const ptb_camera* cam, int W, int H, const do
     if (!c || !in || !out || n <= 0) return PTB_ERR_INVALID;
     CK(cudaSetDevice(c->device));
     if (which == PTB_KAT_MERL_EVAL && (!c->committed || c->host.merl_tables.empty())) { c->err = "kat: MERL needs a committed scene with a table"; return PTB_ERR_STATE; }
-    if (which == PTB_KAT_NODE_HALF) {
-        if (!PTB_NODE_HALF) { c->err = "kat: this build traverses with the float node test"; return PTB_ERR_UNSUPPORTED; }
-        if (!c->committed || !c->sc.has_mesh) { c->err = "kat: the node test needs a committed scene with a mesh"; return PTB_ERR_STATE; }
-        const double n_nodes = (double)(c->bytes_nodes / (int64_t)sizeof(Node8));
-        for (int k = 0; k < n; k++) if (!(in[(size_t)k * is + 7] >= 0 && in[(size_t)k * is + 7] < n_nodes)) { c->err = "kat: node index out of range"; return PTB_ERR_INVALID; }
-    }
     CameraDev cd;
     memset(&cd, 0, sizeof(cd));
     if (cam) camera_from_abi(cd, cam, W, H);

@@ -14,7 +14,7 @@ namespace ptb {
 struct Bvh8Stats {
     int64_t n_nodes = 0, n_binary_nodes = 0, leaves = 0;
     int depth = 0;
-    int half_c = 0;                        // the scene's half grid (ptb_bvh8.h half_grid_c), SceneDev::half_c
+    int e_floor = 0;                       // no node cell finer than 2^e_floor = 2^-25 of the root's cells (the builder's and the refit's floor)
     std::vector<uint32_t> level_start;     // nodes are emitted breadth first: level l is [level_start[l], level_start[l + 1]) (refit walks them bottom-up)
 };
 // verts9: 9 floats per triangle (world space).  leaf_order[k] = input index of the k-th stored triangle.  boxes6 (or null): lo[3], hi[3]
@@ -105,7 +105,6 @@ void build_matrix(HostObject& o);          // Object::build_matrix (Geometry.h:3
 inline void scene_header(SceneDev& sc, FlatScene& f) {
     sc.n_objects = (int32_t)f.objects.size();
     sc.has_mesh = f.nodes.empty() ? 0 : 1;
-    sc.half_c = f.bvh.half_c;
     sc.envW = f.envW; sc.envH = f.envH; sc.has_envmap = (f.envW > 0 && f.envH > 0) ? 1 : 0;
     sc.envmap_intensity = f.envmap_intensity; sc.lightPower = f.lightPower; sc.radiusLight = f.radiusLight;
     sc.centerLight = v3(f.centerLight[0], f.centerLight[1], f.centerLight[2]);

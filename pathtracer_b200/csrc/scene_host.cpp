@@ -377,7 +377,6 @@ int HostScene::flatten(FlatScene& out, std::string& err) {
     std::vector<Src> src(n_tri);
     std::vector<float> boxes6;      // only with yarns in the scene: the box a covering triangle enters the BVH with (NaN: its own)
     if (n_tri > 0) {
-        static const bool classify = !(getenv("PTB_ALPHA_CLASSIFY") && atoi(getenv("PTB_ALPHA_CLASSIFY")) == 0);   // experiments: 0 = test every alpha-mapped triangle
         int64_t w = 0;
         for (int oi = 0; oi < (int)objects.size(); oi++) {
             const HostObject& o = objects[oi];
@@ -427,12 +426,9 @@ int HostScene::flatten(FlatScene& out, std::string& err) {
                 if (uv_all && group >= 0 && group < (int)o.groups.size() && (o.groups[group].present & SLOT_ALPHA)) {
                     const HostTex& a = o.groups[group].alpha;
                     if (a.W > 0 && a.H > 0) {
-                        cls = ALPHA_TEST;
-                        if (classify) {
-                            if (sats[group].W == 0) sats[group].build(a);
-                            cls = (uint8_t)alpha_class(sats[group], &o.uvs[2 * (size_t)t[3]], &o.uvs[2 * (size_t)t[4]], &o.uvs[2 * (size_t)t[5]]);
-                        }
-                    } else if (a.mult[0] < 0.5f) cls = classify ? ALPHA_INVISIBLE : ALPHA_TEST;   // a constant below 0.5 rejects every hit
+                        if (sats[group].W == 0) sats[group].build(a);
+                        cls = (uint8_t)alpha_class(sats[group], &o.uvs[2 * (size_t)t[3]], &o.uvs[2 * (size_t)t[4]], &o.uvs[2 * (size_t)t[5]]);
+                    } else if (a.mult[0] < 0.5f) cls = ALPHA_INVISIBLE;   // a constant below 0.5 rejects every hit
                     if (cls == ALPHA_OPAQUE && a.W > 0) out.n_tri_alpha_opaque++;
                     else if (cls == ALPHA_INVISIBLE) out.n_tri_alpha_invisible++;
                     else if (cls == ALPHA_TEST) out.n_tri_alpha_tested++;

@@ -1,4 +1,4 @@
-"""One process = one library configuration (environment knobs such as PTB_BVH_COLLAPSE_DP are read at load time):
+"""One process = one library configuration (a variant library built with `make variant` is selected with PTB_LIB_PATH):
 device ms per render for C2/C3/C4 at 1 and 2 pass pipelines, kernel breakdown and traversal counters.
 usage: [ENV=...] python scripts/gpu_ab2.py <tag> [C2:256 C3:128 C4:256]"""
 import os, sys

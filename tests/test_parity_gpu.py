@@ -9,7 +9,7 @@ import os
 import numpy as np
 import pytest
 from golden_scenes import ANIM_SCENES, BRANCH_SCENES, SCENES
-from parity_cases import (EDGE_VARIANTS, case_branch_converged, case_branch_errors, case_branch_passes, case_branch_scene, case_converged, case_sss_converged, case_denoiser_inputs, case_edge, case_errors, case_kats, case_merl_index_fast, case_node_test_half, case_triangle_soup, case_passes_and_shards,
+from parity_cases import (EDGE_VARIANTS, case_branch_converged, case_branch_errors, case_branch_passes, case_branch_scene, case_converged, case_sss_converged, case_denoiser_inputs, case_edge, case_errors, case_kats, case_merl_index_fast, case_triangle_soup, case_passes_and_shards,
                           case_progressive, case_scene, mode_scene_exotic, case_yarn_cloth, case_yarn_from_inside, check_ids, check_images)
 
 from pathtracer_b200 import _abi, scenes
@@ -33,20 +33,6 @@ def test_kats_gpu(gpu):
 def test_triangle_soup_gpu(gpu, port):
     """irregular trees (random unconnected triangles): persistent-warp traversal, valid24 / compact indices, postponed triangle groups"""
     case_triangle_soup(gpu, port, n=20000, agree=0.998)   # 6912 pixels full of silhouette edges: a handful may flip under FMA contraction
-
-
-def test_node_test_with_half_factors_is_conservative(gpu):
-    """FHFMA node step of k_trace (an optional build, -DPTB_NODE_HALF=1) against the float slab test on the same quantised boxes"""
-    from pathtracer_b200 import scenes as _sc, _abi as _ab
-    rt = _sc.config_C2(gpu, 8, 8, 1, nv=8, env=(8, 4)).commit()
-    try:
-        rt.kat(_ab.KAT_NODE_HALF, np.array([[0, 0, 0, 0, 0, 1, 1e30, 0]], np.float64))
-    except Exception as e:
-        if "float node test" in str(e): pytest.skip("this build traverses with the float node test (the default)")
-        raise
-    finally:
-        rt.close()
-    case_node_test_half(gpu)
 
 
 def test_merl_index_fast_gpu(gpu):
@@ -96,17 +82,25 @@ def test_animation_recommit_gpu(gpu, port):
 def test_animation_refit_gpu(gpu, port):
     """Key-framed scene re-posed WITHOUT a rebuild: commit once, then set_frame + render per frame (the BVH8 keeps its topology, the
     triangles are re-derived on the device and the boxes refitted).  Every frame equals a context committed at that frame, agrees
-    with the oracle at that frame, and going back to the commit frame reproduces its image."""
-    rt = scenes.config_anim(gpu, 64, 64, 2, frame=0).commit()
+    with the oracle at that frame, and going back to the commit frame reproduces its image.  The torus is committed at 1/32 of its
+    frame-2 size, so frame 2 re-poses a mesh 32x the size it was committed at: the refit takes whatever cell sizes the boxes need."""
+    def mk(L, frame):
+        rt = scenes.config_anim(L, 64, 64, 2, frame=frame)
+        torus = rt.s.objects[-1]
+        torus.scale_keyframes[0.0] = torus.scale_keyframes[2.0] / 32
+        torus.translation_keyframes[0.0] = torus.translation_keyframes[2.0]
+        torus.rotation_keyframes[0.0] = torus.rotation_keyframes[2.0]
+        return rt
+    rt = mk(gpu, 0).commit()
     first = rt.render_image_nopreviz().copy()
     launches = rt.stats["kernel_launches"]
-    for fr in (5, 12, 3, 8):
+    for fr in (5, 12, 3, 8, 2):
         img = rt.set_frame(fr).render_image_nopreviz().copy()
         info = rt.scene_info()
         assert 0 < info["ms_refit"] < 50.0        # a re-pose happened and was measured (the bound at size: the million-triangle case below)
-        fresh = scenes.config_anim(gpu, 64, 64, 2, frame=fr).commit()
+        fresh = mk(gpu, fr).commit()
         assert np.allclose(img, fresh.render_image_nopreviz(), rtol=1e-5, atol=1e-3), fr
-        ora = scenes.config_anim(port, 64, 64, 2, frame=fr).commit()
+        ora = mk(port, fr).commit()
         check_ids(rt, ora, agree=0.998)
         check_images(img, ora.render_image_nopreviz(), frac=0.01)
     assert rt.stats["kernel_launches"] == launches
