@@ -38,7 +38,6 @@ using namespace ptb;
 //   [2*b] paths queued for bounce b          [2*b+1] shadow rays queued for the BVH at bounce b
 //   [CUR + 2*b] / [CUR + 2*b+1]  work cursors of the persistent trace kernels (closest / any-hit) of bounce b
 //   [SQ + b]  intersection_shadow-equivalent queries made at bounce b (ray statistics)
-#define PTB_MAX_BOUNCES 64
 #define PTB_CNT_CUR (2 * (PTB_MAX_BOUNCES + 1))
 #define PTB_CNT_SQ (4 * (PTB_MAX_BOUNCES + 1))
 #define PTB_CNT_ALLOC (5 * (PTB_MAX_BOUNCES + 1))       // branching renders: side-branch slots handed out in this pass
@@ -46,11 +45,8 @@ using namespace ptb;
 #define PTB_CNT_PROBE (5 * (PTB_MAX_BOUNCES + 1) + 2)   // subsurface probes emitted at the current level
 #define PTB_CNT_DEFER (5 * (PTB_MAX_BOUNCES + 1) + 3)   // [+ 2*b] / [+ 2*b + 1]: rays of bounce b (closest / any-hit) that left candidates for k_exact
 #define PTB_N_COUNTERS (7 * (PTB_MAX_BOUNCES + 1) + 3)
-#define PTB_DEFER_K 4    /* candidates a ray can leave for k_exact; a ray with more is re-traced there with the immediate exact test */
 // 64-bit totals: 0 closest rays, 1 shadow rays, 2/3 node visits / triangle tests of the closest-hit trace, 4/5 of the any-hit trace
 #define PTB_N_TOTALS 10   /* 0-1 rays, 2-5 node visits / triangle tests (closest, any hit), 6-9 triangle-phase warp iterations and their packed minimum (COUNT kernels) */
-#define PTB_BRANCH_MAX_LEVELS 512
-#define PTB_MAX_PIPES 4
 
 // ------------------------------------------------------------------------------------------------ kernels
 __global__ void __launch_bounds__(256) k_rpp(float* rpp, int n) {
@@ -537,41 +533,17 @@ __global__ void __launch_bounds__(256) k_resolve(const F4* accum, size_t n, floa
     resolve_pixel(accum, idx, gamma, imagedouble, sample_count, image);
 }
 
-// has_denoiser tail of render_image_nopreviz (Raytracer.cpp:1676-1693): colour and albedo means, and the two normal images:
-// `normalImage` as the reference computes it (it sums the COLOUR buffers there, 1680-1682, then normalises) and the normalised sum of
-// the first-hit shading normals that line was meant to produce.
 __global__ void __launch_bounds__(256) k_resolve_denoiser(const F4* accum, const F4* albedo, const F4* normal, size_t n, float* imagedouble, float* sample_count,
                                                           float* albedoImage, float* normalImage, float* first_hit_normal) {
     const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= n) return;
-    const F4 a = accum[idx], k = albedo[idx], m = normal[idx];
-    const float nn = sqrtf(a.x * a.x + a.y * a.y + a.z * a.z), nm = sqrtf(m.x * m.x + m.y * m.y + m.z * m.z);
-    if (imagedouble) { imagedouble[idx * 3] = a.x / a.w; imagedouble[idx * 3 + 1] = a.y / a.w; imagedouble[idx * 3 + 2] = a.z / a.w; }
-    if (sample_count) sample_count[idx] = a.w;
-    if (albedoImage) { albedoImage[idx * 3] = k.x / a.w; albedoImage[idx * 3 + 1] = k.y / a.w; albedoImage[idx * 3 + 2] = k.z / a.w; }
-    if (normalImage) { normalImage[idx * 3] = a.x / nn; normalImage[idx * 3 + 1] = a.y / nn; normalImage[idx * 3 + 2] = a.z / nn; }
-    if (first_hit_normal) { first_hit_normal[idx * 3] = m.x / nm; first_hit_normal[idx * 3 + 1] = m.y / nm; first_hit_normal[idx * 3 + 2] = m.z / nm; }
+    resolve_denoiser_pixel(accum, albedo, normal, idx, imagedouble, sample_count, albedoImage, normalImage, first_hit_normal);
 }
 
-// tail of the progressive Raytracer::render_image (Raytracer.cpp:1540-1547): imagedouble stays the un-normalised sums, the display
-// image divides by max(sample_count, 1)
 __global__ void __launch_bounds__(256) k_resolve_progressive(const F4* accum, size_t n, float gamma, float* imagedouble, float* sample_count, uint8_t* image) {
     const size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= n) return;
-    const F4 a = accum[idx];
-    if (imagedouble) { imagedouble[idx * 3] = a.x; imagedouble[idx * 3 + 1] = a.y; imagedouble[idx * 3 + 2] = a.z; }
-    if (sample_count) sample_count[idx] = a.w;
-    if (image) {
-        const double ig = (double)(1 / gamma);
-        const float d = fmaxf(a.w, 1.f);
-        const float c[3] = {a.x, a.y, a.z};
-        for (int q = 0; q < 3; q++) {
-            double v = 255. * pow((double)c[q] / 196964.7 / (double)d, ig);
-            v = v > 0. ? v : 0.;
-            v = v < 255. ? v : 255.;
-            image[idx * 3 + q] = (uint8_t)v;
-        }
-    }
+    resolve_progressive_pixel(accum, idx, gamma, imagedouble, sample_count, image);
 }
 
 __global__ void __launch_bounds__(128) k_primary(SceneDev sc, CameraDev cam, int W, int H, int32_t* obj_id, int32_t* tri_id, float* tout) {
@@ -596,51 +568,13 @@ __global__ void __launch_bounds__(256) k_shard_pack(const F4* rgbw, F4* packed, 
                                                     int rank, int count, long long n_packed, int unpack) {
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= n_packed) return;
-    const int side = tile + 2 * apron;
-    const long long per = (long long)side * side;
-    const int lt = (int)(idx / per);
-    const int r = (int)(idx - (long long)lt * per);
-    const int tile_id = rank + lt * count;
-    if (tile_id >= n_tiles_total) return;
-    int ty, tx;
-    tile_physical(tile_id, tiles_x, shift, ty, tx);
-    const int i = ty * tile - apron + r / side, j = tx * tile - apron + r % side;
-    const bool inside = i >= 0 && i < H && j >= 0 && j < W;
-    if (!unpack) {
-        const int tiles_y = (H + tile - 1) / tile;
-        const bool send = shard_block_sends(tile_id, i, j, W, H, tile, apron, tiles_x, tiles_y, rank, count, shift);
-        F4 z; z.x = z.y = z.z = z.w = 0;
-        packed[idx] = send ? rgbw[(size_t)(H - 1 - i) * W + j] : z;
-    } else if (inside) {
-        const F4 v = packed[idx];
-        if (v.x != 0.f || v.y != 0.f || v.z != 0.f || v.w != 0.f) RedAddV4()(const_cast<F4*>(rgbw) + (size_t)(H - 1 - i) * W + j, v);
-    }
+    shard_texel(const_cast<F4*>(rgbw), packed, idx, W, H, tile, apron, tiles_x, n_tiles_total, shift, rank, count, unpack, RedAddV4());
 }
 
 __global__ void k_kat(int which, SceneDev sc, CameraDev cam, FilterDev filt, int W, int H, const double* in, int n, int is, double* out, int os) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= n) return;
-    const double* a = in + (size_t)k * is;
-    double* o = out + (size_t)k * os;
-    switch (which) {
-    case PTB_KAT_PCG32: { Pcg32 e = pcg32_seed((uint64_t)a[0], (uint64_t)a[1]); for (int q = 0; q < 4; q++) o[q] = (double)pcg32_next(e); } break;
-    case PTB_KAT_LATTICE: { float x, y; extensible_lattice_2d((uint32_t)a[0], x, y); o[0] = x; o[1] = y; } break;
-    case PTB_KAT_CAMERA: { V3 ro, rd; camera_ray(cam, (int)a[0], (int)a[1], (float)a[2], (float)a[3], (float)a[4], (float)a[5], ro, rd);
-        o[0] = ro.x; o[1] = ro.y; o[2] = ro.z; o[3] = rd.x; o[4] = rd.y; o[5] = rd.z; } break;
-    case PTB_KAT_RANDOM_COS: { V3 v = random_cos(v3((float)a[0], (float)a[1], (float)a[2]), (float)a[3], (float)a[4]); o[0] = v.x; o[1] = v.y; o[2] = v.z; } break;
-    case PTB_KAT_RANDOM_PHONG: { V3 v = random_phong(v3((float)a[0], (float)a[1], (float)a[2]), (float)a[3], (float)a[4], (float)a[5]); o[0] = v.x; o[1] = v.y; o[2] = v.z; } break;
-    case PTB_KAT_PHONG_EVAL: { V3 v = phong_eval(v3((float)a[0], (float)a[1], (float)a[2]), v3((float)a[3], (float)a[4], (float)a[5]), v3((float)a[6], (float)a[7], (float)a[8]),
-                                               v3((float)a[9], (float)a[10], (float)a[11]), v3((float)a[12], (float)a[13], (float)a[14]), v3((float)a[15], (float)a[16], (float)a[17]));
-        o[0] = v.x; o[1] = v.y; o[2] = v.z; } break;
-    case PTB_KAT_MERL_EVAL: { V3 v = merl_eval(sc.merl, v3((float)a[0], (float)a[1], (float)a[2]), v3((float)a[3], (float)a[4], (float)a[5]), v3((float)a[6], (float)a[7], (float)a[8]));
-        o[0] = v.x; o[1] = v.y; o[2] = v.z; } break;
-    case PTB_KAT_FAST_EXP: o[0] = fast_exp(a[0]); break;
-    case PTB_KAT_FAST_NORMALIZE: { V3 v = fast_normalize(v3((float)a[0], (float)a[1], (float)a[2])); o[0] = v.x; o[1] = v.y; o[2] = v.z; } break;
-    case PTB_KAT_RANDOM_PER_PIXEL: { float x, y; random_per_pixel((uint32_t)a[0], x, y); o[0] = x; o[1] = y; } break;
-    case PTB_KAT_FILTER_RATIO: { int b0, b1, b2, b3; o[0] = filter_ratio(filt, (int)a[0], (int)a[1], W, H, b0, b1, b2, b3); } break;
-    case PTB_KAT_MERL_INDEX: { int f, e; merl_index_both(v3((float)a[0], (float)a[1], (float)a[2]), v3((float)a[3], (float)a[4], (float)a[5]), f, e); o[0] = f; o[1] = e; } break;
-    default: break;
-    }
+    kat_one(which, sc, cam, filt, W, H, in + (size_t)k * is, out + (size_t)k * os);
 }
 
 // ------------------------------------------------------------------------------------------------ context
@@ -722,11 +656,7 @@ static void free_scene(ptb_ctx* c) {
     c->scene_allocs.clear();
 }
 static void free_pool(ptb_ctx* c) {
-    void* ptrs[] = {c->pool.ray_o, c->pool.ray_d, c->pool.weight, c->pool.radiance, c->pool.hit, c->pool.rng, c->pool.pixel,
-                    c->pool.sh_o, c->pool.sh_d, c->pool.sh_c, c->d_queue[0], c->d_queue[1], c->pool.aov_n, c->pool.aov_kd, c->pool.root, c->pool.probe_o, c->pool.probe_d, c->pool.probe_x, c->pool.hit2, c->pool.defer_prims, c->pool.defer_rays};
-    for (void* p : ptrs) if (p) cudaFree(p);
-    memset(&c->pool, 0, sizeof(c->pool));
-    c->d_queue[0] = c->d_queue[1] = nullptr;
+    for (const PoolArray& a : pool_arrays(c->pool, c->d_queue)) { if (*a.ptr) cudaFree(*a.ptr); *a.ptr = nullptr; }
     c->pool_cap = 0;
 }
 
@@ -746,32 +676,9 @@ static int ensure_pool(ptb_ctx* c, int64_t paths, bool aov = false, bool branch 
     paths = std::max(paths, c->pool_cap);
     aov = aov || c->pool.aov_n; branch = branch || c->pool.root; sss = sss || c->pool.hit2;
     free_pool(c);
-    const size_t n = (size_t)paths;
-    CK(cudaMalloc((void**)&c->pool.ray_o, n * sizeof(F4)));
-    CK(cudaMalloc((void**)&c->pool.ray_d, n * sizeof(F4)));
-    CK(cudaMalloc((void**)&c->pool.weight, n * sizeof(F4)));
-    CK(cudaMalloc((void**)&c->pool.radiance, n * sizeof(F4)));
-    CK(cudaMalloc((void**)&c->pool.hit, n * sizeof(F4)));
-    CK(cudaMalloc((void**)&c->pool.rng, n * sizeof(uint64_t)));
-    CK(cudaMalloc((void**)&c->pool.pixel, n * sizeof(uint32_t)));
-    CK(cudaMalloc((void**)&c->pool.sh_o, n * sizeof(F4)));
-    CK(cudaMalloc((void**)&c->pool.sh_d, n * sizeof(F4)));
-    CK(cudaMalloc((void**)&c->pool.sh_c, n * sizeof(F4)));
-    CK(cudaMalloc((void**)&c->d_queue[0], n * sizeof(uint32_t)));
-    CK(cudaMalloc((void**)&c->d_queue[1], n * sizeof(uint32_t)));
-    CK(cudaMalloc((void**)&c->pool.defer_prims, n * PTB_DEFER_K * sizeof(uint32_t)));
-    CK(cudaMalloc((void**)&c->pool.defer_rays, n * sizeof(U2)));
-    if (aov) {
-        CK(cudaMalloc((void**)&c->pool.aov_n, n * sizeof(F4)));
-        CK(cudaMalloc((void**)&c->pool.aov_kd, n * sizeof(F4)));
-    }
-    if (branch) CK(cudaMalloc((void**)&c->pool.root, n * sizeof(uint32_t)));
-    if (sss) {
-        CK(cudaMalloc((void**)&c->pool.probe_o, n * sizeof(F4)));
-        CK(cudaMalloc((void**)&c->pool.probe_d, n * sizeof(F4)));
-        CK(cudaMalloc((void**)&c->pool.probe_x, n * sizeof(F4)));
-        CK(cudaMalloc((void**)&c->pool.hit2, n * sizeof(F4)));
-    }
+    const bool need[] = {true, aov, branch, sss};   // by PoolArray::need
+    for (const PoolArray& a : pool_arrays(c->pool, c->d_queue))
+        if (need[a.need]) CK(cudaMalloc(a.ptr, (size_t)paths * a.bytes));
     c->pool_cap = paths;
     return PTB_OK;
 }
@@ -1093,25 +1000,8 @@ int ptb_commit(ptb_ctx* c) {
 }
 
 static int frame_setup(ptb_ctx* c, const ptb_camera* cam, const ptb_params* p, FrameDev& f) {
-    if (!cam || !p || p->W <= 0 || p->H <= 0 || p->nrays <= 0 || p->nb_bounces < 0 || p->nb_bounces > PTB_MAX_BOUNCES || !(p->sigma_filter > 0)) {
-        c->err = "render: invalid parameters"; return PTB_ERR_INVALID;
-    }
-    if ((int)ceilf(p->sigma_filter * 2) > PTB_MAX_FILTER) { c->err = "render: sigma_filter too large (filter_size > 4)"; return PTB_ERR_UNSUPPORTED; }
-    if ((int64_t)p->W * p->H >= ((int64_t)1 << 31)) { c->err = "render: frame too large"; return PTB_ERR_UNSUPPORTED; }
-    memset(&f, 0, sizeof(f));
-    camera_from_abi(f.cam, cam, p->W, p->H);
-    filter_setup(f.filter, p->sigma_filter);
-    f.W = p->W; f.H = p->H; f.nb_bounces = p->nb_bounces; f.seed = p->seed;
-    f.tile = p->tile_size > 0 ? p->tile_size : ptb_default_tile(p->shard_count);
-    // a splat reaches ceil(2 sigma) pixels into the neighbouring tiles and the gather looks at the 3x3 tile neighbourhood only
-    if (f.tile < (int)ceilf(p->sigma_filter * 2) || f.tile > 4096) { c->err = "render: tile_size must lie in [ceil(2*sigma_filter), 4096]"; return PTB_ERR_INVALID; }
-    f.tiles_x = (p->W + f.tile - 1) / f.tile; f.tiles_y = (p->H + f.tile - 1) / f.tile;
-    f.shard_count = p->shard_count > 0 ? p->shard_count : 1;
-    f.shard_rank = p->shard_rank;
-    if (f.shard_rank < 0 || f.shard_rank >= f.shard_count) { c->err = "render: shard_rank out of range"; return PTB_ERR_INVALID; }
-    f.tile_shift = shard_tile_shift(f.tiles_x, f.shard_count);
-    const int total_tiles = f.tiles_x * f.tiles_y;
-    f.n_my_tiles = total_tiles > f.shard_rank ? (total_tiles - f.shard_rank + f.shard_count - 1) / f.shard_count : 0;
+    const int rc = frame_geometry(cam, p, f, c->err);
+    if (rc) return rc;
     // randomPerPixel (prepare_render): regenerated when the frame size changes
     const int64_t npix = (int64_t)p->W * p->H;
     if (c->rpp_n != npix) {
@@ -1148,281 +1038,274 @@ struct LaunchTimer {
 static PoolDev pool_slice(const PoolDev& p, size_t off) {
     if (off == 0) return p;
     PoolDev s = p;
-    F4** f4s[] = {&s.ray_o, &s.ray_d, &s.weight, &s.radiance, &s.hit, &s.sh_o, &s.sh_d, &s.sh_c, &s.aov_n, &s.aov_kd, &s.probe_o, &s.probe_d, &s.probe_x, &s.hit2};
-    for (F4** q : f4s) if (*q) *q += off;
-    if (s.rng) s.rng += off;
-    if (s.pixel) s.pixel += off;
-    if (s.root) s.root += off;
-    if (s.defer_prims) s.defer_prims += off * PTB_DEFER_K;
-    if (s.defer_rays) s.defer_rays += off;
+    for (const PoolArray& a : pool_arrays(s))
+        if (*a.ptr) *a.ptr = (char*)*a.ptr + off * a.bytes;
     return s;
 }
 
-// the pass loop; accumulates into d_rgbw (device, W*H float4)
-// samples k_first .. k_first + nrays - 1 of every pixel of the shard
+}  // extern "C"
+
+// One pass pipeline: its stream, pool slice, bounce queues and counters (pipe 0 is the context's own; branching renders only use it)
+struct Pipe { cudaStream_t stream; PoolDev pool; uint32_t *queue[2], *counters; };
+// What a render counts on the host: kernel launches, and the rays of the branching level loop
+struct RenderTally { uint64_t launches = 0; unsigned long long branch_closest = 0, branch_shadow = 0; };
+
+// One BVH query of a queue: k_trace (its COUNT instantiation with PTB_OPT_COUNT_TRAVERSAL), then k_exact for the candidates it left
+template <bool ANY_HIT, bool BRANCH>
+static void launch_trace(ptb_ctx* c, unsigned grid, cudaStream_t st, const PoolDev& p, const uint32_t* queue, const uint32_t* count, int n_static,
+                         uint32_t* cursor, uint32_t* defer_count) {
+    if (c->count_traversal) k_trace<ANY_HIT, true, BRANCH><<<grid, 128, 0, st>>>(c->sc, p, queue, count, n_static, cursor, c->d_totals, c->refill_below, c->tri_den, c->tri_min_pct, defer_count);
+    else k_trace<ANY_HIT, false, BRANCH><<<grid, 128, 0, st>>>(c->sc, p, queue, count, n_static, cursor, c->d_totals, c->refill_below, c->tri_den, c->tri_min_pct, defer_count);
+    k_exact<ANY_HIT, BRANCH><<<c->exact_blocks, 128, 0, st>>>(c->sc, p, defer_count);
+}
+
+// The queues and counters of one shade launch; `items` bounds the entries of its queue (one thread each)
+struct ShadeIO {
+    unsigned items;
+    const uint32_t *queue, *count;
+    int n_static;
+    uint32_t *next_queue, *next_count, *shadow_count, *shadow_queries;
+};
+template <bool MERL, int MINB, bool AOV, bool EXOTIC>
+static void shade_linear(ptb_ctx* c, const FrameDev& f, const PoolDev& p, cudaStream_t st, const ShadeIO& s) {
+    k_shade<MERL, MINB, AOV, EXOTIC><<<(s.items + PTB_SHADE_BLOCK - 1) / PTB_SHADE_BLOCK, PTB_SHADE_BLOCK, 0, st>>>(c->sc, f, p, s.queue, s.count, s.n_static, s.next_queue,
+                                                                                                               s.next_count, s.shadow_count, s.shadow_queries);
+}
+template <bool MERL>
+static void shade_branch(ptb_ctx* c, const FrameDev& f, const ShadeIO& s, uint32_t n_roots, const F4* resume) {
+    k_shade_branch<MERL><<<(s.items + 127) / 128, 128, 0, c->stream>>>(c->sc, f, c->pool, s.queue, s.count, s.n_static, s.next_queue, s.next_count, s.shadow_count,
+                                                                        s.shadow_queries, c->d_counters + PTB_CNT_ALLOC, n_roots, (uint32_t)c->pool_cap,
+                                                                        c->d_counters + PTB_CNT_DROPS, c->d_counters + PTB_CNT_PROBE, resume);
+}
+// The shade launch of a bounce (linear renders) or a level (branching renders, `n_roots` samples, `resume`: the answered subsurface
+// probes to shade again, or null).  Scenes with Cylinder / PointSet / Yarns objects take the k_shade that carries their code (not
+// register-squeezed); the AOV kernels shade the camera rays of a denoiser-input render.
+static void launch_shade(ptb_ctx* c, const FrameDev& f, const PoolDev& p, cudaStream_t st, const ShadeIO& s, bool branch, bool aov_first,
+                         uint32_t n_roots = 0, const F4* resume = nullptr) {
+    const bool merl = c->has_merl;
+    if (branch) merl ? shade_branch<true>(c, f, s, n_roots, resume) : shade_branch<false>(c, f, s, n_roots, resume);
+    else if (c->sc.has_exotic && aov_first) merl ? shade_linear<true, 5, true, true>(c, f, p, st, s) : shade_linear<false, 6, true, true>(c, f, p, st, s);
+    else if (c->sc.has_exotic) merl ? shade_linear<true, 5, false, true>(c, f, p, st, s) : shade_linear<false, 6, false, true>(c, f, p, st, s);
+    else if (aov_first) merl ? shade_linear<true, 5, true, false>(c, f, p, st, s) : shade_linear<false, 6, true, false>(c, f, p, st, s);
+    else merl ? shade_linear<true, 8, false, false>(c, f, p, st, s) : shade_linear<false, 8, false, false>(c, f, p, st, s);
+}
+
+// The linear schedule of one pass on its pipeline: per bounce, closest hits, shading, shadow rays.  Every kernel reads its item count
+// from the pipeline's counters, so the host never waits.
+static void run_bounces(ptb_ctx* c, const FrameDev& f, const Pipe& pp, int n_paths, int n_pipes, LaunchTimer& lt, RenderTally& tally) {
+    const bool mesh = c->sc.has_mesh != 0, aov = f.accum_albedo != nullptr;
+    uint32_t* const pc = pp.counters;
+    // persistent grid: as many blocks as are resident at once, but no more than the queue can feed
+    const unsigned gt = (unsigned)std::max(1, std::min<int>(n_pipes > 1 ? c->trace_blocks_piped : c->trace_blocks, (n_paths + 127) / 128));
+    for (int b = 0; b < f.nb_bounces; b++) {
+        const uint32_t* q = b == 0 ? nullptr : pp.queue[b & 1];
+        const uint32_t* cnt = b == 0 ? nullptr : pc + 2 * b;
+        if (mesh) {
+            lt.begin(1 | (b << 8), pp.stream);
+            launch_trace<false, false>(c, gt, pp.stream, pp.pool, q, cnt, n_paths, pc + PTB_CNT_CUR + 2 * b, pc + PTB_CNT_DEFER + 2 * b);
+            lt.end();
+            tally.launches += 2;
+        }
+        lt.begin(2 | (b << 8), pp.stream);
+        launch_shade(c, f, pp.pool, pp.stream, {(unsigned)n_paths, q, cnt, n_paths, pp.queue[(b + 1) & 1], pc + 2 * (b + 1), pc + 2 * b + 1, pc + PTB_CNT_SQ + b}, false, aov && b == 0);
+        lt.end();
+        tally.launches++;
+        if (mesh) {
+            lt.begin(3 | (b << 8), pp.stream);
+            launch_trace<true, false>(c, gt, pp.stream, pp.pool, nullptr, pc + 2 * b + 1, 0, pc + PTB_CNT_CUR + 2 * b + 1, pc + PTB_CNT_DEFER + 2 * b + 1);
+            lt.end();
+            tally.launches += 2;
+        }
+    }
+}
+
+// The branching schedule of one pass: a level-synchronous walk of the contribution tree on the context's stream, with the host reading
+// each level's queue lengths (these are the reference's compositing / medium modes, not the benchmarked path).  Counter slots alternate
+// with the level's parity.  A straight-through ray keeps its depth (Raytracer.cpp:529-531), and at grazing angles the shading-normal
+// offset can put it back in front of the ghost triangle it just crossed: the reference then re-hits it for up to hundreds of iterations
+// (its ring simply keeps turning).  Here such chains end after PTB_BRANCH_MAX_LEVELS.
+static int run_branch_levels(ptb_ctx* c, const FrameDev& f, int n_paths, unsigned long long valid_here, LaunchTimer& lt, RenderTally& tally) {
+    uint32_t n_level = (uint32_t)n_paths;
+    const bool mesh = c->sc.has_mesh != 0;
+    for (int b = 0; b < PTB_BRANCH_MAX_LEVELS && n_level > 0 && f.nb_bounces > 0; b++) {
+        const int s = b & 1, ns = (b + 1) & 1, kind = std::min(b, 63) << 8;
+        uint32_t* cnt_q = c->d_counters + 2 * s; uint32_t* cnt_sh = c->d_counters + 2 * s + 1; uint32_t* cnt_next = c->d_counters + 2 * ns;
+        uint32_t* cur = c->d_counters + PTB_CNT_CUR + 2 * s; uint32_t* cnt_sq = c->d_counters + PTB_CNT_SQ + s;
+        uint32_t* cnt_def = c->d_counters + PTB_CNT_DEFER + 2 * s;
+        if (b >= 1) {
+            CK(cudaMemsetAsync(cnt_next, 0, sizeof(uint32_t), c->stream));
+            if (b >= 2) {
+                CK(cudaMemsetAsync(cnt_sh, 0, sizeof(uint32_t), c->stream));
+                CK(cudaMemsetAsync(cur, 0, 2 * sizeof(uint32_t), c->stream));
+                CK(cudaMemsetAsync(cnt_sq, 0, sizeof(uint32_t), c->stream));
+                CK(cudaMemsetAsync(cnt_def, 0, 2 * sizeof(uint32_t), c->stream));
+            }
+            CK(cudaMemsetAsync(c->d_counters + PTB_CNT_PROBE, 0, sizeof(uint32_t), c->stream));
+        }
+        const uint32_t* q = b == 0 ? nullptr : c->d_queue[s];
+        const uint32_t* cnt = b == 0 ? nullptr : cnt_q;
+        if (mesh) {
+            const unsigned gt = (unsigned)std::max(1, std::min<int>(c->trace_blocks, (int)((n_level + 127) / 128)));
+            lt.begin(1 | kind);
+            launch_trace<false, false>(c, gt, c->stream, c->pool, q, cnt, n_paths, cur, cnt_def);
+            lt.end();
+            tally.launches += 2;
+        }
+        lt.begin(2 | kind);
+        launch_shade(c, f, c->pool, c->stream, {n_level, q, cnt, n_paths, c->d_queue[ns], cnt_next, cnt_sh, cnt_sq}, true, false, (uint32_t)n_paths);
+        lt.end();
+        tally.launches++;
+        if (c->sc.has_sss) {   // answer this level's subsurface probes, then shade those hits for good
+            uint32_t h_probe = 0;
+            CK(cudaMemcpyAsync(&h_probe, c->d_counters + PTB_CNT_PROBE, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+            CK(cudaStreamSynchronize(c->stream));
+            if (h_probe > 0) {
+                k_probe<<<(h_probe + 127) / 128, 128, 0, c->stream>>>(c->sc, c->pool, (int)h_probe);
+                lt.begin(2 | kind);
+                launch_shade(c, f, c->pool, c->stream, {h_probe, nullptr, nullptr, (int)h_probe, c->d_queue[ns], cnt_next, cnt_sh, cnt_sq}, true, false, (uint32_t)n_paths,
+                             c->pool.probe_d);
+                lt.end();
+                tally.launches += 2;
+            }
+        }
+        uint32_t h_sh = 0, h_next = 0, h_sq = 0;
+        CK(cudaMemcpyAsync(&h_sh, cnt_sh, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaMemcpyAsync(&h_next, cnt_next, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaMemcpyAsync(&h_sq, cnt_sq, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaStreamSynchronize(c->stream));
+        if (mesh && h_sh > 0) {
+            const unsigned ga = (unsigned)std::max(1, std::min<int>(c->trace_blocks, (int)((h_sh + 127) / 128)));
+            lt.begin(3 | kind);
+            launch_trace<true, true>(c, ga, c->stream, c->pool, nullptr, cnt_sh, 0, cur + 1, cnt_def + 1);
+            lt.end();
+            tally.launches += 2;
+        }
+        tally.branch_closest += b == 0 ? valid_here * (unsigned long long)f.spp_pass : (unsigned long long)n_level;
+        tally.branch_shadow += h_sq;
+        n_level = h_next;
+    }
+    uint32_t drops = 0;
+    CK(cudaMemcpyAsync(&drops, c->d_counters + PTB_CNT_DROPS, sizeof(drops), cudaMemcpyDeviceToHost, c->stream));
+    CK(cudaStreamSynchronize(c->stream));
+    if (drops > 0) {
+        c->err = "branching render: contribution pool exhausted (" + std::to_string(drops) + " side branches dropped); raise PTB_OPT_POOL_PATHS";
+        return PTB_ERR_NOMEM;
+    }
+    return PTB_OK;
+}
+
+// After a render's work has finished: the device totals and the host tally folded into ptb_kernel_times and `stats`, the launch
+// timings of PTB_OPT_TIME_KERNELS, and the PTB_DEBUG_TRI / PTB_DEBUG_BOUNCES reports on stderr.
+static int render_stats(ptb_ctx* c, int nb, unsigned long long samples, const RenderTally& tally, ptb_stats* stats, std::chrono::steady_clock::time_point w0) {
+    unsigned long long t[PTB_N_TOTALS];
+    CK(cudaMemcpy(t, c->d_totals, sizeof(t), cudaMemcpyDeviceToHost));
+    t[0] += tally.branch_closest; t[1] += tally.branch_shadow;
+    ptb_kernel_times& kt = c->ktimes;
+    for (size_t i = 0; i < c->ev_kind.size(); i++) {
+        float ms = 0;
+        cudaEventElapsedTime(&ms, c->ev_pool[2 * i], c->ev_pool[2 * i + 1]);
+        kt.ms[c->ev_kind[i] & 0xff] += ms;
+        kt.launches[c->ev_kind[i] & 0xff]++;
+    }
+    if (getenv("PTB_DEBUG_TRI") && t[6]) {   // triangle phase of k_trace (COUNT kernels): warp iterations, lanes per iteration, packed minimum
+        fprintf(stderr, "[ptb] triangle phase, closest: %llu tests in %llu warp iterations (%.1f lanes each), %llu if packed 32 to an iteration (%.1f %% fewer)\n", t[3], t[6],
+                (double)t[3] / (double)t[6], t[7], 100.0 * (1.0 - (double)t[7] / (double)t[6]));
+        if (t[8]) fprintf(stderr, "[ptb] triangle phase, any hit: %llu tests in %llu warp iterations (%.1f lanes each), %llu if packed (%.1f %% fewer)\n", t[5], t[8], (double)t[5] / (double)t[8], t[9],
+                          100.0 * (1.0 - (double)t[9] / (double)t[8]));
+    }
+    if (getenv("PTB_DEBUG_BOUNCES")) {   // per-bounce launch times of the LAST pass + its queue lengths (diagnostics only)
+        uint32_t cnt[PTB_N_COUNTERS];
+        cudaMemcpy(cnt, c->d_counters, sizeof(cnt), cudaMemcpyDeviceToHost);
+        const size_t per_pass = 2 + 3 * (size_t)nb;
+        const size_t first = c->ev_kind.size() >= per_pass ? c->ev_kind.size() - per_pass : 0;
+        for (size_t i = first; i < c->ev_kind.size(); i++) {
+            float ms = 0;
+            cudaEventElapsedTime(&ms, c->ev_pool[2 * i], c->ev_pool[2 * i + 1]);
+            const int kind = c->ev_kind[i] & 0xff, b = c->ev_kind[i] >> 8;
+            const char* names[] = {"raygen", "closest", "shade", "anyhit", "splat"};
+            const unsigned items = kind == 3 ? cnt[2 * b + 1] : ((kind == 1 || kind == 2) ? (b == 0 ? 0u : cnt[2 * b]) : 0u);
+            fprintf(stderr, "[ptb] %-8s b=%d  %8.3f ms  items=%u\n", names[kind], b, ms, items);
+        }
+    }
+    kt.items[0] = kt.items[4] = samples;
+    kt.items[1] = kt.items[2] = t[0]; kt.items[3] = t[1];
+    kt.node_visits[1] = t[2]; kt.tri_tests[1] = t[3]; kt.node_visits[3] = t[4]; kt.tri_tests[3] = t[5];
+    if (stats) {
+        float ms = 0;
+        CK(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+        memset(stats, 0, sizeof(*stats));
+        stats->samples = samples;
+        stats->rays_closest = t[0]; stats->rays_shadow = t[1]; stats->node_visits = t[2] + t[4]; stats->tri_tests = t[3] + t[5];
+        stats->ms_device = ms;
+        stats->ms_wall = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - w0).count();
+        stats->kernel_launches = tally.launches;
+    }
+    return PTB_OK;
+}
+
+// The pass loop: samples k_first .. k_first + nrays - 1 of every pixel of the shard, accumulated into d_rgbw (device, W*H float4).
+// Every pass is raygen -> bounces (or levels of a branching render) -> splat -> k_totals on its pipeline; the pipelines join on the
+// context's stream at the end.
 static int render_passes(ptb_ctx* c, FrameDev f, int nrays, F4* d_rgbw, ptb_stats* stats, int k_first = 0) {
-    auto w0 = std::chrono::steady_clock::now();
+    const auto w0 = std::chrono::steady_clock::now();
     const int64_t pixel_slots = (int64_t)f.n_my_tiles * f.tile * f.tile;
-    uint64_t launches = 0;
-    unsigned long long branch_closest = 0, branch_shadow = 0;   // ray statistics of the branching level loop (counted on the host)
+    RenderTally tally;
     LaunchTimer lt(c);
     memset(&c->ktimes, 0, sizeof(c->ktimes));
     CK(cudaMemsetAsync(c->d_totals, 0, PTB_N_TOTALS * sizeof(unsigned long long), c->stream));
     CK(cudaEventRecord(c->ev0, c->stream));
-    // count the shard's in-image pixels (edge tiles are partial)
-    unsigned long long valid_pixels = 0;
-    for (int lt = 0; lt < f.n_my_tiles; lt++) {
-        const int tile_id = f.shard_rank + lt * f.shard_count;
-        int ty, tx;
-        tile_physical(tile_id, f.tiles_x, f.tile_shift, ty, tx);
-        const int h = std::min(f.tile, f.H - ty * f.tile), w = std::min(f.tile, f.W - tx * f.tile);
-        valid_pixels += (unsigned long long)h * w;
-    }
+    const unsigned long long valid_pixels = tile_range_pixels(f, 0, pixel_slots);
     if (pixel_slots > 0) {
-        // samples per pixel per pass and pixel slots per pass
-        int64_t pool = std::max<int64_t>(c->pool_paths, 1024);
-        // Branching renders keep every live contribution of a sample in the pool: the continuation reuses its slot, each side
-        // branch takes a new one.  A fogged path forks once per iteration (at most 2^depth - 1 forks per sample), a ghost hit once.
-        const bool branch = c->sc.has_fog || c->sc.has_ghost || c->sc.bgW > 0 || c->sc.has_sss;
-        const int fan = !branch ? 1 : (c->sc.has_fog ? (1 << std::min(f.nb_bounces, 6)) : (c->sc.has_ghost ? 8 : 1));
-        if (branch && f.accum_albedo) { c->err = "denoiser inputs are not available with fog, ghost objects, subsurface scattering or a background photograph"; return PTB_ERR_UNSUPPORTED; }
-        const int64_t pool_cap_slots = pool;
-        pool = std::max<int64_t>(pool / fan, 1024);
-        const int n_pipes = branch ? 1 : std::max(1, std::min(c->n_pipes, PTB_MAX_PIPES));
-        if (n_pipes > 1 && pixel_slots * nrays < pool * n_pipes)   // a frame smaller than the pools is still split so that every pipeline gets a pass
-            pool = std::max<int64_t>((pixel_slots * nrays + n_pipes - 1) / n_pipes, (int64_t)1 << 18);
-        int spp_pass; int64_t slots_pass;
-        if (pixel_slots * nrays <= pool) { spp_pass = nrays; slots_pass = pixel_slots; }
-        else if (pixel_slots <= pool) { spp_pass = (int)std::max<int64_t>(1, pool / pixel_slots); slots_pass = pixel_slots; }
-        else { spp_pass = 1; slots_pass = (pool / (f.tile * f.tile)) * (f.tile * f.tile); if (slots_pass <= 0) slots_pass = f.tile * f.tile; }
-        const bool aov = f.accum_albedo != nullptr;
-        const int64_t stride = slots_pass * spp_pass;   // paths per pass = pool slice of one pipeline
-        int rc = ensure_pool(c, branch ? std::max<int64_t>(stride * fan, pool_cap_slots) : stride * n_pipes, aov, branch, c->sc.has_sss != 0);
+        const PassPlan pl = plan_passes(c->sc, f.nb_bounces, f.tile, pixel_slots, nrays, c->pool_paths, c->n_pipes);
+        if (pl.branch && f.accum_albedo) { c->err = "denoiser inputs are not available with fog, ghost objects, subsurface scattering or a background photograph"; return PTB_ERR_UNSUPPORTED; }
+        int rc = ensure_pool(c, pl.pool_paths, f.accum_albedo != nullptr, pl.branch, c->sc.has_sss != 0);
         if (rc) return rc;
-        for (int i = 1; i < n_pipes; i++) {
+        for (int i = 1; i < pl.n_pipes; i++) {
             if (!c->pipe_stream[i]) { CK(cudaStreamCreateWithFlags(&c->pipe_stream[i], cudaStreamNonBlocking)); CK(cudaEventCreateWithFlags(&c->pipe_done[i], cudaEventDisableTiming)); }
             CK(cudaStreamWaitEvent(c->pipe_stream[i], c->ev0, 0));
         }
-        const int nb = f.nb_bounces;
         int64_t pass_index = 0;
-        for (int64_t s0 = 0; s0 < pixel_slots; s0 += slots_pass) {
-            const int64_t ns = std::min(slots_pass, pixel_slots - s0);
-            // valid pixels in this slot range (for the ray statistics)
-            unsigned long long valid_here = 0;
-            {
-                const int tp = f.tile * f.tile;
-                for (int64_t lt = s0 / tp; lt * tp < s0 + ns; lt++) {
-                    const int tile_id = f.shard_rank + (int)lt * f.shard_count;
-                    int ty, tx;
-                    tile_physical(tile_id, f.tiles_x, f.tile_shift, ty, tx);
-                    const int h = std::min(f.tile, f.H - ty * f.tile), w = std::min(f.tile, f.W - tx * f.tile);
-                    valid_here += (unsigned long long)h * w;
-                }
-            }
-            for (int k0 = 0; k0 < nrays; k0 += spp_pass) {
-                f.spp_pass = std::min(spp_pass, nrays - k0);
+        for (int64_t s0 = 0; s0 < pixel_slots; s0 += pl.slots_pass) {
+            const int64_t ns = std::min(pl.slots_pass, pixel_slots - s0);
+            const unsigned long long valid_here = tile_range_pixels(f, s0, ns);   // for the ray statistics
+            for (int k0 = 0; k0 < nrays; k0 += pl.spp_pass) {
+                f.spp_pass = std::min(pl.spp_pass, nrays - k0);
                 f.k0 = k_first + k0;
                 f.slot0 = (int)s0;
                 f.n_pixel_slots = (int)ns;
                 const int n_paths = (int)(ns * f.spp_pass);
-                const unsigned g256 = (unsigned)((n_paths + 255) / 256), g128 = (unsigned)((n_paths + 127) / 128);
-                // this pass's pipeline: stream, pool slice, queues, counters (pipe 0 = the context's own; branching renders only use pipe 0)
-                const int pi = (int)(pass_index++ % n_pipes);
-                cudaStream_t ps = pi ? c->pipe_stream[pi] : c->stream;
-                const PoolDev pp = pool_slice(c->pool, (size_t)pi * (size_t)stride);
-                uint32_t* const pq[2] = {c->d_queue[0] + (size_t)pi * stride, c->d_queue[1] + (size_t)pi * stride};
-                uint32_t* const pc = c->d_counters + (size_t)pi * PTB_N_COUNTERS;
-                CK(cudaMemsetAsync(pc, 0, PTB_N_COUNTERS * sizeof(uint32_t), ps));
-                lt.begin(0, ps);
-                if (c->sc.has_exotic) k_raygen<true><<<g256, 256, 0, ps>>>(c->sc, f, pp, n_paths);
-                else k_raygen<false><<<g256, 256, 0, ps>>>(c->sc, f, pp, n_paths);
+                const size_t pi = (size_t)(pass_index++ % pl.n_pipes);
+                const Pipe pp = {pi ? c->pipe_stream[pi] : c->stream, pool_slice(c->pool, pi * (size_t)pl.stride),
+                                 {c->d_queue[0] + pi * pl.stride, c->d_queue[1] + pi * pl.stride}, c->d_counters + pi * PTB_N_COUNTERS};
+                CK(cudaMemsetAsync(pp.counters, 0, PTB_N_COUNTERS * sizeof(uint32_t), pp.stream));
+                lt.begin(0, pp.stream);
+                if (c->sc.has_exotic) k_raygen<true><<<(unsigned)((n_paths + 255) / 256), 256, 0, pp.stream>>>(c->sc, f, pp.pool, n_paths);
+                else k_raygen<false><<<(unsigned)((n_paths + 255) / 256), 256, 0, pp.stream>>>(c->sc, f, pp.pool, n_paths);
                 lt.end();
-                launches++;
-                int levels = nb;
-                if (branch) {
-                    // Level-synchronous walk of the contribution tree; the host reads each level's queue lengths (these are the
-                    // reference's compositing / medium modes, not the benchmarked path).  Counter slots alternate with the level's
-                    // parity.  A straight-through ray keeps its depth (Raytracer.cpp:529-531), and at grazing angles the shading-normal
-                    // offset can put it back in front of the ghost triangle it just crossed: the reference then re-hits it for up to
-                    // hundreds of iterations (its ring simply keeps turning).  Here such chains end after PTB_BRANCH_MAX_LEVELS.
-                    uint32_t n_level = (uint32_t)n_paths;
-                    const bool mesh = c->sc.has_mesh != 0;
-                    int b = 0;
-                    for (; b < PTB_BRANCH_MAX_LEVELS && n_level > 0 && nb > 0; b++) {
-                        const int s = b & 1, ns = (b + 1) & 1;
-                        uint32_t* cnt_q = c->d_counters + 2 * s; uint32_t* cnt_sh = c->d_counters + 2 * s + 1; uint32_t* cnt_next = c->d_counters + 2 * ns;
-                        uint32_t* cur = c->d_counters + PTB_CNT_CUR + 2 * s; uint32_t* cnt_sq = c->d_counters + PTB_CNT_SQ + s;
-                        uint32_t* cnt_def = c->d_counters + PTB_CNT_DEFER + 2 * s;
-                        if (b >= 1) {
-                            CK(cudaMemsetAsync(cnt_next, 0, sizeof(uint32_t), c->stream));
-                            if (b >= 2) {
-                                CK(cudaMemsetAsync(cnt_sh, 0, sizeof(uint32_t), c->stream));
-                                CK(cudaMemsetAsync(cur, 0, 2 * sizeof(uint32_t), c->stream));
-                                CK(cudaMemsetAsync(cnt_sq, 0, sizeof(uint32_t), c->stream));
-                                CK(cudaMemsetAsync(cnt_def, 0, 2 * sizeof(uint32_t), c->stream));
-                            }
-                            CK(cudaMemsetAsync(c->d_counters + PTB_CNT_PROBE, 0, sizeof(uint32_t), c->stream));
-                        }
-                        const uint32_t* q = b == 0 ? nullptr : c->d_queue[s];
-                        const uint32_t* cnt = b == 0 ? nullptr : cnt_q;
-                        const unsigned gt = (unsigned)std::max(1, std::min<int>(c->trace_blocks, (int)((n_level + 127) / 128)));
-                        const unsigned gs = (unsigned)((n_level + 127) / 128);
-                        if (mesh) {
-                            lt.begin(1 | (std::min(b, 63) << 8));
-                            if (c->count_traversal) k_trace<false, true><<<gt, 128, 0, c->stream>>>(c->sc, c->pool, q, cnt, n_paths, cur, c->d_totals, c->refill_below, c->tri_den, c->tri_min_pct, cnt_def);
-                            else k_trace<false, false><<<gt, 128, 0, c->stream>>>(c->sc, c->pool, q, cnt, n_paths, cur, c->d_totals, c->refill_below, c->tri_den, c->tri_min_pct, cnt_def);
-                            k_exact<false, false><<<c->exact_blocks, 128, 0, c->stream>>>(c->sc, c->pool, cnt_def);
-                            lt.end();
-                            launches += 2;
-                        }
-                        lt.begin(2 | (std::min(b, 63) << 8));
-#define PTB_SHADE_BRANCH(M, GRID, Q, CNT, NSTATIC, RESUME) k_shade_branch<M><<<GRID, 128, 0, c->stream>>>(c->sc, f, c->pool, Q, CNT, NSTATIC, c->d_queue[ns], cnt_next, cnt_sh, cnt_sq, \
-                            c->d_counters + PTB_CNT_ALLOC, (uint32_t)n_paths, (uint32_t)c->pool_cap, c->d_counters + PTB_CNT_DROPS, c->d_counters + PTB_CNT_PROBE, RESUME)
-                        if (c->has_merl) PTB_SHADE_BRANCH(true, gs, q, cnt, n_paths, nullptr); else PTB_SHADE_BRANCH(false, gs, q, cnt, n_paths, nullptr);
-                        lt.end();
-                        launches++;
-                        if (c->sc.has_sss) {   // answer this level's subsurface probes, then shade those hits for good
-                            uint32_t h_probe = 0;
-                            CK(cudaMemcpyAsync(&h_probe, c->d_counters + PTB_CNT_PROBE, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
-                            CK(cudaStreamSynchronize(c->stream));
-                            if (h_probe > 0) {
-                                const unsigned gp = (unsigned)((h_probe + 127) / 128);
-                                k_probe<<<gp, 128, 0, c->stream>>>(c->sc, c->pool, (int)h_probe);
-                                lt.begin(2 | (std::min(b, 63) << 8));
-                                if (c->has_merl) PTB_SHADE_BRANCH(true, gp, nullptr, nullptr, (int)h_probe, c->pool.probe_d); else PTB_SHADE_BRANCH(false, gp, nullptr, nullptr, (int)h_probe, c->pool.probe_d);
-                                lt.end();
-                                launches += 2;
-                            }
-                        }
-#undef PTB_SHADE_BRANCH
-                        uint32_t h_sh = 0, h_next = 0, h_sq = 0;
-                        CK(cudaMemcpyAsync(&h_sh, cnt_sh, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
-                        CK(cudaMemcpyAsync(&h_next, cnt_next, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
-                        CK(cudaMemcpyAsync(&h_sq, cnt_sq, sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
-                        CK(cudaStreamSynchronize(c->stream));
-                        if (mesh && h_sh > 0) {
-                            const unsigned ga = (unsigned)std::max(1, std::min<int>(c->trace_blocks, (int)((h_sh + 127) / 128)));
-                            lt.begin(3 | (std::min(b, 63) << 8));
-                            if (c->count_traversal) k_trace<true, true, true><<<ga, 128, 0, c->stream>>>(c->sc, c->pool, nullptr, cnt_sh, 0, cur + 1, c->d_totals, c->refill_below, c->tri_den, c->tri_min_pct, cnt_def + 1);
-                            else k_trace<true, false, true><<<ga, 128, 0, c->stream>>>(c->sc, c->pool, nullptr, cnt_sh, 0, cur + 1, c->d_totals, c->refill_below, c->tri_den, c->tri_min_pct, cnt_def + 1);
-                            k_exact<true, true><<<c->exact_blocks, 128, 0, c->stream>>>(c->sc, c->pool, cnt_def + 1);
-                            lt.end();
-                            launches += 2;
-                        }
-                        branch_closest += b == 0 ? valid_here * (unsigned long long)f.spp_pass : (unsigned long long)n_level;
-                        branch_shadow += h_sq;
-                        n_level = h_next;
-                    }
-                    levels = 0;   // k_totals adds nothing: the level loop counted on the host
-                    uint32_t drops = 0;
-                    CK(cudaMemcpyAsync(&drops, c->d_counters + PTB_CNT_DROPS, sizeof(drops), cudaMemcpyDeviceToHost, c->stream));
-                    CK(cudaStreamSynchronize(c->stream));
-                    if (drops > 0) {
-                        c->err = "branching render: contribution pool exhausted (" + std::to_string(drops) + " side branches dropped); raise PTB_OPT_POOL_PATHS";
-                        return PTB_ERR_NOMEM;
-                    }
-                }
-                for (int b = 0; b < nb && !branch; b++) {
-                    const uint32_t* q = b == 0 ? nullptr : pq[b & 1];
-                    const uint32_t* cnt = b == 0 ? nullptr : pc + 2 * b;
-                    const bool mesh = c->sc.has_mesh != 0;
-                    // persistent grid: as many blocks as are resident at once, but no more than the queue can feed
-                    const unsigned gt = (unsigned)std::max(1, std::min<int>(n_pipes > 1 ? c->trace_blocks_piped : c->trace_blocks, (n_paths + 127) / 128));
-                    if (mesh) {
-                        lt.begin(1 | (b << 8), ps);
-                        if (c->count_traversal) k_trace<false, true><<<gt, 128, 0, ps>>>(c->sc, pp, q, cnt, n_paths, pc + PTB_CNT_CUR + 2 * b, c->d_totals, c->refill_below, c->tri_den, c->tri_min_pct, pc + PTB_CNT_DEFER + 2 * b);
-                        else k_trace<false, false><<<gt, 128, 0, ps>>>(c->sc, pp, q, cnt, n_paths, pc + PTB_CNT_CUR + 2 * b, c->d_totals, c->refill_below, c->tri_den, c->tri_min_pct, pc + PTB_CNT_DEFER + 2 * b);
-                        k_exact<false, false><<<c->exact_blocks, 128, 0, ps>>>(c->sc, pp, pc + PTB_CNT_DEFER + 2 * b);
-                        lt.end();
-                        launches += 2;
-                    }
-                    lt.begin(2 | (b << 8), ps);
-#define PTB_SHADE(M, MB, A) k_shade<M, MB, A><<<(unsigned)((n_paths + PTB_SHADE_BLOCK - 1) / PTB_SHADE_BLOCK), PTB_SHADE_BLOCK, 0, ps>>>(c->sc, f, pp, q, cnt, n_paths, pq[(b + 1) & 1], pc + 2 * (b + 1), pc + 2 * b + 1, pc + PTB_CNT_SQ + b)
-#define PTB_SHADE_X(M, MB, A) k_shade<M, MB, A, true><<<(unsigned)((n_paths + PTB_SHADE_BLOCK - 1) / PTB_SHADE_BLOCK), PTB_SHADE_BLOCK, 0, ps>>>(c->sc, f, pp, q, cnt, n_paths, pq[(b + 1) & 1], pc + 2 * (b + 1), pc + 2 * b + 1, pc + PTB_CNT_SQ + b)
-                    if (c->sc.has_exotic) {      // scenes with Cylinder / PointSet objects: the kernels that carry their code (not register-squeezed)
-                        if (aov && b == 0) { if (c->has_merl) PTB_SHADE_X(true, 5, true); else PTB_SHADE_X(false, 6, true); }
-                        else if (c->has_merl) PTB_SHADE_X(true, 5, false);
-                        else PTB_SHADE_X(false, 6, false);
-                    } else
-                    if (aov && b == 0) { if (c->has_merl) PTB_SHADE(true, 5, true); else PTB_SHADE(false, 6, true); }   // camera rays of a denoiser-input render
-                    else if (c->has_merl) PTB_SHADE(true, 8, false);
-                    else PTB_SHADE(false, 8, false);
-#undef PTB_SHADE
-#undef PTB_SHADE_X
-                    lt.end();
-                    launches++;
-                    if (mesh) {
-                        lt.begin(3 | (b << 8), ps);
-                        if (c->count_traversal) k_trace<true, true><<<gt, 128, 0, ps>>>(c->sc, pp, nullptr, pc + 2 * b + 1, 0, pc + PTB_CNT_CUR + 2 * b + 1, c->d_totals, c->refill_below, c->tri_den, c->tri_min_pct, pc + PTB_CNT_DEFER + 2 * b + 1);
-                        else k_trace<true, false><<<gt, 128, 0, ps>>>(c->sc, pp, nullptr, pc + 2 * b + 1, 0, pc + PTB_CNT_CUR + 2 * b + 1, c->d_totals, c->refill_below, c->tri_den, c->tri_min_pct, pc + PTB_CNT_DEFER + 2 * b + 1);
-                        k_exact<true, false><<<c->exact_blocks, 128, 0, ps>>>(c->sc, pp, pc + PTB_CNT_DEFER + 2 * b + 1);
-                        lt.end();
-                        launches += 2;
-                    }
-                }
-                lt.begin(4, ps);
-                k_splat<<<(unsigned)((ns + 127) / 128), 128, 0, ps>>>(f, pp, d_rgbw);
+                tally.launches++;
+                if (!pl.branch) run_bounces(c, f, pp, n_paths, pl.n_pipes, lt, tally);
+                else if ((rc = run_branch_levels(c, f, n_paths, valid_here, lt, tally))) return rc;
+                lt.begin(4, pp.stream);
+                k_splat<<<(unsigned)((ns + 127) / 128), 128, 0, pp.stream>>>(f, pp.pool, d_rgbw);
                 lt.end();
-                k_totals<<<1, 32, 0, ps>>>(pc, levels, (nb > 0 && !branch) ? valid_here * (unsigned long long)f.spp_pass : 0ull, c->d_totals);
-                launches += 2;
+                // a branching render counted its rays on the host: k_totals adds nothing then
+                k_totals<<<1, 32, 0, pp.stream>>>(pp.counters, pl.branch ? 0 : f.nb_bounces,
+                                                  (f.nb_bounces > 0 && !pl.branch) ? valid_here * (unsigned long long)f.spp_pass : 0ull, c->d_totals);
+                tally.launches += 2;
                 CK(cudaGetLastError());
             }
         }
-        for (int i = 1; i < n_pipes; i++) {   // join the pipelines on the context's stream
+        for (int i = 1; i < pl.n_pipes; i++) {   // join the pipelines on the context's stream
             CK(cudaEventRecord(c->pipe_done[i], c->pipe_stream[i]));
             CK(cudaStreamWaitEvent(c->stream, c->pipe_done[i], 0));
         }
     }
     CK(cudaEventRecord(c->ev1, c->stream));
     CK(cudaStreamSynchronize(c->stream));
-    unsigned long long t[PTB_N_TOTALS];
-    CK(cudaMemcpy(t, c->d_totals, sizeof(t), cudaMemcpyDeviceToHost));
-    t[0] += branch_closest; t[1] += branch_shadow;
-    {
-        ptb_kernel_times& kt = c->ktimes;
-        for (size_t i = 0; i < c->ev_kind.size(); i++) {
-            float ms = 0;
-            cudaEventElapsedTime(&ms, c->ev_pool[2 * i], c->ev_pool[2 * i + 1]);
-            kt.ms[c->ev_kind[i] & 0xff] += ms;
-            kt.launches[c->ev_kind[i] & 0xff]++;
-        }
-        if (getenv("PTB_DEBUG_TRI") && t[6]) {   // triangle phase of k_trace (COUNT kernels): warp iterations, lanes per iteration, packed minimum
-            fprintf(stderr, "[ptb] triangle phase, closest: %llu tests in %llu warp iterations (%.1f lanes each), %llu if packed 32 to an iteration (%.1f %% fewer)\n", t[3], t[6],
-                    (double)t[3] / (double)t[6], t[7], 100.0 * (1.0 - (double)t[7] / (double)t[6]));
-            if (t[8]) fprintf(stderr, "[ptb] triangle phase, any hit: %llu tests in %llu warp iterations (%.1f lanes each), %llu if packed (%.1f %% fewer)\n", t[5], t[8], (double)t[5] / (double)t[8], t[9],
-                              100.0 * (1.0 - (double)t[9] / (double)t[8]));
-        }
-        if (getenv("PTB_DEBUG_BOUNCES")) {   // per-bounce launch times of the LAST pass + its queue lengths (diagnostics only)
-            uint32_t cnt[PTB_N_COUNTERS];
-            cudaMemcpy(cnt, c->d_counters, sizeof(cnt), cudaMemcpyDeviceToHost);
-            const size_t per_pass = 2 + 3 * (size_t)f.nb_bounces;
-            const size_t first = c->ev_kind.size() >= per_pass ? c->ev_kind.size() - per_pass : 0;
-            for (size_t i = first; i < c->ev_kind.size(); i++) {
-                float ms = 0;
-                cudaEventElapsedTime(&ms, c->ev_pool[2 * i], c->ev_pool[2 * i + 1]);
-                const int kind = c->ev_kind[i] & 0xff, b = c->ev_kind[i] >> 8;
-                const char* names[] = {"raygen", "closest", "shade", "anyhit", "splat"};
-                const unsigned items = kind == 3 ? cnt[2 * b + 1] : ((kind == 1 || kind == 2) ? (b == 0 ? 0u : cnt[2 * b]) : 0u);
-                fprintf(stderr, "[ptb] %-8s b=%d  %8.3f ms  items=%u\n", names[kind], b, ms, items);
-            }
-        }
-        (void)k_first;
-        kt.items[0] = kt.items[4] = valid_pixels * (unsigned long long)nrays;
-        kt.items[1] = kt.items[2] = t[0]; kt.items[3] = t[1];
-        kt.node_visits[1] = t[2]; kt.tri_tests[1] = t[3]; kt.node_visits[3] = t[4]; kt.tri_tests[3] = t[5];
-    }
-    if (stats) {
-        float ms = 0;
-        CK(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
-        memset(stats, 0, sizeof(*stats));
-        stats->samples = valid_pixels * (unsigned long long)nrays;
-        stats->rays_closest = t[0]; stats->rays_shadow = t[1]; stats->node_visits = t[2] + t[4]; stats->tri_tests = t[3] + t[5];
-        stats->ms_device = ms;
-        stats->ms_wall = std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - w0).count();
-        stats->kernel_launches = launches;
-    }
-    return PTB_OK;
+    return render_stats(c, f.nb_bounces, valid_pixels * (unsigned long long)nrays, tally, stats, w0);
 }
+
+extern "C" {
 
 int ptb_render_accum(ptb_ctx* c, const ptb_camera* cam, const ptb_params* p, float* d_rgbw, ptb_stats* stats) {
     if (!c) return PTB_ERR_INVALID;
@@ -1436,17 +1319,23 @@ int ptb_render_accum(ptb_ctx* c, const ptb_camera* cam, const ptb_params* p, flo
     return render_passes(c, f, p->nrays, reinterpret_cast<F4*>(d_rgbw), stats);
 }
 
+// The staging buffers of a resolved n-pixel frame (imagedouble, sample_count, image), sized together
+static int ensure_staging(ptb_ctx* c, int64_t n) {
+    if (c->out_n >= n) return PTB_OK;
+    void* ptrs[] = {c->d_out_img, c->d_out_cnt, c->d_out_u8};
+    for (void* q : ptrs) if (q) cudaFree(q);
+    c->d_out_img = nullptr; c->d_out_cnt = nullptr; c->d_out_u8 = nullptr; c->out_n = 0;
+    CK(cudaMalloc((void**)&c->d_out_img, (size_t)n * 3 * sizeof(float)));
+    CK(cudaMalloc((void**)&c->d_out_cnt, (size_t)n * sizeof(float)));
+    CK(cudaMalloc((void**)&c->d_out_u8, (size_t)n * 3));
+    c->out_n = n;
+    return PTB_OK;
+}
+
 static int resolve_to_host(ptb_ctx* c, const F4* d_rgbw, int W, int H, float gamma, float* imagedouble, float* sample_count, uint8_t* image) {
     const int64_t n = (int64_t)W * H;
-    if (c->out_n < n) {
-        void* ptrs[] = {c->d_out_img, c->d_out_cnt, c->d_out_u8};
-        for (void* q : ptrs) if (q) cudaFree(q);
-        c->d_out_img = nullptr; c->d_out_cnt = nullptr; c->d_out_u8 = nullptr; c->out_n = 0;
-        CK(cudaMalloc((void**)&c->d_out_img, (size_t)n * 3 * sizeof(float)));
-        CK(cudaMalloc((void**)&c->d_out_cnt, (size_t)n * sizeof(float)));
-        CK(cudaMalloc((void**)&c->d_out_u8, (size_t)n * 3));
-        c->out_n = n;
-    }
+    const int rc = ensure_staging(c, n);
+    if (rc) return rc;
     k_resolve<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(d_rgbw, (size_t)n, gamma, imagedouble ? c->d_out_img : nullptr,
                                                                  sample_count ? c->d_out_cnt : nullptr, image ? c->d_out_u8 : nullptr);
     CK(cudaGetLastError());
@@ -1473,12 +1362,7 @@ int ptb_render(ptb_ctx* c, const ptb_camera* cam, const ptb_params* p, float* im
     int rc = frame_setup(c, cam, p, f);
     if (rc) return rc;
     const int64_t n = (int64_t)p->W * p->H;
-    if (c->accum_n < n) {
-        if (c->d_accum) cudaFree(c->d_accum);
-        c->d_accum = nullptr; c->accum_n = 0;
-        CK(cudaMalloc((void**)&c->d_accum, (size_t)n * sizeof(F4)));
-        c->accum_n = n;
-    }
+    if ((rc = grow(c, &c->d_accum, &c->accum_n, n))) return rc;
     CK(cudaMemsetAsync(c->d_accum, 0, (size_t)n * sizeof(F4), c->stream));
     rc = render_passes(c, f, p->nrays, c->d_accum, stats);
     if (rc) return rc;
@@ -1562,15 +1446,8 @@ int ptb_progressive_read(ptb_ctx* c, float* imagedouble, float* sample_count, ui
     CK(cudaSetDevice(c->device));
     const ptb_params& p = c->prog_p;
     const int64_t n = (int64_t)p.W * p.H;
-    if (c->out_n < n) {   // the staging buffers of resolve_to_host, sized together
-        void* ptrs[] = {c->d_out_img, c->d_out_cnt, c->d_out_u8};
-        for (void* q : ptrs) if (q) cudaFree(q);
-        c->d_out_img = nullptr; c->d_out_cnt = nullptr; c->d_out_u8 = nullptr; c->out_n = 0;
-        CK(cudaMalloc((void**)&c->d_out_img, (size_t)n * 3 * sizeof(float)));
-        CK(cudaMalloc((void**)&c->d_out_cnt, (size_t)n * sizeof(float)));
-        CK(cudaMalloc((void**)&c->d_out_u8, (size_t)n * 3));
-        c->out_n = n;
-    }
+    const int rc = ensure_staging(c, n);
+    if (rc) return rc;
     k_resolve_progressive<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(c->d_prog_accum, (size_t)n, p.gamma, imagedouble ? c->d_out_img : nullptr,
                                                                              sample_count ? c->d_out_cnt : nullptr, image ? c->d_out_u8 : nullptr);
     CK(cudaGetLastError());
@@ -1583,33 +1460,20 @@ int ptb_progressive_read(ptb_ctx* c, float* imagedouble, float* sample_count, ui
     return PTB_OK;
 }
 
-static void shard_geometry(const ptb_params* p, int rank, int& tile, int& apron, int& tiles_x, int& total, int& mine) {
-    tile = p->tile_size > 0 ? p->tile_size : ptb_default_tile(p->shard_count);
-    apron = (int)ceilf(p->sigma_filter * 2);
-    tiles_x = (p->W + tile - 1) / tile;
-    total = tiles_x * ((p->H + tile - 1) / tile);
-    const int count = p->shard_count > 0 ? p->shard_count : 1;
-    mine = total > rank ? (total - rank + count - 1) / count : 0;
-}
-
 int ptb_shard_pack_size(const ptb_params* p, int shard_rank, int64_t* out_floats) {
     if (!p || !out_floats || p->W <= 0 || p->H <= 0) return PTB_ERR_INVALID;
-    int tile, apron, tiles_x, total, mine;
-    shard_geometry(p, shard_rank, tile, apron, tiles_x, total, mine);
-    const int64_t side = tile + 2 * apron;
-    *out_floats = (int64_t)mine * side * side * 4;
+    *out_floats = shard_geometry(p, shard_rank).texels() * 4;
     return PTB_OK;
 }
 
 static int shard_move(ptb_ctx* c, const ptb_params* p, int shard_rank, const float* d_rgbw, float* d_packed, int unpack) {
     if (!c || !p || !d_rgbw || !d_packed) return PTB_ERR_INVALID;
     CK(cudaSetDevice(c->device));
-    int tile, apron, tiles_x, total, mine;
-    shard_geometry(p, shard_rank, tile, apron, tiles_x, total, mine);
-    const long long side = tile + 2 * apron, n = (long long)mine * side * side;
+    const ShardGeometry g = shard_geometry(p, shard_rank);
+    const long long n = g.texels();
     if (n == 0) return PTB_OK;
-    k_shard_pack<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(reinterpret_cast<const F4*>(d_rgbw), reinterpret_cast<F4*>(d_packed), p->W, p->H, tile, apron,
-                                                                    tiles_x, total, shard_tile_shift(tiles_x, p->shard_count > 0 ? p->shard_count : 1), shard_rank, p->shard_count > 0 ? p->shard_count : 1, n, unpack);
+    k_shard_pack<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(reinterpret_cast<const F4*>(d_rgbw), reinterpret_cast<F4*>(d_packed), p->W, p->H, g.tile, g.apron,
+                                                                    g.tiles_x, g.total, g.shift, shard_rank, g.count, n, unpack);
     CK(cudaGetLastError());
     CK(cudaStreamSynchronize(c->stream));
     return PTB_OK;

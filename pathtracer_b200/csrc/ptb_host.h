@@ -145,4 +145,118 @@ inline int scene_modes(SceneDev& sc, const HostScene& h, std::string& err) {
     return PTB_OK;
 }
 
+// ---- frame and pass geometry (host only: the engine and the test-only devsim share it) -------------------------------------------
+#define PTB_MAX_BOUNCES 64
+#define PTB_MAX_PIPES 4
+#define PTB_BRANCH_MAX_LEVELS 512   // a branching render's contribution tree is cut off below this many levels
+
+// Camera, filter and the shard's tiles of a render; the per-pass fields and the buffers (rpp, AOV sums, preview) are the caller's.
+inline int frame_geometry(const ptb_camera* cam, const ptb_params* p, FrameDev& f, std::string& err) {
+    if (!cam || !p || p->W <= 0 || p->H <= 0 || p->nrays <= 0 || p->nb_bounces < 0 || p->nb_bounces > PTB_MAX_BOUNCES || !(p->sigma_filter > 0)) {
+        err = "render: invalid parameters"; return PTB_ERR_INVALID;
+    }
+    if ((int)ceilf(p->sigma_filter * 2) > PTB_MAX_FILTER) { err = "render: sigma_filter too large (filter_size > 4)"; return PTB_ERR_UNSUPPORTED; }
+    if ((int64_t)p->W * p->H >= ((int64_t)1 << 31)) { err = "render: frame too large"; return PTB_ERR_UNSUPPORTED; }
+    memset(&f, 0, sizeof(f));
+    camera_setup(f.cam, cam->position, cam->direction, cam->up, cam->fov, cam->focus_distance, cam->aperture, p->W, p->H);
+    filter_setup(f.filter, p->sigma_filter);
+    f.W = p->W; f.H = p->H; f.nb_bounces = p->nb_bounces; f.seed = p->seed;
+    f.tile = p->tile_size > 0 ? p->tile_size : ptb_default_tile(p->shard_count);
+    // a splat reaches ceil(2 sigma) pixels into the neighbouring tiles and the gather looks at the 3x3 tile neighbourhood only
+    if (f.tile < (int)ceilf(p->sigma_filter * 2) || f.tile > 4096) { err = "render: tile_size must lie in [ceil(2*sigma_filter), 4096]"; return PTB_ERR_INVALID; }
+    f.tiles_x = (p->W + f.tile - 1) / f.tile; f.tiles_y = (p->H + f.tile - 1) / f.tile;
+    f.shard_count = p->shard_count > 0 ? p->shard_count : 1;
+    f.shard_rank = p->shard_rank;
+    if (f.shard_rank < 0 || f.shard_rank >= f.shard_count) { err = "render: shard_rank out of range"; return PTB_ERR_INVALID; }
+    f.tile_shift = shard_tile_shift(f.tiles_x, f.shard_count);
+    const int total_tiles = f.tiles_x * f.tiles_y;
+    f.n_my_tiles = total_tiles > f.shard_rank ? (total_tiles - f.shard_rank + f.shard_count - 1) / f.shard_count : 0;
+    return PTB_OK;
+}
+
+// in-image pixels of the shard's pixel slots [s0, s0 + ns) (edge tiles are partial)
+inline unsigned long long tile_range_pixels(const FrameDev& f, int64_t s0, int64_t ns) {
+    const int tp = f.tile * f.tile;
+    unsigned long long n = 0;
+    for (int64_t lt = s0 / tp; lt * tp < s0 + ns; lt++) {
+        int ty, tx;
+        tile_physical(f.shard_rank + (int)lt * f.shard_count, f.tiles_x, f.tile_shift, ty, tx);
+        n += (unsigned long long)std::min(f.tile, f.H - ty * f.tile) * std::min(f.tile, f.W - tx * f.tile);
+    }
+    return n;
+}
+
+// The tiles of shard `rank` in the multi-GPU gather: each travels with an apron of ceil(2 sigma) pixels, (tile + 2 apron)^2 texels
+struct ShardGeometry {
+    int tile, apron, tiles_x, total, count, shift, mine;   // total: tiles of the frame; mine: tiles of this shard
+    int64_t texels() const { return (int64_t)mine * (tile + 2 * apron) * (tile + 2 * apron); }
+};
+inline ShardGeometry shard_geometry(const ptb_params* p, int rank) {
+    ShardGeometry g;
+    g.tile = p->tile_size > 0 ? p->tile_size : ptb_default_tile(p->shard_count);
+    g.apron = (int)ceilf(p->sigma_filter * 2);
+    g.tiles_x = (p->W + g.tile - 1) / g.tile;
+    g.total = g.tiles_x * ((p->H + g.tile - 1) / g.tile);
+    g.count = p->shard_count > 0 ? p->shard_count : 1;
+    g.shift = shard_tile_shift(g.tiles_x, g.count);
+    g.mine = g.total > rank ? (g.total - rank + g.count - 1) / g.count : 0;
+    return g;
+}
+
+// Branching renders (fog, ghost objects, a background photograph, subsurface scattering) walk each sample's contribution tree.
+inline bool is_branching(const SceneDev& sc) { return sc.has_fog || sc.has_ghost || sc.bgW > 0 || sc.has_sss; }
+// Pool slots one sample may hold at once.  A branching render keeps every live contribution of a sample in the pool: the
+// continuation reuses its slot, each side branch takes a new one.  A fogged path forks once per iteration (at most 2^depth - 1
+// forks per sample), a ghost hit once; a background photograph or a subsurface material forks nothing.
+inline int slots_per_sample(const SceneDev& sc, int nb_bounces) {
+    if (!is_branching(sc)) return 1;
+    return sc.has_fog ? (1 << std::min(nb_bounces, 6)) : (sc.has_ghost ? 8 : 1);
+}
+
+// How a render of `pixel_slots` pixel slots x `nrays` samples is cut into passes.
+struct PassPlan {
+    bool branch;
+    int n_pipes;           // pipelines the passes go round-robin to (branching renders: one)
+    int spp_pass;          // samples per pixel of a pass
+    int64_t slots_pass;    // pixel slots of a pass
+    int64_t stride;        // paths of a pass = the pool slice of one pipeline
+    int64_t pool_paths;    // paths the pool must hold
+};
+inline PassPlan plan_passes(const SceneDev& sc, int nb_bounces, int tile, int64_t pixel_slots, int nrays, int64_t pool_paths, int n_pipes) {
+    PassPlan pl;
+    pl.branch = is_branching(sc);
+    const int fan = slots_per_sample(sc, nb_bounces);
+    const int64_t pool_cap_slots = std::max<int64_t>(pool_paths, 1024);
+    int64_t pool = std::max<int64_t>(pool_cap_slots / fan, 1024);
+    pl.n_pipes = pl.branch ? 1 : std::max(1, std::min(n_pipes, PTB_MAX_PIPES));
+    if (pl.n_pipes > 1 && pixel_slots * nrays < pool * pl.n_pipes)   // a frame smaller than the pools is still split so that every pipeline gets a pass
+        pool = std::max<int64_t>((pixel_slots * nrays + pl.n_pipes - 1) / pl.n_pipes, (int64_t)1 << 18);
+    if (pixel_slots * nrays <= pool) { pl.spp_pass = nrays; pl.slots_pass = pixel_slots; }
+    else if (pixel_slots <= pool) { pl.spp_pass = (int)std::max<int64_t>(1, pool / pixel_slots); pl.slots_pass = pixel_slots; }
+    else { pl.spp_pass = 1; pl.slots_pass = (pool / (tile * tile)) * (tile * tile); if (pl.slots_pass <= 0) pl.slots_pass = tile * tile; }
+    pl.stride = pl.slots_pass * pl.spp_pass;
+    pl.pool_paths = pl.branch ? std::max<int64_t>(pl.stride * fan, pool_cap_slots) : pl.stride * pl.n_pipes;
+    return pl;
+}
+
+// ---- the path pool's arrays ------------------------------------------------------------------------------------------------------
+// Every array of PoolDev with its bytes per path and the renders that need it; allocation, release and slicing all walk this list.
+// `queue` (or null) adds the two bounce queues, which live outside PoolDev, in their place of the allocation order.
+enum { POOL_ALWAYS, POOL_AOV, POOL_BRANCH, POOL_SSS };
+struct PoolArray { void** ptr; size_t bytes; int need; };
+inline std::vector<PoolArray> pool_arrays(PoolDev& p, uint32_t** queue = nullptr) {
+    std::vector<PoolArray> a = {{(void**)&p.ray_o, sizeof(F4), POOL_ALWAYS}, {(void**)&p.ray_d, sizeof(F4), POOL_ALWAYS},
+                                {(void**)&p.weight, sizeof(F4), POOL_ALWAYS}, {(void**)&p.radiance, sizeof(F4), POOL_ALWAYS},
+                                {(void**)&p.hit, sizeof(F4), POOL_ALWAYS}, {(void**)&p.rng, sizeof(uint64_t), POOL_ALWAYS},
+                                {(void**)&p.pixel, sizeof(uint32_t), POOL_ALWAYS}, {(void**)&p.sh_o, sizeof(F4), POOL_ALWAYS},
+                                {(void**)&p.sh_d, sizeof(F4), POOL_ALWAYS}, {(void**)&p.sh_c, sizeof(F4), POOL_ALWAYS}};
+    if (queue) { a.push_back({(void**)&queue[0], sizeof(uint32_t), POOL_ALWAYS}); a.push_back({(void**)&queue[1], sizeof(uint32_t), POOL_ALWAYS}); }
+    a.insert(a.end(), {{(void**)&p.defer_prims, PTB_DEFER_K * sizeof(uint32_t), POOL_ALWAYS}, {(void**)&p.defer_rays, sizeof(U2), POOL_ALWAYS},
+                       {(void**)&p.aov_n, sizeof(F4), POOL_AOV}, {(void**)&p.aov_kd, sizeof(F4), POOL_AOV},
+                       {(void**)&p.root, sizeof(uint32_t), POOL_BRANCH},
+                       {(void**)&p.probe_o, sizeof(F4), POOL_SSS}, {(void**)&p.probe_d, sizeof(F4), POOL_SSS},
+                       {(void**)&p.probe_x, sizeof(F4), POOL_SSS}, {(void**)&p.hit2, sizeof(F4), POOL_SSS}});
+    return a;
+}
+
 }  // namespace ptb

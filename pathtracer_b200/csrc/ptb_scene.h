@@ -12,6 +12,7 @@
 // of shade_one: the same loop body with those branches, walking the contribution tree level by level
 // (DESIGN.md section 10).
 #pragma once
+#include "../../include/ptb200.h"
 #include "ptb_bvh8.h"
 
 namespace ptb {
@@ -534,6 +535,7 @@ PTB_HD void surface_from_hit(const SceneDev& sc, V3 o, V3 d, const Hit& hit, int
 }
 
 // ---- path pool (structure of arrays in HBM) ---------------------------------------------------------
+#define PTB_DEFER_K 4    /* candidates a ray can leave for k_exact; a ray with more is re-traced there with the immediate exact test */
 struct PoolDev {
     F4* ray_o;        // xyz origin
     F4* ray_d;        // xyz direction
@@ -1404,6 +1406,89 @@ PTB_HD void resolve_pixel(const F4* accum, size_t idx, float gamma, float* image
             image[idx * 3 + q] = (uint8_t)v;
         }
     }
+}
+
+// has_denoiser tail of render_image_nopreviz (Raytracer.cpp:1676-1693): colour and albedo means, and the two normal images:
+// `normalImage` as the reference computes it (it sums the COLOUR buffers there, 1680-1682, then normalises) and the normalised sum of
+// the first-hit shading normals that line was meant to produce.
+PTB_HD void resolve_denoiser_pixel(const F4* accum, const F4* albedo, const F4* normal, size_t idx, float* imagedouble, float* sample_count,
+                                   float* albedoImage, float* normalImage, float* first_hit_normal) {
+    const F4 a = accum[idx], k = albedo[idx], m = normal[idx];
+    const float nn = sqrtf(a.x * a.x + a.y * a.y + a.z * a.z), nm = sqrtf(m.x * m.x + m.y * m.y + m.z * m.z);
+    if (imagedouble) { imagedouble[idx * 3] = a.x / a.w; imagedouble[idx * 3 + 1] = a.y / a.w; imagedouble[idx * 3 + 2] = a.z / a.w; }
+    if (sample_count) sample_count[idx] = a.w;
+    if (albedoImage) { albedoImage[idx * 3] = k.x / a.w; albedoImage[idx * 3 + 1] = k.y / a.w; albedoImage[idx * 3 + 2] = k.z / a.w; }
+    if (normalImage) { normalImage[idx * 3] = a.x / nn; normalImage[idx * 3 + 1] = a.y / nn; normalImage[idx * 3 + 2] = a.z / nn; }
+    if (first_hit_normal) { first_hit_normal[idx * 3] = m.x / nm; first_hit_normal[idx * 3 + 1] = m.y / nm; first_hit_normal[idx * 3 + 2] = m.z / nm; }
+}
+
+// tail of the progressive Raytracer::render_image (Raytracer.cpp:1540-1547): imagedouble stays the un-normalised sums, the display
+// image divides by max(sample_count, 1)
+PTB_HD void resolve_progressive_pixel(const F4* accum, size_t idx, float gamma, float* imagedouble, float* sample_count, uint8_t* image) {
+    const F4 a = accum[idx];
+    if (imagedouble) { imagedouble[idx * 3] = a.x; imagedouble[idx * 3 + 1] = a.y; imagedouble[idx * 3 + 2] = a.z; }
+    if (sample_count) sample_count[idx] = a.w;
+    if (image) {
+        const double ig = (double)(1 / gamma);
+        const float d = fmaxf(a.w, 1.f);
+        const float c[3] = {a.x, a.y, a.z};
+        for (int q = 0; q < 3; q++) {
+            double v = 255. * pow((double)c[q] / 196964.7 / (double)d, ig);
+            v = v > 0. ? v : 0.;
+            v = v < 255. ? v : 255.;
+            image[idx * 3 + q] = (uint8_t)v;
+        }
+    }
+}
+
+// ---- multi-GPU gather: texel `idx` of shard `rank`'s packed tiles, each tile with its apron ((tile + 2 apron)^2 texels, tile-major) ----
+// pack: the frame texel if this tile's block sends it (shard_block_sends), else zero; unpack: ADD(addr, value) a non-zero texel into the frame.
+template <class ADD>
+PTB_HD void shard_texel(F4* rgbw, F4* packed, long long idx, int W, int H, int tile, int apron, int tiles_x, int n_tiles_total, int shift,
+                        int rank, int count, int unpack, ADD add) {
+    const int side = tile + 2 * apron;
+    const long long per = (long long)side * side;
+    const int lt = (int)(idx / per);
+    const int r = (int)(idx - (long long)lt * per);
+    const int tile_id = rank + lt * count;
+    if (tile_id >= n_tiles_total) return;
+    int ty, tx;
+    tile_physical(tile_id, tiles_x, shift, ty, tx);
+    const int i = ty * tile - apron + r / side, j = tx * tile - apron + r % side;
+    const bool inside = i >= 0 && i < H && j >= 0 && j < W;
+    if (!unpack) {
+        const int tiles_y = (H + tile - 1) / tile;
+        const bool send = shard_block_sends(tile_id, i, j, W, H, tile, apron, tiles_x, tiles_y, rank, count, shift);
+        F4 z; z.x = z.y = z.z = z.w = 0;
+        packed[idx] = send ? rgbw[(size_t)(H - 1 - i) * W + j] : z;
+    } else if (inside) {
+        const F4 v = packed[idx];
+        if (v.x != 0.f || v.y != 0.f || v.z != 0.f || v.w != 0.f) add(rgbw + (size_t)(H - 1 - i) * W + j, v);
+    }
+}
+
+// ---- known-answer tests (ptb_kat): one input row `a` of test `which` -> its output row `o`; false for an unknown test --------------
+PTB_HD bool kat_one(int which, const SceneDev& sc, const CameraDev& cam, const FilterDev& filt, int W, int H, const double* a, double* o) {
+    switch (which) {
+    case PTB_KAT_PCG32: { Pcg32 e = pcg32_seed((uint64_t)a[0], (uint64_t)a[1]); for (int q = 0; q < 4; q++) o[q] = (double)pcg32_next(e); } break;
+    case PTB_KAT_LATTICE: { float x, y; extensible_lattice_2d((uint32_t)a[0], x, y); o[0] = x; o[1] = y; } break;
+    case PTB_KAT_CAMERA: { V3 ro, rd; camera_ray(cam, (int)a[0], (int)a[1], (float)a[2], (float)a[3], (float)a[4], (float)a[5], ro, rd);
+        o[0] = ro.x; o[1] = ro.y; o[2] = ro.z; o[3] = rd.x; o[4] = rd.y; o[5] = rd.z; } break;
+    case PTB_KAT_RANDOM_COS: { V3 v = random_cos(v3((float)a[0], (float)a[1], (float)a[2]), (float)a[3], (float)a[4]); o[0] = v.x; o[1] = v.y; o[2] = v.z; } break;
+    case PTB_KAT_RANDOM_PHONG: { V3 v = random_phong(v3((float)a[0], (float)a[1], (float)a[2]), (float)a[3], (float)a[4], (float)a[5]); o[0] = v.x; o[1] = v.y; o[2] = v.z; } break;
+    case PTB_KAT_PHONG_EVAL: { V3 v = phong_eval(v3((float)a[0], (float)a[1], (float)a[2]), v3((float)a[3], (float)a[4], (float)a[5]), v3((float)a[6], (float)a[7], (float)a[8]),
+                                               v3((float)a[9], (float)a[10], (float)a[11]), v3((float)a[12], (float)a[13], (float)a[14]), v3((float)a[15], (float)a[16], (float)a[17]));
+        o[0] = v.x; o[1] = v.y; o[2] = v.z; } break;
+    case PTB_KAT_MERL_EVAL: { V3 v = merl_eval(sc.merl, v3((float)a[0], (float)a[1], (float)a[2]), v3((float)a[3], (float)a[4], (float)a[5]), v3((float)a[6], (float)a[7], (float)a[8]));
+        o[0] = v.x; o[1] = v.y; o[2] = v.z; } break;
+    case PTB_KAT_FAST_EXP: o[0] = fast_exp(a[0]); break;
+    case PTB_KAT_FAST_NORMALIZE: { V3 v = fast_normalize(v3((float)a[0], (float)a[1], (float)a[2])); o[0] = v.x; o[1] = v.y; o[2] = v.z; } break;
+    case PTB_KAT_RANDOM_PER_PIXEL: { float x, y; random_per_pixel((uint32_t)a[0], x, y); o[0] = x; o[1] = y; } break;
+    case PTB_KAT_FILTER_RATIO: { int b0, b1, b2, b3; o[0] = filter_ratio(filt, (int)a[0], (int)a[1], W, H, b0, b1, b2, b3); } break;
+    case PTB_KAT_MERL_INDEX: { int f, e; merl_index_both(v3((float)a[0], (float)a[1], (float)a[2]), v3((float)a[3], (float)a[4], (float)a[5]), f, e); o[0] = f; o[1] = e; } break;
+    default: return false;
+    }
+    return true;
 }
 
 }  // namespace ptb

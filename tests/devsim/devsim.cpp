@@ -79,16 +79,9 @@ int ptb_commit(ptb_ctx* c) {
 static int render_into(ptb_ctx* c, const ptb_camera* cam, const ptb_params* p, F4* accum_out, ptb_stats* stats, const Extras& x = Extras()) {
     if (!c->committed) return PTB_ERR_STATE;
     auto t0 = std::chrono::steady_clock::now();
-    FrameDev f; memset(&f, 0, sizeof(f));
-    camera_setup(f.cam, cam->position, cam->direction, cam->up, cam->fov, cam->focus_distance, cam->aperture, p->W, p->H);
-    filter_setup(f.filter, p->sigma_filter);
-    f.W = p->W; f.H = p->H; f.nb_bounces = p->nb_bounces; f.seed = p->seed;
-    f.tile = p->tile_size > 0 ? p->tile_size : ptb_default_tile(p->shard_count);
-    f.tiles_x = (p->W + f.tile - 1) / f.tile; f.tiles_y = (p->H + f.tile - 1) / f.tile;
-    f.shard_count = p->shard_count > 0 ? p->shard_count : 1; f.shard_rank = p->shard_rank;
-    f.tile_shift = shard_tile_shift(f.tiles_x, f.shard_count);
-    const int total = f.tiles_x * f.tiles_y;
-    f.n_my_tiles = total > f.shard_rank ? (total - f.shard_rank + f.shard_count - 1) / f.shard_count : 0;
+    FrameDev f;
+    int rc = frame_geometry(cam, p, f, c->err);
+    if (rc) return rc;
     const size_t npix = (size_t)p->W * p->H;
     std::vector<float> rpp(2 * npix);
     for (size_t i = 0; i < npix; i++) random_per_pixel((uint32_t)i, rpp[2 * i], rpp[2 * i + 1]);
@@ -96,25 +89,24 @@ static int render_into(ptb_ctx* c, const ptb_camera* cam, const ptb_params* p, F
     f.spp_pass = p->nrays; f.k0 = x.k_first; f.slot0 = 0; f.n_pixel_slots = f.n_my_tiles * f.tile * f.tile;
     f.box_filter = x.box ? 1 : 0; f.accum_albedo = x.albedo; f.accum_normal = x.normal;
     f.lowres = x.lowres; f.lowresW = (int)ceilf(p->W / 16.f); f.lowresH = (int)ceilf(p->H / 16.f);
-    const bool branch = c->sc.has_fog || c->sc.has_ghost || c->sc.bgW > 0 || c->sc.has_sss;
+    // one pass holds every sample: the pool the engine would need for it
+    const bool branch = is_branching(c->sc);
     const size_t n_roots = (size_t)f.n_pixel_slots * f.spp_pass;
-    const size_t P = n_roots * (branch ? (c->sc.has_fog ? ((size_t)1 << std::min(f.nb_bounces, 6)) : 8) : 1);
-    std::vector<uint32_t> root(branch ? P : 0);
-    std::vector<F4> probe_o(c->sc.has_sss ? P : 0), probe_d(probe_o.size()), probe_x(probe_o.size()), hit2(probe_o.size());
-    std::vector<F4> ray_o(P), ray_d(P), weight(P), radiance(P), hit(P), sh_o(P), sh_d(P), sh_c(P);
-    std::vector<uint64_t> rng(P); std::vector<uint32_t> pixel(P), q0, q1;
-    std::vector<F4> aov_n(x.albedo ? P : 0), aov_kd(x.albedo ? P : 0);
-    PoolDev pool{ray_o.data(), ray_d.data(), weight.data(), radiance.data(), hit.data(), rng.data(), pixel.data(), sh_o.data(), sh_d.data(), sh_c.data(),
-                 x.albedo ? aov_n.data() : nullptr, x.albedo ? aov_kd.data() : nullptr, branch ? root.data() : nullptr,
-                 probe_o.data(), probe_d.data(), probe_x.data(), hit2.data()};
+    const size_t P = n_roots * slots_per_sample(c->sc, f.nb_bounces);
+    PoolDev pool = {};
+    const bool need[] = {true, x.albedo != nullptr, branch, c->sc.has_sss != 0};   // by PoolArray::need
+    std::vector<std::vector<F4>> arrays;                                             // zeroed, F4-aligned storage of the pool arrays
+    for (const PoolArray& a : pool_arrays(pool))
+        if (need[a.need]) { arrays.emplace_back((P * a.bytes + sizeof(F4) - 1) / sizeof(F4)); *a.ptr = arrays.back().data(); }
+    std::vector<uint32_t> q0, q1;
     unsigned long long closest = 0, shadow = 0, nodes = 0, tris = 0, samples = 0;
 #pragma omp parallel for schedule(static)
     for (long long i = 0; i < (long long)n_roots; i++) raygen_one(c->sc, f, pool, (int)i);
-    for (size_t i = 0; i < n_roots; i++) if (pixel[i] != 0xffffffffu) { q0.push_back((uint32_t)i); }
+    for (size_t i = 0; i < n_roots; i++) if (pool.pixel[i] != 0xffffffffu) { q0.push_back((uint32_t)i); }
     samples = q0.size();
-    if (branch) {   // the level loop of render_passes' branching mode, single-threaded
+    if (branch) {   // the engine's branching level loop (run_branch_levels), single-threaded
         size_t next_slot = n_roots;
-        for (int b = 0; b < 512 && !q0.empty() && f.nb_bounces > 0; b++) {   // PTB_BRANCH_MAX_LEVELS
+        for (int b = 0; b < PTB_BRANCH_MAX_LEVELS && !q0.empty() && f.nb_bounces > 0; b++) {
             closest += q0.size();
             q1.clear();
             size_t ns = 0;
@@ -128,9 +120,9 @@ static int render_into(ptb_ctx* c, const ptb_camera* cam, const ptb_params* p, F
             for (size_t i = 0; i < visit.size(); i++) {     // hits that emit a subsurface probe are answered and revisited at the end of the list
                 const int path = (int)visit[i];
                 BranchOut out;
-                if (getenv("PTB_DBG") && (f2u(weight[path].w) & 0xffffu)) {
-                    const int32_t hid = (int32_t)f2u(hit[path].w);
-                    fprintf(stderr, "P %u %u %d %.4f\n", pixel[path], f2u(weight[path].w) & 0xffffu, hid >= 0 ? (c->sc.tri_uv[hid].object_has_uv & 0x7fffffff) : (hid == -1 ? -1 : -2 - hid), hid == -1 ? 0.f : hit[path].x);
+                if (getenv("PTB_DBG") && (f2u(pool.weight[path].w) & 0xffffu)) {
+                    const int32_t hid = (int32_t)f2u(pool.hit[path].w);
+                    fprintf(stderr, "P %u %u %d %.4f\n", pool.pixel[path], f2u(pool.weight[path].w) & 0xffffu, hid >= 0 ? (c->sc.tri_uv[hid].object_has_uv & 0x7fffffff) : (hid == -1 ? -1 : -2 - hid), hid == -1 ? 0.f : pool.hit[path].x);
                 }
                 shade_branch_one<true>(c->sc, f, pool, path, out);
                 uint32_t ghost_slot = 0x7fffffffu;
@@ -138,7 +130,7 @@ static int render_into(ptb_ctx* c, const ptb_camera* cam, const ptb_params* p, F
                     const ChildOut& ch = k == 0 ? out.fog : out.ghost;
                     if (!ch.want) continue;
                     if (next_slot >= P) { c->err = "devsim: branching pool exhausted"; return PTB_ERR_NOMEM; }
-                    store_child(c->sc, pool, (uint32_t)next_slot, ch, root[path], pixel[path]);
+                    store_child(c->sc, pool, (uint32_t)next_slot, ch, pool.root[path], pool.pixel[path]);
                     if (k == 1) ghost_slot = (uint32_t)next_slot;
                     q1.push_back((uint32_t)next_slot++);
                 }
@@ -146,17 +138,17 @@ static int render_into(ptb_ctx* c, const ptb_camera* cam, const ptb_params* p, F
                 if (out.base.shadow) {
                     F4 cc = out.base.sh_c;
                     if (out.ghost_pending) cc.w = u2f(0x80000000u | ghost_slot);
-                    sh_o[ns] = out.base.sh_o; sh_d[ns] = out.base.sh_d; sh_c[ns] = cc; ns++;
+                    pool.sh_o[ns] = out.base.sh_o; pool.sh_d[ns] = out.base.sh_d; pool.sh_c[ns] = cc; ns++;
                 }
                 if (out.base.shadow_query) shadow++;
-                if (out.probe) { probe_o[0] = out.probe_o; probe_d[0] = out.probe_d; probe_x[0] = out.probe_x; probe_one(c->sc, pool, 0); visit.push_back((uint32_t)path); }
+                if (out.probe) { pool.probe_o[0] = out.probe_o; pool.probe_d[0] = out.probe_d; pool.probe_x[0] = out.probe_x; probe_one(c->sc, pool, 0); visit.push_back((uint32_t)path); }
             }
             for (size_t i = 0; i < ns; i++) {
                 TraverseCounters tc{0, 0};
                 const AlphaCtx ac = alpha_ctx(c->sc);
                 Hit h;
-                const bool occ = traverse<true, true>(c->sc.nodes, c->sc.tris, &ac, v3(sh_o[i].x, sh_o[i].y, sh_o[i].z), v3(sh_d[i].x, sh_d[i].y, sh_d[i].z), sh_o[i].w, h, &tc);
-                shadow_settle_branch(pool, (int)i, f2u(sh_d[i].w), occ);
+                const bool occ = traverse<true, true>(c->sc.nodes, c->sc.tris, &ac, v3(pool.sh_o[i].x, pool.sh_o[i].y, pool.sh_o[i].z), v3(pool.sh_d[i].x, pool.sh_d[i].y, pool.sh_d[i].z), pool.sh_o[i].w, h, &tc);
+                shadow_settle_branch(pool, (int)i, f2u(pool.sh_d[i].w), occ);
                 nodes += tc.nodes; tris += tc.tris;
             }
             q0.swap(q1);
@@ -174,7 +166,7 @@ static int render_into(ptb_ctx* c, const ptb_camera* cam, const ptb_params* p, F
         size_t ns = 0;
         for (long long i = 0; i < n; i++) {
             if (outs[i].cont) q1.push_back(q0[i]);
-            if (outs[i].shadow) { sh_o[ns] = outs[i].sh_o; sh_d[ns] = outs[i].sh_d; sh_c[ns] = outs[i].sh_c; ns++; }
+            if (outs[i].shadow) { pool.sh_o[ns] = outs[i].sh_o; pool.sh_d[ns] = outs[i].sh_d; pool.sh_c[ns] = outs[i].sh_c; ns++; }
             if (outs[i].shadow_query) shadow++;
         }
 #pragma omp parallel for schedule(dynamic, 256) reduction(+ : nodes, tris)
@@ -206,15 +198,7 @@ int ptb_render_denoiser_inputs(ptb_ctx* c, const ptb_camera* cam, const ptb_para
     Extras x; x.box = true; x.albedo = alb.data(); x.normal = nrm.data();
     int rc = render_into(c, cam, p, acc.data(), stats, x);
     if (rc) return rc;
-    for (size_t i = 0; i < n; i++) {     // k_resolve_denoiser
-        const F4 a = acc[i], k = alb[i], m = nrm[i];
-        const float nn = sqrtf(a.x * a.x + a.y * a.y + a.z * a.z), nm = sqrtf(m.x * m.x + m.y * m.y + m.z * m.z);
-        if (imagedouble) { imagedouble[i * 3] = a.x / a.w; imagedouble[i * 3 + 1] = a.y / a.w; imagedouble[i * 3 + 2] = a.z / a.w; }
-        if (sample_count) sample_count[i] = a.w;
-        if (albedoImage) { albedoImage[i * 3] = k.x / a.w; albedoImage[i * 3 + 1] = k.y / a.w; albedoImage[i * 3 + 2] = k.z / a.w; }
-        if (normalImage) { normalImage[i * 3] = a.x / nn; normalImage[i * 3 + 1] = a.y / nn; normalImage[i * 3 + 2] = a.z / nn; }
-        if (first_hit_normal) { first_hit_normal[i * 3] = m.x / nm; first_hit_normal[i * 3 + 1] = m.y / nm; first_hit_normal[i * 3 + 2] = m.z / nm; }
-    }
+    for (size_t i = 0; i < n; i++) resolve_denoiser_pixel(acc.data(), alb.data(), nrm.data(), i, imagedouble, sample_count, albedoImage, normalImage, first_hit_normal);
     return PTB_OK;
 }
 int ptb_progressive_begin(ptb_ctx* c, const ptb_camera* cam, const ptb_params* p) {
@@ -239,16 +223,7 @@ int ptb_progressive_pass(ptb_ctx* c, int n_spp, ptb_stats* stats) {
 int ptb_progressive_read(ptb_ctx* c, float* imagedouble, float* sample_count, uint8_t* image, float* imagedouble_lowres, int32_t* current_nb_rays) {
     if (!c->prog) return PTB_ERR_STATE;
     const ptb_params& p = c->prog_p;
-    for (size_t i = 0; i < (size_t)p.W * p.H; i++) {     // k_resolve_progressive
-        const F4 a = c->prog_accum[i];
-        if (imagedouble) { imagedouble[i * 3] = a.x; imagedouble[i * 3 + 1] = a.y; imagedouble[i * 3 + 2] = a.z; }
-        if (sample_count) sample_count[i] = a.w;
-        if (image) {
-            const double ig = (double)(1 / p.gamma);
-            const float d = a.w < 1.f ? 1.f : a.w, cc[3] = {a.x, a.y, a.z};
-            for (int q = 0; q < 3; q++) { double v = 255. * pow((double)cc[q] / 196964.7 / (double)d, ig); v = v > 0. ? v : 0.; v = v < 255. ? v : 255.; image[i * 3 + q] = (uint8_t)v; }
-        }
-    }
+    for (size_t i = 0; i < (size_t)p.W * p.H; i++) resolve_progressive_pixel(c->prog_accum.data(), i, p.gamma, imagedouble, sample_count, image);
     if (imagedouble_lowres) memcpy(imagedouble_lowres, c->prog_lowres.data(), c->prog_lowres.size() * sizeof(float));
     if (current_nb_rays) *current_nb_rays = c->prog_iter;
     return PTB_OK;
@@ -259,39 +234,13 @@ int ptb_resolve(ptb_ctx*, const float* d_rgbw, int W, int H, float gamma, float*
     for (size_t i = 0; i < (size_t)W * H; i++) resolve_pixel(reinterpret_cast<const F4*>(d_rgbw), i, gamma, imagedouble, sample_count, image);
     return PTB_OK;
 }
-static void shard_geometry(const ptb_params* p, int rank, int& tile, int& apron, int& tiles_x, int& total, int& mine) {
-    tile = p->tile_size > 0 ? p->tile_size : ptb_default_tile(p->shard_count);
-    apron = (int)ceilf(p->sigma_filter * 2);
-    tiles_x = (p->W + tile - 1) / tile;
-    total = tiles_x * ((p->H + tile - 1) / tile);
-    const int count = p->shard_count > 0 ? p->shard_count : 1;
-    mine = total > rank ? (total - rank + count - 1) / count : 0;
-}
 int ptb_shard_pack_size(const ptb_params* p, int rank, int64_t* out) {
-    int tile, apron, tiles_x, total, mine;
-    shard_geometry(p, rank, tile, apron, tiles_x, total, mine);
-    const int64_t side = tile + 2 * apron;
-    *out = (int64_t)mine * side * side * 4;
+    *out = shard_geometry(p, rank).texels() * 4;
     return PTB_OK;
 }
 static int shard_move(const ptb_params* p, int rank, F4* rgbw, F4* packed, int unpack) {
-    int tile, apron, tiles_x, total, mine;
-    shard_geometry(p, rank, tile, apron, tiles_x, total, mine);
-    const int side = tile + 2 * apron, count = p->shard_count > 0 ? p->shard_count : 1;
-    for (int lt = 0; lt < mine; lt++) {
-        const int tile_id = rank + lt * count, shift = shard_tile_shift(tiles_x, count);
-        int ty, tx;
-        tile_physical(tile_id, tiles_x, shift, ty, tx);
-        for (int r = 0; r < side * side; r++) {
-            const int i = ty * tile - apron + r / side, j = tx * tile - apron + r % side;
-            const bool inside = i >= 0 && i < p->H && j >= 0 && j < p->W;
-            F4& q = packed[(size_t)lt * side * side + r];
-            const int tiles_y = (p->H + tile - 1) / tile;
-            const bool send = shard_block_sends(tile_id, i, j, p->W, p->H, tile, apron, tiles_x, tiles_y, rank, count, shift);
-            if (!unpack) { F4 z; z.x = z.y = z.z = z.w = 0; q = send ? rgbw[(size_t)(p->H - 1 - i) * p->W + j] : z; }
-            else if (inside) { F4& d = rgbw[(size_t)(p->H - 1 - i) * p->W + j]; d.x += q.x; d.y += q.y; d.z += q.z; d.w += q.w; }
-        }
-    }
+    const ShardGeometry g = shard_geometry(p, rank);
+    for (long long idx = 0; idx < g.texels(); idx++) shard_texel(rgbw, packed, idx, p->W, p->H, g.tile, g.apron, g.tiles_x, g.total, g.shift, rank, g.count, unpack, PlainAdd());
     return PTB_OK;
 }
 int ptb_shard_pack(ptb_ctx*, const ptb_params* p, int rank, const float* d_rgbw, float* d_packed) { return shard_move(p, rank, (F4*)d_rgbw, (F4*)d_packed, 0); }
@@ -329,24 +278,9 @@ int ptb_kat(ptb_ctx* c, int which, const ptb_camera* cam, int W, int H, const do
     if (cam) camera_setup(cd, cam->position, cam->direction, cam->up, cam->fov, cam->focus_distance, cam->aperture, W, H);
     FilterDev fd; memset(&fd, 0, sizeof(fd));
     if (which == PTB_KAT_FILTER_RATIO) filter_setup(fd, (float)in[2]);
-    for (int k = 0; k < n; k++) {
-        const double* a = in + (size_t)k * is; double* o = out + (size_t)k * os;
-        switch (which) {
-        case PTB_KAT_PCG32: { Pcg32 e = pcg32_seed((uint64_t)a[0], (uint64_t)a[1]); for (int q = 0; q < 4; q++) o[q] = (double)pcg32_next(e); } break;
-        case PTB_KAT_LATTICE: { float x, y; extensible_lattice_2d((uint32_t)a[0], x, y); o[0] = x; o[1] = y; } break;
-        case PTB_KAT_CAMERA: { V3 ro, rd; camera_ray(cd, (int)a[0], (int)a[1], (float)a[2], (float)a[3], (float)a[4], (float)a[5], ro, rd); o[0] = ro.x; o[1] = ro.y; o[2] = ro.z; o[3] = rd.x; o[4] = rd.y; o[5] = rd.z; } break;
-        case PTB_KAT_RANDOM_COS: { V3 v = random_cos(v3((float)a[0], (float)a[1], (float)a[2]), (float)a[3], (float)a[4]); o[0] = v.x; o[1] = v.y; o[2] = v.z; } break;
-        case PTB_KAT_RANDOM_PHONG: { V3 v = random_phong(v3((float)a[0], (float)a[1], (float)a[2]), (float)a[3], (float)a[4], (float)a[5]); o[0] = v.x; o[1] = v.y; o[2] = v.z; } break;
-        case PTB_KAT_PHONG_EVAL: { V3 v = phong_eval(v3((float)a[0], (float)a[1], (float)a[2]), v3((float)a[3], (float)a[4], (float)a[5]), v3((float)a[6], (float)a[7], (float)a[8]), v3((float)a[9], (float)a[10], (float)a[11]), v3((float)a[12], (float)a[13], (float)a[14]), v3((float)a[15], (float)a[16], (float)a[17])); o[0] = v.x; o[1] = v.y; o[2] = v.z; } break;
-        case PTB_KAT_MERL_EVAL: { if (!c->committed || c->host.merl_tables.empty()) return PTB_ERR_STATE; V3 v = merl_eval(c->sc.merl, v3((float)a[0], (float)a[1], (float)a[2]), v3((float)a[3], (float)a[4], (float)a[5]), v3((float)a[6], (float)a[7], (float)a[8])); o[0] = v.x; o[1] = v.y; o[2] = v.z; } break;
-        case PTB_KAT_FAST_EXP: o[0] = fast_exp(a[0]); break;
-        case PTB_KAT_FAST_NORMALIZE: { V3 v = fast_normalize(v3((float)a[0], (float)a[1], (float)a[2])); o[0] = v.x; o[1] = v.y; o[2] = v.z; } break;
-        case PTB_KAT_RANDOM_PER_PIXEL: { float x, y; random_per_pixel((uint32_t)a[0], x, y); o[0] = x; o[1] = y; } break;
-        case PTB_KAT_FILTER_RATIO: { int b0, b1, b2, b3; o[0] = filter_ratio(fd, (int)a[0], (int)a[1], W, H, b0, b1, b2, b3); } break;
-        case PTB_KAT_MERL_INDEX: { int f, e; merl_index_both(v3((float)a[0], (float)a[1], (float)a[2]), v3((float)a[3], (float)a[4], (float)a[5]), f, e); o[0] = f; o[1] = e; } break;
-        default: return PTB_ERR_UNSUPPORTED;
-        }
-    }
+    if (which == PTB_KAT_MERL_EVAL && (!c->committed || c->host.merl_tables.empty())) return PTB_ERR_STATE;
+    for (int k = 0; k < n; k++)
+        if (!kat_one(which, c->sc, cd, fd, W, H, in + (size_t)k * is, out + (size_t)k * os)) return PTB_ERR_UNSUPPORTED;
     return PTB_OK;
 }
 
