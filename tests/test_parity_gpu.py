@@ -2,7 +2,9 @@
 inputs, plus size-independent properties at the benchmark configurations' full sizes.  Run on the B200 box:
     python -m pytest tests -m gpu
 The oracle here is oracle/port (bit-identical to the reference's own code on the golden vectors, see
-tests/test_oracle_pinning.py); oracle/_ref is used as well when its prebuilt library travelled."""
+tests/test_oracle_pinning.py); oracle/_ref is used as well when its prebuilt library travelled.
+`check_ids` measures `primary_ids`, i.e. k_primary over the plain traverse<>: no rendered pixel takes its hit from there.  The hits
+of the render kernels (k_trace and k_exact) are compared pixel by pixel in tests/test_wavefront_hits.py."""
 import ctypes as C
 import os
 
@@ -262,7 +264,8 @@ def test_errors_gpu(gpu):
 
 
 def test_primary_ids_on_a_quarter_million_triangles(gpu, port):
-    """BASELINE.json north_star: primary-ray hit triangle ids agree on >= 99.99 % of pixels (C4's mesh, 512x512)."""
+    """BASELINE.json north_star: primary-ray hit triangle ids agree on >= 99.99 % of pixels (C4's mesh, 512x512).  The ids come
+    from k_primary; tests/test_wavefront_hits.py checks the hits of the render kernels."""
     mk = lambda L: scenes.config_C4(L, 512, 512, 1)
     a, b = mk(port).commit(), mk(gpu).commit()
     check_ids(b, a)
@@ -608,7 +611,7 @@ def test_ngan_preset_scene_vs_oracle_and_golden(gpu, port):
 
 @pytest.mark.parametrize("name", ["C2", "C3"])
 def test_full_size_equal_seed_parity(gpu, port, name):
-    """BASELINE.json configs[1] and [2] at their full triangle counts and resolutions, 1 spp: primary-hit triangle ids (the north
+    """BASELINE.json configs[1] and [2] at their full triangle counts and resolutions, 1 spp: primary-hit triangle ids (k_primary; the north
     star's criterion, >= 99.99 %, asserted literally) and the fixed-seed single-sample image against the oracle on the same seeded
     input.  C3 puts 2.5 M triangles under 2.07 M pixels with a checker alpha map inside the traversal.  Round 1 measured 293
     differing pixels there (99.9859 %: 152 equal-distance ties on shared edges, 141 silhouette / alpha-border rays where the
