@@ -557,6 +557,11 @@ struct PoolDev {
     uint32_t* defer_prims;  // PTB_DEFER_K per ray (closest: path slot, any hit: shadow entry): triangle | flags << 28 left for k_exact
     U2* defer_rays;         // queue of the rays that left some: {path slot or shadow entry, how many}
 };
+// a hit as the pool stores it (hit, hit2)
+PTB_HD F4 hit_record(const Hit& h) {
+    F4 q; q.x = h.t; q.y = h.b1; q.z = h.b2; q.w = u2f((uint32_t)h.prim);
+    return q;
+}
 
 struct FrameDev {     // per-render constants (Raytracer fields + prepare_render results)
     CameraDev cam;
@@ -648,6 +653,14 @@ enum { ST_SHOW_LIGHTS = 0x10000u, ST_SHOW_ENV = 0x20000u, ST_HAD_SS = 0x40000u, 
        ST_FOG_PENDING = 1u << 21, ST_FOG_UNIFORM = 1u << 22, ST_SSS_WAIT = 1u << 23 /* the subsurface probe of this hit is in flight / answered */ };
 PTB_HD uint32_t pack_state(int depth, bool show_lights) { return (uint32_t)depth | (show_lights ? ST_SHOW_LIGHTS : 0u) | ST_SHOW_ENV; }
 
+// the hit record of a new ray before the BVH has seen it: the analytic half of Scene::intersection rides with the ray producer
+template <bool EXOTIC = true>
+PTB_HD F4 analytic_hit(const SceneDev& sc, V3 o, V3 d) {
+    Hit h; h.b1 = 0; h.b2 = 0;
+    analytic_closest<EXOTIC>(sc, o, d, h.t, h.prim);
+    return hit_record(h);
+}
+
 // ---- stage 1: camera samples --------------------------------------------------------------------------
 template <bool EXOTIC = true>
 PTB_HD void raygen_one(const SceneDev& sc, const FrameDev& f, PoolDev& p, int path) {
@@ -655,8 +668,7 @@ PTB_HD void raygen_one(const SceneDev& sc, const FrameDev& f, PoolDev& p, int pa
     int i, j;
     if (!slot_to_pixel(f, f.slot0 + ps, i, j)) {   // slot of an edge tile that lies outside the frame: an empty path
         p.pixel[path] = 0xffffffffu;
-        F4 m; m.x = INFINITY; m.y = 0; m.z = 0; m.w = u2f((uint32_t)PTB_HIT_MISS);
-        p.hit[path] = m;
+        p.hit[path] = hit_record(Hit{INFINITY, 0, 0, PTB_HIT_MISS});
         return;
     }
     const uint32_t pix = (uint32_t)(i * f.W + j);
@@ -674,9 +686,7 @@ PTB_HD void raygen_one(const SceneDev& sc, const FrameDev& f, PoolDev& p, int pa
     q.x = 1; q.y = 1; q.z = 1; q.w = u2f(pack_state(f.nb_bounces, true)); p.weight[path] = q;
     q.x = 0; q.y = 0; q.z = 0; q.w = 0; p.radiance[path] = q;
     if (f.accum_albedo) { p.aov_n[path] = q; p.aov_kd[path] = q; }   // `Vector normal, albedo;` start at zero (Vector.h:45) and stay there on a miss
-    float ta; int32_t ida;
-    analytic_closest<EXOTIC>(sc, o, d, ta, ida);        // the analytic half of Scene::intersection rides with the ray producer
-    q.x = ta; q.y = 0; q.z = 0; q.w = u2f((uint32_t)ida); p.hit[path] = q;
+    p.hit[path] = analytic_hit<EXOTIC>(sc, o, d);
     p.rng[path] = e.state;
     p.pixel[path] = pix;
     if (p.root) p.root[path] = (uint32_t)path;
@@ -689,11 +699,7 @@ PTB_HD void extend_one(const SceneDev& sc, PoolDev& p, int path, TraverseCounter
     const F4 h0 = p.hit[path];
     const AlphaCtx ac = alpha_ctx(sc);
     Hit h;
-    if (traverse<false, COUNT>(sc.nodes, sc.tris, &ac, v3(o.x, o.y, o.z), v3(d.x, d.y, d.z), h0.x, h, cnt)) {
-        F4 q;
-        q.x = h.t; q.y = h.b1; q.z = h.b2; q.w = u2f((uint32_t)h.prim);
-        p.hit[path] = q;
-    }
+    if (traverse<false, COUNT>(sc.nodes, sc.tris, &ac, v3(o.x, o.y, o.z), v3(d.x, d.y, d.z), h0.x, h, cnt)) p.hit[path] = hit_record(h);
 }
 
 // ---- stage 3: shade ---------------------------------------------------------------------------------------
@@ -703,6 +709,52 @@ struct ShadeOut {
     bool shadow_query;  // an intersection_shadow-equivalent query was made (ray statistics)
     F4 sh_o, sh_d, sh_c;
 };
+
+// ---- pieces of one getColor iteration shared by shade_one and shade_branch_one ------------------------------------------------
+// next-event estimation: a point of the spherical light seen from P (Raytracer.cpp:494-510) and the density of its direction
+struct LightSample { V3 axeOP, dirl, xl, wi; float d2; };
+PTB_HD LightSample light_sample(const SceneDev& sc, V3 P, Pcg32& e) {
+    LightSample l;
+    l.axeOP = fast_normalize(P - sc.centerLight);
+    const float l1 = pcg32_uniform(e);
+    const float l2 = pcg32_uniform(e);
+    l.dirl = random_cos(l.axeOP, l1, l2);
+    l.xl = l.dirl * sc.radiusLight + sc.centerLight;
+    const V3 toL = l.xl - P;
+    l.wi = fast_normalize(toL);
+    l.d2 = norm2(toL);
+    return l;
+}
+PTB_HD float light_proba(const SceneDev& sc, const LightSample& l) {
+#if defined(__CUDA_ARCH__)
+    return dot(l.axeOP, l.dirl) / (PTB_PI_F * (sc.radiusLight * sc.radiusLight));
+#else
+    return (float)((double)dot(l.axeOP, l.dirl) / (PTB_PI_D * (double)(sc.radiusLight * sc.radiusLight)));
+#endif
+}
+// the MERL-or-Phong choice of shade_branch_one.  shade_one spells it out: through a helper nvcc fuses different products of the MERL
+// lookup into FMAs, and the linear render would no longer compute what it did.
+template <bool MERL>
+PTB_HD V3 brdf_eval(const SceneDev& sc, const ObjectDev& ob, const Surface& s, V3 wi, V3 wo, V3 N) {
+    if (MERL && ob.brdf == 1) return merl_eval(sc.merl + (size_t)ob.merl * 3 * PTB_MERL_N, wi, wo, N);
+    return phong_eval(s.Kd, s.Ks, s.Ne, wi, wo, N);
+}
+// the shadow ray of a direct term, for the BVH: `owner` = path or sample slot, `tag` = sh_c.w
+PTB_HD void queue_shadow(ShadeOut& out, V3 so, V3 wi, float dist, uint32_t owner, V3 c, uint32_t tag) {
+    out.shadow = true;
+    out.sh_o.x = so.x; out.sh_o.y = so.y; out.sh_o.z = so.z; out.sh_o.w = (float)((double)dist * 0.999);
+    out.sh_d.x = wi.x; out.sh_d.y = wi.y; out.sh_d.z = wi.z; out.sh_d.w = u2f(owner);
+    out.sh_c.x = c.x; out.sh_c.y = c.y; out.sh_c.z = c.z; out.sh_c.w = u2f(tag);
+}
+// the path's next ray, with the analytic half of its closest hit
+template <bool EXOTIC = true>
+PTB_HD void set_next_ray(const SceneDev& sc, PoolDev& p, int path, V3 no, V3 nd, V3 nw, uint32_t state) {
+    F4 q;
+    q.x = no.x; q.y = no.y; q.z = no.z; q.w = 0; p.ray_o[path] = q;
+    q.x = nd.x; q.y = nd.y; q.z = nd.z; q.w = 0; p.ray_d[path] = q;
+    q.x = nw.x; q.y = nw.y; q.z = nw.z; q.w = u2f(state); p.weight[path] = q;
+    p.hit[path] = analytic_hit<EXOTIC>(sc, no, nd);
+}
 
 // MERL = the scene holds at least one IsoMERLBRDF object; scenes without one get a kernel free of the double-precision
 // lookup code (fewer registers, higher occupancy).
@@ -752,6 +804,7 @@ PTB_HD void shade_one(const SceneDev& sc, const FrameDev& f, PoolDev& p, int pat
         nd = reflect(rd, N);
         no = P + 0.001f * N;
     } else if (s.transp) {                                           // 438-489
+        // (shade_branch_one has the same lines: as a shared helper nvcc fuses dot(Nt, rd) into FMAs the other way round)
         float n1 = 1.f, n2 = s.refr_index;
         V3 Nt = N;
         bool entering = true;
@@ -776,24 +829,15 @@ PTB_HD void shade_one(const SceneDev& sc, const FrameDev& f, PoolDev& p, int pat
     } else {                                                         // opaque, 490-649
         Pcg32 e; e.state = p.rng[path]; e.inc = path_inc(f, path);
         // -- next-event estimation on the spherical light (494-566)
-        const V3 axeOP = fast_normalize(P - sc.centerLight);
-        const float l1 = pcg32_uniform(e);
-        const float l2 = pcg32_uniform(e);
-        const V3 dirl = random_cos(axeOP, l1, l2);
-        const V3 xl = dirl * sc.radiusLight + sc.centerLight;
-        const V3 toL = xl - P;
-        const V3 wi = fast_normalize(toL);
-        const float d2 = norm2(toL);
+        const LightSample l = light_sample(sc, P, e);
+        const V3 wi = l.wi;
+        const float d2 = l.d2;
         if (!(dot(N, wi) < 0)) {
             V3 fr;
             if (MERL && ob.brdf == 1) fr = merl_eval(sc.merl + (size_t)ob.merl * 3 * PTB_MERL_N, wi, -rd, N);
             else fr = phong_eval(s.Kd, s.Ks, s.Ne, wi, -rd, N);
-            const float J = dot(dirl, -wi) / d2;
-#if defined(__CUDA_ARCH__)
-            const float proba = dot(axeOP, dirl) / (PTB_PI_F * (sc.radiusLight * sc.radiusLight));
-#else
-            const float proba = (float)((double)dot(axeOP, dirl) / (PTB_PI_D * (double)(sc.radiusLight * sc.radiusLight)));
-#endif
+            const float J = dot(l.dirl, -wi) / d2;
+            const float proba = light_proba(sc, l);
             if (proba > 0.f) {
                 const float g = sc.lightPower * fmaxf(0.f, dot(N, wi)) * J / proba;
                 const V3 c = w * (g * fr);
@@ -803,12 +847,8 @@ PTB_HD void shade_one(const SceneDev& sc, const FrameDev& f, PoolDev& p, int pat
                 // analytic occluders (incl. the light itself and the dome, App. D#8) are tested here, coherently;
                 // only rays they do not block go on to the BVH
                 if (!analytic_occluded<EXOTIC>(sc, so, wi, dist)) {
-                    if (sc.has_mesh) {
-                        out.shadow = true;
-                        out.sh_o.x = so.x; out.sh_o.y = so.y; out.sh_o.z = so.z; out.sh_o.w = (float)((double)dist * 0.999);
-                        out.sh_d.x = wi.x; out.sh_d.y = wi.y; out.sh_d.z = wi.z; out.sh_d.w = u2f((uint32_t)path);
-                        out.sh_c.x = c.x; out.sh_c.y = c.y; out.sh_c.z = c.z; out.sh_c.w = 0;
-                    } else {
+                    if (sc.has_mesh) queue_shadow(out, so, wi, dist, (uint32_t)path, c, 0u);
+                    else {
                         Lq.x += c.x; Lq.y += c.y; Lq.z += c.z;
                         p.radiance[path] = Lq;
                     }
@@ -847,28 +887,24 @@ PTB_HD void shade_one(const SceneDev& sc, const FrameDev& f, PoolDev& p, int pat
     // loop-top tests of the next iteration (240-241): depth exhausted or weight below 0.01
     if (ndepth == 0 || norm2(nw) < 0.01f * 0.01f) return;
     // NaN weights fall through `<` like the reference; keep tracing them as it does
-    F4 q;
-    q.x = no.x; q.y = no.y; q.z = no.z; q.w = 0; p.ray_o[path] = q;
-    q.x = nd.x; q.y = nd.y; q.z = nd.z; q.w = 0; p.ray_d[path] = q;
-    q.x = nw.x; q.y = nw.y; q.z = nw.z; q.w = u2f(pack_state(ndepth, nshow)); p.weight[path] = q;
-    float ta; int32_t ida;
-    analytic_closest<EXOTIC>(sc, no, nd, ta, ida);
-    q.x = ta; q.y = 0; q.z = 0; q.w = u2f((uint32_t)ida); p.hit[path] = q;
+    set_next_ray<EXOTIC>(sc, p, path, no, nd, nw, pack_state(ndepth, nshow));
     out.cont = true;
 }
 
 // ---- stage 4: shadow rays through the wide BVH; unoccluded ones deliver the deferred direct term -----------------------
+// an unoccluded shadow ray of a linear render adds its deferred direct term to its path's radiance (Raytracer.cpp:545-566)
+PTB_HD void deliver_direct(PoolDev& p, uint32_t entry, uint32_t path) {
+    const F4 c = p.sh_c[entry];
+    F4 L = p.radiance[path];
+    L.x += c.x; L.y += c.y; L.z += c.z;
+    p.radiance[path] = L;
+}
 template <bool COUNT>
 PTB_HD void shadow_one(const SceneDev& sc, PoolDev& p, int entry, TraverseCounters* cnt) {
     const F4 o = p.sh_o[entry], d = p.sh_d[entry];
     const AlphaCtx ac = alpha_ctx(sc);
     Hit h;
-    if (traverse<true, COUNT>(sc.nodes, sc.tris, &ac, v3(o.x, o.y, o.z), v3(d.x, d.y, d.z), o.w, h, cnt)) return;
-    const uint32_t path = f2u(d.w);
-    const F4 c = p.sh_c[entry];
-    F4 L = p.radiance[path];
-    L.x += c.x; L.y += c.y; L.z += c.z;
-    p.radiance[path] = L;
+    if (!traverse<true, COUNT>(sc.nodes, sc.tris, &ac, v3(o.x, o.y, o.z), v3(d.x, d.y, d.z), o.w, h, cnt)) deliver_direct(p, (uint32_t)entry, f2u(d.w));
 }
 
 // ---- branching contributions: participating medium, ghost objects, background photograph ----------------------------
@@ -990,7 +1026,7 @@ PTB_HD float fog_sample(const SceneDev& sc, V3 ro, V3 rd, V3 lightPos, float t, 
 }
 
 // One iteration of getColor's loop (Raytracer.cpp:227-660) for the contribution in slot `path`, with the fog, ghost and
-// background branches; the subsurface branch (318-406) is not built.
+// background and subsurface (318-406) branches.
 template <bool MERL>
 PTB_HD void shade_branch_one(const SceneDev& sc, const FrameDev& f, PoolDev& p, int path, BranchOut& out) {
     out.base.cont = false; out.base.shadow = false; out.base.shadow_query = false;
@@ -1156,14 +1192,9 @@ PTB_HD void shade_branch_one(const SceneDev& sc, const FrameDev& f, PoolDev& p, 
         nstate = st_next | (show_lights ? ST_SHOW_LIGHTS : 0u) | ST_SHOW_ENV;
     } else {                                                         // opaque, 490-649
         const bool ghost = (ob.flags & FLAG_GHOST) != 0;
-        const V3 axeOP = fast_normalize(P - sc.centerLight);
-        const float l1 = pcg32_uniform(e);
-        const float l2 = pcg32_uniform(e);
-        const V3 dirl = random_cos(axeOP, l1, l2);
-        const V3 xl = dirl * sc.radiusLight + sc.centerLight;
-        const V3 toL = xl - P;
-        const V3 wi = fast_normalize(toL);
-        const float d2 = norm2(toL);
+        const LightSample l = light_sample(sc, P, e);
+        const V3 wi = l.wi, xl = l.xl;
+        const float d2 = l.d2;
         bool shadowed = true, pending = false;                       // pending: only the BVH can tell
         const V3 so = P + 0.01f * wi;
         const float dist = sqrtf(d2) - 0.01f;
@@ -1186,14 +1217,9 @@ PTB_HD void shade_branch_one(const SceneDev& sc, const FrameDev& f, PoolDev& p, 
             } else {
                 V3 fr;
                 if (sub_interaction) fr = s.Ksub / PTB_PI_F;
-                else if (MERL && ob.brdf == 1) fr = merl_eval(sc.merl + (size_t)ob.merl * 3 * PTB_MERL_N, wi, -sd, N);
-                else fr = phong_eval(s.Kd, s.Ks, s.Ne, wi, -sd, N);
-                const float J = dot(dirl, -wi) / d2;
-#if defined(__CUDA_ARCH__)
-                const float proba = dot(axeOP, dirl) / (PTB_PI_F * (sc.radiusLight * sc.radiusLight));
-#else
-                const float proba = (float)((double)dot(axeOP, dirl) / (PTB_PI_D * (double)(sc.radiusLight * sc.radiusLight)));
-#endif
+                else fr = brdf_eval<MERL>(sc, ob, s, wi, -sd, N);
+                const float J = dot(l.dirl, -wi) / d2;
+                const float proba = light_proba(sc, l);
                 if (proba > 0.f) direct = (subsW * (sc.lightPower * fmaxf(0.f, dot(N, wi)) * J / proba)) * fr;
             }
         }
@@ -1203,17 +1229,10 @@ PTB_HD void shade_branch_one(const SceneDev& sc, const FrameDev& f, PoolDev& p, 
         if (has_fog) att = fog_sample(sc, ro, cur_d, xl, t, w, st_fogchild, e, out.fog);
         const V3 c = (w * att) * direct;
         if (!shadowed && !ghost) {
-            if (pending) {
-                out.base.shadow = true;
-                out.base.sh_o.x = so.x; out.base.sh_o.y = so.y; out.base.sh_o.z = so.z; out.base.sh_o.w = (float)((double)dist * 0.999);
-                out.base.sh_d.x = wi.x; out.base.sh_d.y = wi.y; out.base.sh_d.z = wi.z; out.base.sh_d.w = u2f(root);
-                out.base.sh_c.x = c.x; out.base.sh_c.y = c.y; out.base.sh_c.z = c.z; out.base.sh_c.w = u2f(0u);
-            } else radiance_add(p, root, c);
+            if (pending) queue_shadow(out.base, so, wi, dist, root, c, 0u);
+            else radiance_add(p, root, c);
         } else if (ghost && out.ghost_pending) {                     // the shadow ray decides the ghost child's fate and showenvmap below
-            out.base.shadow = true;
-            out.base.sh_o.x = so.x; out.base.sh_o.y = so.y; out.base.sh_o.z = so.z; out.base.sh_o.w = (float)((double)dist * 0.999);
-            out.base.sh_d.x = wi.x; out.base.sh_d.y = wi.y; out.base.sh_d.z = wi.z; out.base.sh_d.w = u2f((uint32_t)path);
-            out.base.sh_c.x = 0; out.base.sh_c.y = 0; out.base.sh_c.z = 0; out.base.sh_c.w = u2f(0x80000000u);   // | child slot, set by the kernel
+            queue_shadow(out.base, so, wi, dist, (uint32_t)path, v3(0, 0, 0), 0x80000000u);   // | child slot, set by the kernel
         }
         // -- continuation (570-632)
         float sx, sy;
@@ -1235,10 +1254,7 @@ PTB_HD void shade_branch_one(const SceneDev& sc, const FrameDev& f, PoolDev& p, 
             dir = phong_sample(s.Ks, s.Ne, -sd, N, r1, r2, u, pdf, diffuse);
         }
         if (dot(dir, N) < 0 || dot(dir, reflect(sd, N)) < 0 || pdf <= 0) return;
-        V3 fi;
-        if (sub_interaction) fi = s.Ksub / PTB_PI_F;
-        else if (MERL && ob.brdf == 1) fi = merl_eval(sc.merl + (size_t)ob.merl * 3 * PTB_MERL_N, dir, -sd, N);
-        else fi = phong_eval(s.Kd, s.Ks, s.Ne, dir, -sd, N);
+        const V3 fi = sub_interaction ? s.Ksub / PTB_PI_F : brdf_eval<MERL>(sc, ob, s, dir, -sd, N);
         nw = ((w * subsW) * fi) * (dot(N, dir) / pdf);
         if (ghost && sc.bgW > 0) nw = nw * (background_at(sc, f, pix) / 196964.699f);   // 614-621
         if (has_fog) nw = att * nw;
@@ -1251,13 +1267,7 @@ PTB_HD void shade_branch_one(const SceneDev& sc, const FrameDev& f, PoolDev& p, 
     }
     p.rng[path] = e.state;
     if (depth - 1 == 0 || norm2(nw) < 0.01f * 0.01f) return;         // 240-241 of the next iteration
-    F4 q;
-    q.x = no.x; q.y = no.y; q.z = no.z; q.w = 0; p.ray_o[path] = q;
-    q.x = nd.x; q.y = nd.y; q.z = nd.z; q.w = 0; p.ray_d[path] = q;
-    q.x = nw.x; q.y = nw.y; q.z = nw.z; q.w = u2f(nstate); p.weight[path] = q;
-    float ta; int32_t ida;
-    analytic_closest(sc, no, nd, ta, ida);
-    q.x = ta; q.y = 0; q.z = 0; q.w = u2f((uint32_t)ida); p.hit[path] = q;
+    set_next_ray(sc, p, path, no, nd, nw, nstate);
     out.base.cont = true;
 }
 // Scene::get_random_intersection restricted to one TriMesh (Geometry.cpp:339-472, TriangleMesh.cpp:1321-1424): a uniformly random
@@ -1285,18 +1295,14 @@ PTB_HD void probe_one(const SceneDev& sc, PoolDev& p, int entry) {
         const AlphaCtx ac = alpha_ctx(sc);
         traverse_all(sc.nodes, sc.tris, &ac, v3(o.x, o.y, o.z), v3(d.x, d.y, d.z), o.w, pick);
     }
-    F4 q; q.x = pick.best.t; q.y = pick.best.b1; q.z = pick.best.b2; q.w = u2f((uint32_t)pick.best.prim);
-    p.hit2[f2u(d.w)] = q;
+    p.hit2[f2u(d.w)] = hit_record(pick.best);
 }
 
 // Store a side branch in pool slot `slot` (the kernel / host loop allocated it) and give its ray the analytic hit record.
 PTB_HD void store_child(const SceneDev& sc, PoolDev& p, uint32_t slot, const ChildOut& ch, uint32_t root, uint32_t pix) {
     p.ray_o[slot] = ch.o; p.ray_d[slot] = ch.d; p.weight[slot] = ch.w;
     p.rng[slot] = ch.rng; p.pixel[slot] = pix; p.root[slot] = root;
-    float ta; int32_t ida;
-    analytic_closest(sc, v3(ch.o.x, ch.o.y, ch.o.z), v3(ch.d.x, ch.d.y, ch.d.z), ta, ida);
-    F4 q; q.x = ta; q.y = 0; q.z = 0; q.w = u2f((uint32_t)ida);
-    p.hit[slot] = q;
+    p.hit[slot] = analytic_hit(sc, v3(ch.o.x, ch.o.y, ch.o.z), v3(ch.d.x, ch.d.y, ch.d.z));
 }
 // What the any-hit pass does with a finished shadow ray of a branching render: deliver the deferred direct term to the sample
 // slot, or settle a ghost hit (Raytracer.cpp:519-537, 626-629): blocked -> the straight-through child dies; clear -> the
