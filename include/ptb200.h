@@ -270,7 +270,8 @@ int ptb_render(ptb_ctx*, const ptb_camera*, const ptb_params*,
  *   imagedouble       mean radiance                           albedoImage   mean first-hit albedo
  *   normalImage       what the reference stores there: it sums the COLOUR buffers instead of the normals (1680-1682) and
  *                     normalises, i.e. the normalised radiance sum (NaN where it is zero)
- *   first_hit_normal  the normalised sum of the first-hit shading normals, the quantity 1680-1682 was written to produce */
+ *   first_hit_normal  the normalised sum of the first-hit shading normals, the quantity 1680-1682 was written to produce
+ * With p->shard_count > 1 only the shard's tiles are rendered: the outputs stay full-frame, sample_count 0 outside them. */
 int ptb_render_denoiser_inputs(ptb_ctx*, const ptb_camera*, const ptb_params*, float* imagedouble, float* sample_count,
                                float* albedoImage, float* normalImage, float* first_hit_normal, ptb_stats* stats);
 
@@ -284,7 +285,8 @@ int ptb_render_denoiser_inputs(ptb_ctx*, const ptb_camera*, const ptb_params*, f
  *   sample_count        W*H   filter weight sums (1495)
  *   image               W*H*3 255*(imagedouble/196964.7/max(sample_count,1))^(1/gamma) (1543-1545)
  *   imagedouble_lowres  ceil(W/16)*ceil(H/16)*3: every sample adds colour/256 to its 16x16 block (1508-1510)
- *   current_nb_rays     passes accumulated so far (Raytracer::current_nb_rays, 1445) */
+ *   current_nb_rays     passes accumulated so far (Raytracer::current_nb_rays, 1445)
+ * With p->shard_count > 1 the session renders the shard's tiles only (sample_count 0 outside them, and their splat apron). */
 int ptb_progressive_begin(ptb_ctx*, const ptb_camera*, const ptb_params*);
 int ptb_progressive_pass(ptb_ctx*, int n_spp, ptb_stats* stats);
 int ptb_progressive_read(ptb_ctx*, float* imagedouble, float* sample_count, uint8_t* image, float* imagedouble_lowres,
@@ -324,6 +326,20 @@ int ptb_comm_destroy(ptb_ctx*);
 int ptb_render_sharded(ptb_ctx*, const ptb_camera*, const ptb_params*,
                        float* imagedouble, float* sample_count, uint8_t* image, ptb_stats* stats);
 int ptb_resolve_last(ptb_ctx*, int W, int H, float gamma, float* imagedouble, float* sample_count, uint8_t* image);
+/* The other two renderers on every rank of the communicator, called like ptb_render_sharded (same camera and parameters on every
+ * rank; the shard comes from the communicator, one rank renders the whole frame).
+ * replaces: Raytracer::render_image_nopreviz with has_denoiser (ptb_render_denoiser_inputs).  Rank 0 receives the outputs of
+ * ptb_render_denoiser_inputs; the other ranks ignore their output pointers.  The samples are box-filtered, so the tiles travel
+ * without an apron (colour, albedo and normal sums: 48 bytes per owned pixel).
+ * replaces: Raytracer::render_image (ptb_progressive_begin / _read).  begin_sharded starts a session over this rank's tiles and
+ * ptb_progressive_pass renders them.  read_sharded is COLLECTIVE: every rank calls it after the same passes; rank 0 receives the
+ * outputs of ptb_progressive_read (the 16x16 preview is summed over the ranks) and the session goes on.  ptb_progressive_read on
+ * a session begun here, and ptb_progressive_read_sharded on one begun with ptb_progressive_begin, return PTB_ERR_STATE. */
+int ptb_render_denoiser_inputs_sharded(ptb_ctx*, const ptb_camera*, const ptb_params*, float* imagedouble, float* sample_count,
+                                       float* albedoImage, float* normalImage, float* first_hit_normal, ptb_stats* stats);
+int ptb_progressive_begin_sharded(ptb_ctx*, const ptb_camera*, const ptb_params*);
+int ptb_progressive_read_sharded(ptb_ctx*, float* imagedouble, float* sample_count, uint8_t* image, float* imagedouble_lowres,
+                                 int32_t* current_nb_rays);
 
 /* (2) One process, several GPUs: a group owns one context (and, during a render, one host thread) per device.  The scene is handed
  * to the LEADER context, ptb_group_ctx(g, 0), with the ptb_add_* / ptb_set_* calls above; ptb_group_commit flattens it and builds
@@ -339,6 +355,15 @@ int  ptb_group_commit(ptb_group*);
 int  ptb_group_set_option(ptb_group*, int option, int64_t value);
 int  ptb_group_render(ptb_group*, const ptb_camera*, const ptb_params*,
                       float* imagedouble, float* sample_count, uint8_t* image, ptb_stats* stats);
+/* replaces: ptb_render_denoiser_inputs on all the group's devices (stats as ptb_group_render) */
+int  ptb_group_render_denoiser_inputs(ptb_group*, const ptb_camera*, const ptb_params*, float* imagedouble, float* sample_count,
+                                      float* albedoImage, float* normalImage, float* first_hit_normal, ptb_stats* stats);
+/* replaces: ptb_progressive_begin / _pass / _read on all the group's devices (pass stats as ptb_group_render).  Pass or read
+ * before begin returns PTB_ERR_STATE.  Like ptb_group_render, begin re-poses a key-framed scene after ptb_set_frame on the leader. */
+int  ptb_group_progressive_begin(ptb_group*, const ptb_camera*, const ptb_params*);
+int  ptb_group_progressive_pass(ptb_group*, int n_spp, ptb_stats* stats);
+int  ptb_group_progressive_read(ptb_group*, float* imagedouble, float* sample_count, uint8_t* image, float* imagedouble_lowres,
+                                int32_t* current_nb_rays);
 
 /* Host output buffers that live across frames (Raytracer::imagedouble / sample_count / image are members, Raytracer.h:90-105) can
  * be page-locked once, so that the device->host copies that end a render run at PCIe speed without a staging copy.  The buffer

@@ -112,7 +112,9 @@ SYMBOLS = ["create", "destroy", "last_error", "version", "add_sphere", "add_plan
            "progressive_read"]
 # material presets, multi-GPU and host-buffer entry points: the CUDA library only (the CPU checkers under oracle/ and tests/devsim do not have them)
 MULTI_SYMBOLS = ["preset_count", "preset_get", "preset_find", "comm_unique_id", "comm_init", "comm_destroy", "render_sharded", "resolve_last", "group_create", "group_destroy", "group_last_error",
-                 "group_size", "group_ctx", "group_commit", "group_set_option", "group_render", "pin_host_buffer", "unpin_host_buffer"]
+                 "group_size", "group_ctx", "group_commit", "group_set_option", "group_render", "pin_host_buffer", "unpin_host_buffer",
+                 "render_denoiser_inputs_sharded", "progressive_begin_sharded", "progressive_read_sharded", "group_render_denoiser_inputs",
+                 "group_progressive_begin", "group_progressive_pass", "group_progressive_read"]
 
 
 # ---- include/ptb_sceneio.h -------------------------------------------------------------------------
@@ -262,6 +264,13 @@ class Lib:
             "group_render": (C.c_int, [vp, C.POINTER(Camera), C.POINTER(Params), _fp, _fp, u8p, C.POINTER(Stats)]),
             "pin_host_buffer": (C.c_int, [vp, vp, C.c_int64]),
             "unpin_host_buffer": (C.c_int, [vp, vp]),
+            "render_denoiser_inputs_sharded": (C.c_int, [vp, C.POINTER(Camera), C.POINTER(Params), _fp, _fp, _fp, _fp, _fp, C.POINTER(Stats)]),
+            "progressive_begin_sharded": (C.c_int, [vp, C.POINTER(Camera), C.POINTER(Params)]),
+            "progressive_read_sharded": (C.c_int, [vp, _fp, _fp, u8p, _fp, C.POINTER(C.c_int32)]),
+            "group_render_denoiser_inputs": (C.c_int, [vp, C.POINTER(Camera), C.POINTER(Params), _fp, _fp, _fp, _fp, _fp, C.POINTER(Stats)]),
+            "group_progressive_begin": (C.c_int, [vp, C.POINTER(Camera), C.POINTER(Params)]),
+            "group_progressive_pass": (C.c_int, [vp, C.c_int, C.POINTER(Stats)]),
+            "group_progressive_read": (C.c_int, [vp, _fp, _fp, u8p, _fp, C.POINTER(C.c_int32)]),
         }
         assert sorted(multi) == sorted(MULTI_SYMBOLS)
         self.has_multi = hasattr(cdll, prefix + "render_sharded")

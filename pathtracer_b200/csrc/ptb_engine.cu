@@ -553,6 +553,24 @@ __global__ void __launch_bounds__(256) k_shard_pack(const F4* rgbw, F4* packed, 
     shard_texel(const_cast<F4*>(rgbw), packed, idx, W, H, tile, apron, tiles_x, n_tiles_total, shift, rank, count, unpack, RedAddV4());
 }
 
+// The same gather over up to three float4 planes of the frame at once (denoiser inputs: colour, albedo and normal sums): plane k of
+// the packed tiles lies at packed + k * n_packed, so that one message per rank carries them all.
+#define PTB_MAX_PLANES 3
+struct ShardPlanes { F4* p[PTB_MAX_PLANES]; int n; };
+__global__ void __launch_bounds__(256) k_shard_pack_planes(ShardPlanes pl, F4* packed, int W, int H, int tile, int apron, int tiles_x, int n_tiles_total, int shift,
+                                                           int rank, int count, long long n_packed, int unpack) {
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= n_packed) return;
+    for (int k = 0; k < pl.n; k++)
+        shard_texel(pl.p[k], packed + k * n_packed, idx, W, H, tile, apron, tiles_x, n_tiles_total, shift, rank, count, unpack, RedAddV4());
+}
+
+// dst[i] += src[i]: the progressive preview sums of one rank added into rank 0's copy
+__global__ void __launch_bounds__(256) k_add(const float* __restrict__ src, float* dst, long long n) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) dst[i] += src[i];
+}
+
 __global__ void k_kat(int which, SceneDev sc, CameraDev cam, FilterDev filt, int W, int H, const double* in, int n, int is, double* out, int os) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= n) return;
@@ -588,6 +606,9 @@ struct ptb_ctx {
     int64_t out_aux_n = 0;
     // progressive session (Raytracer::render_image): persistent accumulator + low-resolution preview
     bool prog_active = false;
+    bool prog_sharded = false;                 // begun with ptb_progressive_begin_sharded: read with ptb_progressive_read_sharded
+    F4* d_prog_gather = nullptr;               // rank 0 of a sharded session: the gathered sums of a read (the accumulator stays this rank's own)
+    int64_t prog_gather_n = 0;
     FrameDev prog_f;
     ptb_params prog_p;
     int prog_iter = 0;
@@ -837,7 +858,7 @@ void ptb_destroy(ptb_ctx* c) {
     c->pinned.clear();
     free_scene(c);
     free_pool(c);
-    void* ptrs[] = {c->d_counters, c->d_totals, c->d_rpp, c->d_accum, c->d_out_img, c->d_out_cnt, c->d_out_u8, c->d_aux, c->d_out_aux, c->d_prog_accum, c->d_lowres, c->d_pack, c->d_node_box};
+    void* ptrs[] = {c->d_counters, c->d_totals, c->d_rpp, c->d_accum, c->d_out_img, c->d_out_cnt, c->d_out_u8, c->d_aux, c->d_out_aux, c->d_prog_accum, c->d_prog_gather, c->d_lowres, c->d_pack, c->d_node_box};
     for (void* p : ptrs) if (p) cudaFree(p);
     cudaEventDestroy(c->ev0); cudaEventDestroy(c->ev1);
     for (cudaEvent_t e : c->ev_pool) cudaEventDestroy(e);
@@ -1354,18 +1375,12 @@ int ptb_render(ptb_ctx* c, const ptb_camera* cam, const ptb_params* p, float* im
     return PTB_OK;
 }
 
-// render_image_nopreviz with has_denoiser == true (Raytracer.cpp:1631-1645, 1676-1693), up to the point where the reference
-// hands the buffers to Open Image Denoise
-int ptb_render_denoiser_inputs(ptb_ctx* c, const ptb_camera* cam, const ptb_params* p, float* imagedouble, float* sample_count, float* albedoImage,
-                               float* normalImage, float* first_hit_normal, ptb_stats* stats) {
-    if (!c) return PTB_ERR_INVALID;
-    if (!c->committed) { c->err = "render before commit"; return PTB_ERR_STATE; }
-    { const int rf = ensure_frame(c); if (rf) return rf; }
-    CK(cudaSetDevice(c->device));
+// The has_denoiser accumulation of the shard `p` names (every tile for a whole frame): colour and count sums in d_accum, first-hit
+// albedo sums in d_aux[0, n), first-hit normal sums in d_aux[n, 2n) (n = W*H; pixels outside the shard stay zero)
+static int denoiser_render(ptb_ctx* c, const ptb_camera* cam, const ptb_params* p, ptb_stats* stats) {
     FrameDev f;
     int rc = frame_setup(c, cam, p, f);
     if (rc) return rc;
-    if (f.shard_count != 1) { c->err = "render_denoiser_inputs: whole frames only"; return PTB_ERR_UNSUPPORTED; }
     const int64_t n = (int64_t)p->W * p->H;
     if ((rc = grow(c, &c->d_accum, &c->accum_n, n))) return rc;
     if ((rc = grow(c, &c->d_aux, &c->aux_n, 2 * n))) return rc;
@@ -1375,7 +1390,10 @@ int ptb_render_denoiser_inputs(ptb_ctx* c, const ptb_camera* cam, const ptb_para
     f.box_filter = 1;
     f.accum_albedo = c->d_aux;
     f.accum_normal = c->d_aux + n;
-    if ((rc = render_passes(c, f, p->nrays, c->d_accum, stats))) return rc;
+    return render_passes(c, f, p->nrays, c->d_accum, stats);
+}
+// ... and its resolve into host outputs (any may be NULL)
+static int denoiser_resolve(ptb_ctx* c, int64_t n, float* imagedouble, float* sample_count, float* albedoImage, float* normalImage, float* first_hit_normal) {
     float* o = c->d_out_aux;   // staged back to back: imagedouble 3n | sample_count n | albedo 3n | normal 3n | first-hit normal 3n
     k_resolve_denoiser<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(c->d_accum, c->d_aux, c->d_aux + n, (size_t)n, o, o + 3 * n, o + 4 * n, o + 7 * n, o + 10 * n);
     CK(cudaGetLastError());
@@ -1385,16 +1403,26 @@ int ptb_render_denoiser_inputs(ptb_ctx* c, const ptb_camera* cam, const ptb_para
     return PTB_OK;
 }
 
-// ---- progressive rendering: Raytracer::render_image (Raytracer.cpp:1424-1563) one batch of passes at a time ---------------------
-int ptb_progressive_begin(ptb_ctx* c, const ptb_camera* cam, const ptb_params* p) {
+// render_image_nopreviz with has_denoiser == true (Raytracer.cpp:1631-1645, 1676-1693), up to the point where the reference
+// hands the buffers to Open Image Denoise.  A shard (p->shard_count > 1) fills the full-frame outputs; its pixels outside its
+// tiles have sample_count 0.
+int ptb_render_denoiser_inputs(ptb_ctx* c, const ptb_camera* cam, const ptb_params* p, float* imagedouble, float* sample_count, float* albedoImage,
+                               float* normalImage, float* first_hit_normal, ptb_stats* stats) {
     if (!c) return PTB_ERR_INVALID;
     if (!c->committed) { c->err = "render before commit"; return PTB_ERR_STATE; }
     { const int rf = ensure_frame(c); if (rf) return rf; }
     CK(cudaSetDevice(c->device));
+    int rc = denoiser_render(c, cam, p, stats);
+    if (rc) return rc;
+    return denoiser_resolve(c, (int64_t)p->W * p->H, imagedouble, sample_count, albedoImage, normalImage, first_hit_normal);
+}
+
+// ---- progressive rendering: Raytracer::render_image (Raytracer.cpp:1424-1563) one batch of passes at a time ---------------------
+// A session over the shard `p` names (every tile for a whole frame); `sharded`: begun by ptb_progressive_begin_sharded
+static int progressive_begin(ptb_ctx* c, const ptb_camera* cam, const ptb_params* p, bool sharded) {
     c->prog_active = false;
     int rc = frame_setup(c, cam, p, c->prog_f);
     if (rc) return rc;
-    if (c->prog_f.shard_count != 1) { c->err = "progressive: whole frames only"; return PTB_ERR_UNSUPPORTED; }
     const int64_t n = (int64_t)p->W * p->H;
     const int Wlr = (int)ceilf(p->W / 16.f), Hlr = (int)ceilf(p->H / 16.f);     // Raytracer.cpp:1329-1330
     if ((rc = grow(c, &c->d_prog_accum, &c->prog_n, n))) return rc;
@@ -1405,8 +1433,18 @@ int ptb_progressive_begin(ptb_ctx* c, const ptb_camera* cam, const ptb_params* p
     c->prog_f.lowres = c->d_lowres; c->prog_f.lowresW = Wlr; c->prog_f.lowresH = Hlr;
     c->prog_p = *p;
     c->prog_iter = 0;
+    c->prog_sharded = sharded;
     c->prog_active = true;
     return PTB_OK;
+}
+
+// A shard (p->shard_count > 1) renders its tiles only: read gives full-frame outputs whose pixels outside them have sample_count 0.
+int ptb_progressive_begin(ptb_ctx* c, const ptb_camera* cam, const ptb_params* p) {
+    if (!c) return PTB_ERR_INVALID;
+    if (!c->committed) { c->err = "render before commit"; return PTB_ERR_STATE; }
+    { const int rf = ensure_frame(c); if (rf) return rf; }
+    CK(cudaSetDevice(c->device));
+    return progressive_begin(c, cam, p, false);
 }
 
 int ptb_progressive_pass(ptb_ctx* c, int n_spp, ptb_stats* stats) {
@@ -1422,24 +1460,31 @@ int ptb_progressive_pass(ptb_ctx* c, int n_spp, ptb_stats* stats) {
     return PTB_OK;
 }
 
-int ptb_progressive_read(ptb_ctx* c, float* imagedouble, float* sample_count, uint8_t* image, float* imagedouble_lowres, int32_t* current_nb_rays) {
-    if (!c) return PTB_ERR_INVALID;
-    if (!c->prog_active) { c->err = "progressive_read before progressive_begin"; return PTB_ERR_STATE; }
-    CK(cudaSetDevice(c->device));
+// The outputs of a progressive read from the session's sums `accum` (W*H float4) and preview sums `lowres`
+static int progressive_resolve(ptb_ctx* c, const F4* accum, const float* lowres, float* imagedouble, float* sample_count, uint8_t* image, float* imagedouble_lowres,
+                               int32_t* current_nb_rays) {
     const ptb_params& p = c->prog_p;
     const int64_t n = (int64_t)p.W * p.H;
     const int rc = ensure_staging(c, n);
     if (rc) return rc;
-    k_resolve_progressive<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(c->d_prog_accum, (size_t)n, p.gamma, imagedouble ? c->d_out_img : nullptr,
+    k_resolve_progressive<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(accum, (size_t)n, p.gamma, imagedouble ? c->d_out_img : nullptr,
                                                                              sample_count ? c->d_out_cnt : nullptr, image ? c->d_out_u8 : nullptr);
     CK(cudaGetLastError());
     if (imagedouble) CK(cudaMemcpyAsync(imagedouble, c->d_out_img, (size_t)n * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
     if (sample_count) CK(cudaMemcpyAsync(sample_count, c->d_out_cnt, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
     if (image) CK(cudaMemcpyAsync(image, c->d_out_u8, (size_t)n * 3, cudaMemcpyDeviceToHost, c->stream));
-    if (imagedouble_lowres) CK(cudaMemcpyAsync(imagedouble_lowres, c->d_lowres, (size_t)c->prog_f.lowresW * c->prog_f.lowresH * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    if (imagedouble_lowres) CK(cudaMemcpyAsync(imagedouble_lowres, lowres, (size_t)c->prog_f.lowresW * c->prog_f.lowresH * 3 * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
     CK(cudaStreamSynchronize(c->stream));
     if (current_nb_rays) *current_nb_rays = c->prog_iter;
     return PTB_OK;
+}
+
+int ptb_progressive_read(ptb_ctx* c, float* imagedouble, float* sample_count, uint8_t* image, float* imagedouble_lowres, int32_t* current_nb_rays) {
+    if (!c) return PTB_ERR_INVALID;
+    if (!c->prog_active) { c->err = "progressive_read before progressive_begin"; return PTB_ERR_STATE; }
+    if (c->prog_sharded) { c->err = "progressive_read: the session was begun with ptb_progressive_begin_sharded; read it with ptb_progressive_read_sharded"; return PTB_ERR_STATE; }
+    CK(cudaSetDevice(c->device));
+    return progressive_resolve(c, c->d_prog_accum, c->d_lowres, imagedouble, sample_count, image, imagedouble_lowres, current_nb_rays);
 }
 
 int ptb_shard_pack_size(const ptb_params* p, int shard_rank, int64_t* out_floats) {
