@@ -433,6 +433,13 @@ int ptb_get_scene_info(const ptb_ctx*, ptb_scene_info*);
 #define PTB_KAT_MERL_INDEX     12  /* in: wi3,wo3 (local frame, z = normal) -> out: bin index of the float path (-1: it declined), bin index of
                                       the double path (MERLBRDFRead.cpp:76-207); the two must agree wherever the first is >= 0 */
 /* KAT 13 is retired (the half-factor node test, measured slower and removed).  Do not reuse the number. */
+#define PTB_KAT_RAY            14  /* needs a committed scene.  in: o[3], d[3], tmax, any_hit (float rays: the doubles are narrowed,
+                                      -0.0 stays -0.0).  Closest hit (any_hit = 0): Scene::intersection restricted to t < tmax -> out:
+                                      object id, original triangle id (-1: not a triangle), t, b1, b2; a miss is -1, -1, -1, 0, 0.
+                                      Any hit: Scene::intersection_shadow(o, d, dist_light = tmax) (ghosts pass) -> out: occluded 0/1,
+                                      0, 0, 0, 0.  One thread per ray over the plain BVH8 walk (traverse<>, as k_primary). */
+#define PTB_KAT_RAY_WAVEFRONT  15  /* the same rows through the render's wavefront kernels: k_trace then k_exact, over the path pool
+                                      (closest hit) or the shadow queue (any hit).  The CPU checkers answer it like PTB_KAT_RAY. */
 int ptb_kat(ptb_ctx*, int which, const ptb_camera* cam, int W, int H,
             const double* in, int n, int in_stride, double* out, int out_stride);
 

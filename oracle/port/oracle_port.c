@@ -1942,9 +1942,35 @@ int ptb_get_scene_info(const ptb_ctx* c, ptb_scene_info* info) {
     return PTB_OK;
 }
 int ptb_get_kernel_times(const ptb_ctx* c, ptb_kernel_times* t) { (void)c; (void)t; return PTB_ERR_UNSUPPORTED; }
+/* PTB_KAT_RAY / PTB_KAT_RAY_WAVEFRONT on one float ray (the doubles narrowed, a zero keeps its sign): Scene::intersection restricted to
+ * t < tmax -> object id, original triangle id (-1: not a triangle), t, b1, b2 (a miss: -1, -1, -1, 0, 0), or, any_hit != 0,
+ * Scene::intersection_shadow(o, d, dist_light = tmax) -> occluded 0/1, 0, 0, 0, 0.  The reference's decisions near edges. */
+static void kat_ray(const struct ptb_ctx* c, const double* a, double* out) {
+    vec o = V((float)a[0], (float)a[1], (float)a[2]), d = V((float)a[3], (float)a[4], (float)a[5]);
+    float tmax = (float)a[6];
+    out[0] = -1; out[1] = -1; out[2] = -1; out[3] = 0; out[4] = 0;
+    if (a[7] != 0) { out[0] = scene_shadow(c, o, d, tmax, NULL); out[1] = out[2] = 0; return; }
+    vec P; matvals m = matvals_default(); int id = -1, tri = -1; float t;
+    if (!scene_hit(c, o, d, &P, &id, &t, &m, &tri, NULL) || !(t < tmax)) return;
+    const object* ob = c->objs[id];
+    out[0] = id; out[2] = t;
+    if (ob->type == T_MESH && tri >= 0) {
+        vec dl = xf_dir(ob->inv, d), ol = xf_point(ob->inv, o), lp; float lt, al, be, ga;
+        soup_hit(&ob->soup[tri], ol, dl, &lp, &lt, &al, &be, &ga);   /* the barycentrics mesh_hit found the hit with */
+        out[1] = ob->permuted[tri]; out[3] = be; out[4] = ga;
+    }
+}
+
 int ptb_kat(ptb_ctx* c, int which, const ptb_camera* cam, int W, int H, const double* in, int n, int is, double* out, int os) {
     if (!c || !in || !out) return PTB_ERR_INVALID;
     if (cam) set_frame(c, cam, W, H);
+    if (which == PTB_KAT_RAY || which == PTB_KAT_RAY_WAVEFRONT) {
+        if (!c->committed) return PTB_ERR_STATE;
+        for (int i = 0; i < c->n_objs; i++) build_matrix(c->objs[i], (float)c->current_frame);
+#pragma omp parallel for schedule(dynamic, 256)
+        for (int k = 0; k < n; k++) kat_ray(c, in + (size_t)k * is, out + (size_t)k * os);
+        return PTB_OK;
+    }
     if (which == PTB_KAT_RANDOM_PER_PIXEL || which == PTB_KAT_FILTER_RATIO) {
         if (!c->committed) return PTB_ERR_STATE;
         c->W = W; c->H = H;

@@ -24,10 +24,12 @@ ORC_OPT_THREADS = 100
 (KAT_PCG32, KAT_LATTICE, KAT_CAMERA, KAT_RANDOM_COS, KAT_RANDOM_PHONG, KAT_PHONG_EVAL, KAT_MERL_EVAL,
  KAT_FAST_EXP, KAT_FAST_NORMALIZE, KAT_RANDOM_PER_PIXEL, KAT_FILTER_RATIO, KAT_MERL_INDEX) = range(1, 13)
 # KAT 13 is retired (the half-factor node test, removed): do not reuse
+KAT_RAY, KAT_RAY_WAVEFRONT = 14, 15   # ray queries on a committed scene: the plain BVH8 walk / the render's k_trace + k_exact
 KAT_SHAPES = {  # which -> (n_in, n_out)
     KAT_PCG32: (2, 4), KAT_LATTICE: (1, 2), KAT_CAMERA: (6, 6), KAT_RANDOM_COS: (5, 3),
     KAT_RANDOM_PHONG: (6, 3), KAT_PHONG_EVAL: (18, 3), KAT_MERL_EVAL: (9, 3), KAT_FAST_EXP: (1, 1),
     KAT_FAST_NORMALIZE: (3, 3), KAT_RANDOM_PER_PIXEL: (1, 2), KAT_FILTER_RATIO: (3, 1), KAT_MERL_INDEX: (6, 2),
+    KAT_RAY: (8, 5), KAT_RAY_WAVEFRONT: (8, 5),
 }
 
 _fp = C.POINTER(C.c_float)

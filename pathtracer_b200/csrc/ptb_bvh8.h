@@ -84,10 +84,14 @@ PTB_HD RayPrep ray_prep(V3 o, V3 d) {
     RayPrep r;
     r.o = o; r.d = d;
     const float eps = 1e-30f;
-    r.idir.x = 1.f / (fabsf(d.x) > eps ? d.x : copysignf(eps, d.x));
-    r.idir.y = 1.f / (fabsf(d.y) > eps ? d.y : copysignf(eps, d.y));
-    r.idir.z = 1.f / (fabsf(d.z) > eps ? d.z : copysignf(eps, d.z));
-    const uint32_t oinv = (d.x < 0 ? 0u : 4u) | (d.y < 0 ? 0u : 2u) | (d.z < 0 ? 0u : 1u);
+    // One sign per axis for the substitute of a tiny component, the octant and node_hitmask's entry plane: `d < 0`.  The sign bit
+    // (copysignf) would call -0.0 negative where the slab test calls it positive, swap the entry and exit planes on that axis and
+    // reject every node whose slab holds the origin (axis-aligned subsurface probes: -N0 of a face normal (0, 0, 1) is (-0, -0, -1)).
+    const bool nx = d.x < 0, ny = d.y < 0, nz = d.z < 0;
+    r.idir.x = 1.f / (fabsf(d.x) > eps ? d.x : (nx ? -eps : eps));
+    r.idir.y = 1.f / (fabsf(d.y) > eps ? d.y : (ny ? -eps : eps));
+    r.idir.z = 1.f / (fabsf(d.z) > eps ? d.z : (nz ? -eps : eps));
+    const uint32_t oinv = (nx ? 0u : 4u) | (ny ? 0u : 2u) | (nz ? 0u : 1u);
     // children are visited in descending (slot ^ oinv): first the half of the slots whose bit 2 differs from oinv's, ...
     r.oct_inv4 = oinv | ((oinv & 4u) ? 0x0f00u : 0xf000u) | ((oinv & 2u) ? 0x330000u : 0xcc0000u) | ((oinv & 1u) ? 0x55000000u : 0xaa000000u);
     return r;

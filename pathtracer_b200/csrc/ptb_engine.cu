@@ -577,6 +577,42 @@ __global__ void k_kat(int which, SceneDev sc, CameraDev cam, FilterDev filt, int
     kat_one(which, sc, cam, filt, W, H, in + (size_t)k * is, out + (size_t)k * os);
 }
 
+// PTB_KAT_RAY_WAVEFRONT: row k becomes path slot k and shadow entry k, as the render's producers write them.  Closest hit: ray_o,
+// ray_d and the analytic hit cut at tmax as the hit record (an any-hit row gets pixel = ~0, which k_trace skips).  Any hit: the shadow
+// ray with tmax = 0.999 * dist_light (queue_shadow), a unit direct term owed to slot k (zero if an analytic object occludes the ray)
+// and zeroed radiance, so that slot k's radiance is 1 exactly when k_trace / k_exact delivered the term: the ray is unoccluded.
+__global__ void __launch_bounds__(128) k_kat_rays(SceneDev sc, PoolDev p, const double* in, int n, int is) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    const double* a = in + (size_t)k * is;
+    V3 o, d;
+    float tmax;
+    kat_ray_in(a, o, d, tmax);
+    const bool any = a[7] != 0;
+    F4 q;
+    q.x = o.x; q.y = o.y; q.z = o.z; q.w = 0; p.ray_o[k] = q;
+    q.w = any ? (float)((double)tmax * 0.999) : 0.f; p.sh_o[k] = q;
+    q.x = d.x; q.y = d.y; q.z = d.z; q.w = 0; p.ray_d[k] = q;
+    q.w = u2f((uint32_t)k); p.sh_d[k] = q;
+    p.hit[k] = hit_record(kat_ray_analytic(sc, o, d, tmax));
+    p.pixel[k] = any ? 0xffffffffu : (uint32_t)k;
+    const float unit = (any && !analytic_occluded(sc, o, d, tmax)) ? 1.f : 0.f;
+    q.x = q.y = q.z = unit; q.w = 0; p.sh_c[k] = q;
+    q.x = q.y = q.z = 0; p.radiance[k] = q;
+}
+__global__ void __launch_bounds__(128) k_kat_rays_out(SceneDev sc, PoolDev p, const double* in, int n, int is, double* out, int os) {
+    const int k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= n) return;
+    double* o = out + (size_t)k * os;
+    if (in[(size_t)k * is + 7] != 0) {
+        o[0] = p.radiance[k].x == 1.f ? 0 : 1; o[1] = o[2] = o[3] = o[4] = 0;
+    } else {
+        const F4 h = p.hit[k];
+        const int32_t id = (int32_t)f2u(h.w);
+        kat_ray_out(sc, Hit{h.x, h.y, h.z, id}, id, o);
+    }
+}
+
 // ------------------------------------------------------------------------------------------------ context
 struct ptb_ctx {
     int device = 0;
@@ -1570,10 +1606,46 @@ int ptb_get_kernel_times(const ptb_ctx* c, ptb_kernel_times* out) {
     return PTB_OK;
 }
 
+}  // extern "C"
+
+// PTB_KAT_RAY_WAVEFRONT: the rows through k_trace + k_exact of both kinds (launch_trace, as a bounce runs them) over path slots / shadow
+// entries 0..n-1 of the pool
+static int kat_wavefront(ptb_ctx* c, const double* in, int n, int is, double* out, int os) {
+    int rc = ensure_pool(c, n);
+    if (rc) return rc;
+    double *d_in = nullptr, *d_out = nullptr;
+    uint32_t* d_cnt = nullptr;   // cursor and deferred-ray count of the closest-hit trace, then of the any-hit trace
+    CK(cudaMalloc((void**)&d_in, (size_t)n * is * 8)); CK(cudaMalloc((void**)&d_out, (size_t)n * os * 8)); CK(cudaMalloc((void**)&d_cnt, 4 * sizeof(uint32_t)));
+    const unsigned blocks = (unsigned)((n + 127) / 128), grid = (unsigned)std::max(1, std::min<int>(c->trace_blocks, (n + 127) / 128));
+    cudaError_t e = cudaMemcpyAsync(d_in, in, (size_t)n * is * 8, cudaMemcpyHostToDevice, c->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(d_cnt, 0, 4 * sizeof(uint32_t), c->stream);
+    if (e == cudaSuccess) {
+        k_kat_rays<<<blocks, 128, 0, c->stream>>>(c->sc, c->pool, d_in, n, is);
+        launch_trace<false, false>(c, grid, c->stream, c->pool, nullptr, nullptr, n, d_cnt, d_cnt + 1);
+        launch_trace<true, false>(c, grid, c->stream, c->pool, nullptr, nullptr, n, d_cnt + 2, d_cnt + 3);
+        k_kat_rays_out<<<blocks, 128, 0, c->stream>>>(c->sc, c->pool, d_in, n, is, d_out, os);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out, d_out, (size_t)n * os * 8, cudaMemcpyDeviceToHost, c->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+    cudaFree(d_in); cudaFree(d_out); cudaFree(d_cnt);
+    if (e != cudaSuccess) { c->err = std::string("kat: ") + cudaGetErrorString(e); return PTB_ERR_CUDA; }
+    return PTB_OK;
+}
+
+extern "C" {
+
 int ptb_kat(ptb_ctx* c, int which, const ptb_camera* cam, int W, int H, const double* in, int n, int is, double* out, int os) {
     if (!c || !in || !out || n <= 0) return PTB_ERR_INVALID;
     CK(cudaSetDevice(c->device));
     if (which == PTB_KAT_MERL_EVAL && (!c->committed || c->host.merl_tables.empty())) { c->err = "kat: MERL needs a committed scene with a table"; return PTB_ERR_STATE; }
+    if (which == PTB_KAT_RAY || which == PTB_KAT_RAY_WAVEFRONT) {
+        if (!c->committed) { c->err = "kat: ray queries need a committed scene"; return PTB_ERR_STATE; }
+        if (is < 8 || os < 5) return PTB_ERR_INVALID;
+        const int rf = ensure_frame(c);
+        if (rf) return rf;
+        if (which == PTB_KAT_RAY_WAVEFRONT) return kat_wavefront(c, in, n, is, out, os);
+    }
     CameraDev cd;
     memset(&cd, 0, sizeof(cd));
     if (cam) camera_from_abi(cd, cam, W, H);
@@ -1582,14 +1654,16 @@ int ptb_kat(ptb_ctx* c, int which, const ptb_camera* cam, int W, int H, const do
     if (which == PTB_KAT_FILTER_RATIO) filter_setup(fd, (float)in[2]);
     double *d_in = nullptr, *d_out = nullptr;
     CK(cudaMalloc((void**)&d_in, (size_t)n * is * 8)); CK(cudaMalloc((void**)&d_out, (size_t)n * os * 8));
-    cudaError_t e = cudaMemcpy(d_in, in, (size_t)n * is * 8, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMemset(d_out, 0, (size_t)n * os * 8);
+    // everything on the context's stream: it does not synchronise with the legacy default stream (cudaStreamNonBlocking), so a
+    // cudaMemset of d_out there could land after k_kat had written some rows and zero them
+    cudaError_t e = cudaMemcpyAsync(d_in, in, (size_t)n * is * 8, cudaMemcpyHostToDevice, c->stream);
+    if (e == cudaSuccess) e = cudaMemsetAsync(d_out, 0, (size_t)n * os * 8, c->stream);
     if (e == cudaSuccess) {
         k_kat<<<(n + 63) / 64, 64, 0, c->stream>>>(which, c->sc, cd, fd, W, H, d_in, n, is, d_out, os);
         e = cudaGetLastError();
     }
+    if (e == cudaSuccess) e = cudaMemcpyAsync(out, d_out, (size_t)n * os * 8, cudaMemcpyDeviceToHost, c->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-    if (e == cudaSuccess) e = cudaMemcpy(out, d_out, (size_t)n * os * 8, cudaMemcpyDeviceToHost);
     cudaFree(d_in); cudaFree(d_out);
     if (e != cudaSuccess) { c->err = std::string("kat: ") + cudaGetErrorString(e); return PTB_ERR_CUDA; }
     return PTB_OK;

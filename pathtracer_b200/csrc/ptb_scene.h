@@ -1473,6 +1473,48 @@ PTB_HD void shard_texel(F4* rgbw, F4* packed, long long idx, int W, int H, int t
     }
 }
 
+// ---- ray queries of the known-answer tests (PTB_KAT_RAY, PTB_KAT_RAY_WAVEFRONT) ------------------------------------------------------
+// input row: o[3], d[3], tmax, any_hit, narrowed to float (the sign of a zero survives the narrowing)
+PTB_HD void kat_ray_in(const double* a, V3& o, V3& d, float& tmax) {
+    o = v3((float)a[0], (float)a[1], (float)a[2]);
+    d = v3((float)a[3], (float)a[4], (float)a[5]);
+    tmax = (float)a[6];
+}
+// output row of a closest hit in extend_ray's convention (id >= 0: stored triangle, PTB_HIT_MISS, or an analytic object): object id,
+// original triangle id, t, b1, b2; a miss is -1, -1, -1, 0, 0
+PTB_HD void kat_ray_out(const SceneDev& sc, const Hit& h, int32_t id, double* o) {
+    o[0] = -1; o[1] = -1; o[2] = -1; o[3] = 0; o[4] = 0;
+    if (id >= 0) { o[0] = sc.tri_uv[id].object_has_uv & 0x7fffffff; o[1] = sc.tri_shade[id].orig; o[2] = h.t; o[3] = h.b1; o[4] = h.b2; }
+    else if (id != PTB_HIT_MISS) { o[0] = -2 - id; o[2] = h.t; }
+}
+// the analytic half of a closest-hit query, cut at tmax: the hit record a ray producer writes (analytic_hit) before the BVH sees the ray
+PTB_HD Hit kat_ray_analytic(const SceneDev& sc, V3 o, V3 d, float tmax) {
+    Hit h; h.b1 = 0; h.b2 = 0;
+    analytic_closest(sc, o, d, h.t, h.prim);
+    if (!(h.t < tmax)) { h.t = tmax; h.prim = PTB_HIT_MISS; }
+    return h;
+}
+// Closest hit: extend_ray (as k_primary runs it) with the analytic objects' t cut at tmax.  Any hit: the shadow query of shade_one,
+// analytic_occluded then the BVH8 up to 0.999 * dist_light (queue_shadow's bound), ghosts passing.
+PTB_HD void kat_ray(const SceneDev& sc, const double* a, double* out) {
+    V3 o, d;
+    float tmax;
+    kat_ray_in(a, o, d, tmax);
+    const AlphaCtx ac = alpha_ctx(sc);
+    Hit h;
+    if (a[7] != 0) {
+        const bool occ = analytic_occluded(sc, o, d, tmax) ||
+                         (sc.has_mesh && traverse<true, false>(sc.nodes, sc.tris, &ac, o, d, (float)((double)tmax * 0.999), h, nullptr));
+        out[0] = occ ? 1 : 0; out[1] = out[2] = out[3] = out[4] = 0;
+        return;
+    }
+    h = kat_ray_analytic(sc, o, d, tmax);
+    int32_t id = h.prim;
+    Hit m;
+    if (sc.has_mesh && traverse<false, false>(sc.nodes, sc.tris, &ac, o, d, h.t, m, nullptr)) { h = m; id = m.prim; }
+    kat_ray_out(sc, h, id, out);
+}
+
 // ---- known-answer tests (ptb_kat): one input row `a` of test `which` -> its output row `o`; false for an unknown test --------------
 PTB_HD bool kat_one(int which, const SceneDev& sc, const CameraDev& cam, const FilterDev& filt, int W, int H, const double* a, double* o) {
     switch (which) {
@@ -1492,6 +1534,7 @@ PTB_HD bool kat_one(int which, const SceneDev& sc, const CameraDev& cam, const F
     case PTB_KAT_RANDOM_PER_PIXEL: { float x, y; random_per_pixel((uint32_t)a[0], x, y); o[0] = x; o[1] = y; } break;
     case PTB_KAT_FILTER_RATIO: { int b0, b1, b2, b3; o[0] = filter_ratio(filt, (int)a[0], (int)a[1], W, H, b0, b1, b2, b3); } break;
     case PTB_KAT_MERL_INDEX: { int f, e; merl_index_both(v3((float)a[0], (float)a[1], (float)a[2]), v3((float)a[3], (float)a[4], (float)a[5]), f, e); o[0] = f; o[1] = e; } break;
+    case PTB_KAT_RAY: kat_ray(sc, a, o); break;
     default: return false;
     }
     return true;

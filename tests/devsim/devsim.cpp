@@ -279,6 +279,8 @@ int ptb_kat(ptb_ctx* c, int which, const ptb_camera* cam, int W, int H, const do
     FilterDev fd; memset(&fd, 0, sizeof(fd));
     if (which == PTB_KAT_FILTER_RATIO) filter_setup(fd, (float)in[2]);
     if (which == PTB_KAT_MERL_EVAL && (!c->committed || c->host.merl_tables.empty())) return PTB_ERR_STATE;
+    if (which == PTB_KAT_RAY_WAVEFRONT) which = PTB_KAT_RAY;   // no k_trace / k_exact here: the rows take the plain walk
+    if (which == PTB_KAT_RAY && !c->committed) return PTB_ERR_STATE;
     for (int k = 0; k < n; k++)
         if (!kat_one(which, c->sc, cd, fd, W, H, in + (size_t)k * is, out + (size_t)k * os)) return PTB_ERR_UNSUPPORTED;
     return PTB_OK;

@@ -156,12 +156,13 @@ def case_branch_converged(test_lib, oracle_lib):
     assert float(np.mean(rel_err(ia, ib) > 1e-3)) <= 0.03
 
 
-def case_sss_converged(test_lib, oracle_lib, spp=64):
+def case_sss_converged(test_lib, oracle_lib, spp=64, mk=None):
     """Subsurface scattering.  The reference picks the re-emergence point by reservoir sampling over the hits of a probe ray,
     one draw per hit in the traversal order of ITS binary BVH; a different BVH meets the hits in another order, so the two
     sides cannot draw the same numbers and the comparison is the north star's converged-image bound: at equal spp the test
-    image is as close to a high-spp oracle image as the oracle's own image of that spp, and the means agree within 2 %."""
-    mk = lambda L: scenes.config_sss(L, 40, 40, spp)
+    image is as close to a high-spp oracle image as the oracle's own image of that spp, and the means agree within 2 %.
+    `mk(lib)`: another subsurface scene (default: config_sss at 40 x 40, `spp`)."""
+    mk = mk or (lambda L: scenes.config_sss(L, 40, 40, spp))
     hi = mk(oracle_lib).commit()
     hi.nrays, hi.seed = 1024, 99
     ref_hi = hi.render_image_nopreviz().copy()
